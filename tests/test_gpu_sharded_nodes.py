@@ -177,8 +177,9 @@ def test_two_processes_over_cuda_ipc():
     processes on one device, and the device-side waits make progress because the two processes' kernels are
     time-sliced; every wait is bounded (SCS_ERR_PEER after the configured timeout), so a stall fails, not hangs."""
     env = dict(os.environ, PYTHONPATH=str(ROOT))
-    cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node=2", "--master-addr",
-           "127.0.0.1", "--master-port", "29617", str(ROOT / "tests" / "mp_sharded_worker.py")]  # fmt: skip
+    # --standalone: the rendezvous takes a free local port, so a busy fixed port cannot fail the test
+    cmd = [sys.executable, "-m", "torch.distributed.run", "--standalone", "--nnodes=1", "--nproc-per-node=2",
+           str(ROOT / "tests" / "mp_sharded_worker.py")]  # fmt: skip
     done = subprocess.run(cmd, env=env, capture_output=True, text=True, timeout=300, check=False)
     assert done.returncode == 0, done.stdout[-3000:] + done.stderr[-3000:]
     assert "SHARDED-OK" in done.stdout
