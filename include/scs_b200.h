@@ -257,6 +257,11 @@ const char *scs_newick_last_error(void);
  * NUL-terminated string ending in ';' (release with scs_free), *text_bytes its length. */
 int scs_flat_tree_newick(int64_t num_nodes, const int32_t *parent, const int32_t *taxon, const char *names,
                          size_t names_bytes, int num_taxa, char **text, size_t *text_bytes);
+/* scs_flat_tree_newick with a numeric label after every internal non-root node whose value is finite
+ * (printf "%.*f", digits, 0 <= digits <= 17); NaN = no label.  value[num_nodes] is indexed like parent. */
+int scs_flat_tree_newick_values(int64_t num_nodes, const int32_t *parent, const int32_t *taxon, const char *names,
+                                size_t names_bytes, int num_taxa, const double *value, int digits, char **text,
+                                size_t *text_bytes);
 void scs_free(void *ptr);
 int scs_forest_num_trees(const scs_forest *f);
 int64_t scs_forest_num_nodes(const scs_forest *f);
@@ -390,6 +395,18 @@ int scs_supertree_record_size(const scs_supertree *tree, int64_t index);
 int scs_supertree_record_wave(const scs_supertree *tree, int64_t index);
 int scs_supertree_record(const scs_supertree *tree, int64_t index, int32_t *taxa, int32_t *part,
                          scs_node_stats *stats);
+
+/* ---- source-tree support of the clades of a supertree ----------------------------------------------------- *
+ * Source-tree support of every clade of a supertree (parent[i] < i, taxon >= 0 on tips, ids in the forest's id
+ * space, no repeated taxon).  For internal node u and source tree t, A = leaves(u) restricted to the taxa X_t that t
+ * shares with the supertree is classified against t restricted to X_t (as scs_forest_induce restricts): irrelevant
+ * (|A| < 2 or A = X_t), support (A is one of its clusters), conflict (A overlaps one of its non-trivial clusters
+ * without nesting), permitted (otherwise).  counts[3 * num_nodes]: support, conflict, permitted per node (tips: 0);
+ * weighted (may be NULL) the same summed with the tree weights, in tree order; per_tree[4 * T]: shared clusters,
+ * source clusters, supertree clusters and their rooted Robinson-Foulds distance, all over the non-trivial clusters on
+ * X_t (0 when |X_t| < 2).  SCS_ERR_INPUT for a malformed supertree.  Returns after the results landed. */
+int scs_supertree_support(scs_ctx *ctx, const scs_forest *sources, int64_t num_nodes, const int32_t *parent,
+                          const int32_t *taxon, int32_t *counts, double *weighted, int32_t *per_tree);
 
 /* ---- one recursion node over several GPUs of one NVLink box (one process per GPU) ------------- *
  * The reference is single-process (scs.py:239 n_jobs=1); this is the B200 answer to its largest

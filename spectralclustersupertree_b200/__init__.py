@@ -1,7 +1,8 @@
 """Spectral Cluster Supertree on B200: the reference's public surface over a CUDA hot path.
 
 ``construct_supertree`` and ``load_trees`` keep the reference's signatures
-(ref: src/sc_supertree/__init__.py:6-12); the ``scs`` command lives in ``.cli``.
+(ref: src/sc_supertree/__init__.py:6-12); the ``scs`` command lives in ``.cli``.  ``clade_support`` scores a
+supertree against its source trees (per-clade support and conflict, per-tree Robinson-Foulds distance).
 Importing the package does not touch the GPU; the first ``construct_supertree`` call loads
 ``libscs_b200.so`` and raises if it (or a CUDA device) is missing -- there is no CPU fallback.
 """
@@ -10,5 +11,6 @@ __version__ = "2025.12.9+b200.1"
 
 from .load import load_trees  # noqa: E402
 from .scs import construct_supertree  # noqa: E402
+from .support import CladeSupport, clade_support  # noqa: E402
 
-__all__ = ["__version__", "construct_supertree", "load_trees"]
+__all__ = ["CladeSupport", "__version__", "clade_support", "construct_supertree", "load_trees"]

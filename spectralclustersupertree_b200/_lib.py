@@ -116,6 +116,11 @@ SIGNATURES: dict[str, tuple] = {
     "scs_newick_last_error": (c_char_p, []),
     "scs_forest_last_error": (c_char_p, []),
     "scs_flat_tree_newick": (c_int, [c_int64, _P, _P, c_char_p, c_size_t, c_int, POINTER(_P), POINTER(c_size_t)]),
+    "scs_flat_tree_newick_values": (
+        c_int,
+        [c_int64, _P, _P, c_char_p, c_size_t, c_int, _P, c_int, POINTER(_P), POINTER(c_size_t)],
+    ),
+    "scs_supertree_support": (c_int, [_P, _P, c_int64, _P, _P, _P, _P, _P]),
     "scs_profiler_range": (c_int, [c_int]),
     "scs_debug_small_cycles": (c_int, [_P, _P, c_int]),
     "scs_free": (None, [_P]),

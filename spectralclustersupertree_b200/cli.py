@@ -16,17 +16,29 @@ import click
 
 from . import __version__
 from .load import load_forest
-from .scs import supertree_newick_of_forest
+from .engine import default_engine
+from .scs import flat_newick, supertree_newick_of_forest
+from .support import flat_clade_support
 
 
-def run(in_file: str, out_file: str, weighting: str = "branch", contract_edges: bool = True) -> None:
-    """``load_trees`` + ``construct_supertree`` + ``write`` of the reference's command (ref: cli.py:33-39)."""
+def run(in_file: str, out_file: str, weighting: str = "branch", contract_edges: bool = True,
+        support_out: str | None = None) -> None:
+    """``load_trees`` + ``construct_supertree`` + ``write`` of the reference's command (ref: cli.py:33-39).  With
+    ``support_out`` the supertree is also written there with the V support index of every internal non-root node
+    (``support.flat_clade_support``) as its label."""
     forest = load_forest(in_file)
     if forest.num_trees == 0:  # what construct_supertree says about an empty list (ref: scs.py:63-65)
         msg = "There must be at least one tree to make a supertree."
         raise ValueError(msg)
-    text = supertree_newick_of_forest(forest, weighting.lower(), contract_edges=contract_edges)
-    Path(out_file).write_text(text + "\n")
+    if support_out is None:
+        text = supertree_newick_of_forest(forest, weighting.lower(), contract_edges=contract_edges)
+        Path(out_file).write_text(text + "\n")
+        return
+    engine = default_engine()
+    built = engine.supertree_build(forest, weighting.lower(), contract_edges=contract_edges)
+    Path(out_file).write_text(flat_newick(built["parent"], built["taxon"], forest.names) + "\n")
+    scored = flat_clade_support(forest, built["parent"], built["taxon"], engine=engine)
+    Path(support_out).write_text(scored.newick + "\n")
 
 
 @click.command(no_args_is_help=True)
@@ -46,15 +58,21 @@ def run(in_file: str, out_file: str, weighting: str = "branch", contract_edges: 
     default=False,
     is_flag=True,
 )
+@click.option(
+    "--support-out",
+    help="Also write the supertree with the V support index of each clade from the source trees.",
+    default=None,
+)
 def scs(
     in_file: str,
     out_file: str,
     pcg_weighting: Literal["one", "depth", "branch", "bootstrap"],
     *,
     disable_contraction: bool,
+    support_out: str | None,
 ) -> None:
     """Run spectral cluster supertree over the given set of source trees."""
-    run(in_file, out_file, pcg_weighting, contract_edges=not disable_contraction)
+    run(in_file, out_file, pcg_weighting, contract_edges=not disable_contraction, support_out=support_out)
 
 
 if __name__ == "__main__":

@@ -17,6 +17,7 @@
 #include <algorithm>
 #include <cerrno>
 #include <cmath>
+#include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <new>
@@ -323,9 +324,11 @@ int scs_forest_parse_newick(const char *text, size_t bytes, scs_forest **out, ch
  * PhyloNode.write, /root/reference/src/sc_supertree/cli.py:39): children in index order, tip labels quoted as
  * cogent3 quotes them (single quotes around a label with blanks or Newick punctuation, a quote doubled), no
  * branch lengths (the supertree has none), terminated by ';'. */
-int scs_flat_tree_newick(int64_t num_nodes, const int32_t *parent, const int32_t *taxon, const char *names,
-                         size_t names_bytes, int num_taxa, char **text_out, size_t *text_bytes) {
+static int flat_tree_newick(int64_t num_nodes, const int32_t *parent, const int32_t *taxon, const char *names,
+                            size_t names_bytes, int num_taxa, const double *value, int digits, char **text_out,
+                            size_t *text_bytes) {
     if (num_nodes <= 0 || !parent || !taxon || !names || !text_out || !text_bytes || num_taxa < 0) return SCS_ERR_INVALID;
+    if (value && (digits < 0 || digits > 17)) return SCS_ERR_INVALID;
     *text_out = nullptr;
     *text_bytes = 0;
     std::vector<const char *> label(static_cast<size_t>(num_taxa));
@@ -384,6 +387,12 @@ int scs_flat_tree_newick(int64_t num_nodes, const int32_t *parent, const int32_t
             const int32_t node = top.first;
             if (top.second == first[node + 1]) {
                 text.push_back(')');
+                if (value && node != 0 && std::isfinite(value[node])) {
+                    char label[64];
+                    const int len = std::snprintf(label, sizeof(label), "%.*f", digits, value[node]);
+                    if (len < 0 || len >= static_cast<int>(sizeof(label))) return SCS_ERR_INVALID;
+                    text.append(label, static_cast<size_t>(len));
+                }
                 stack.pop_back();
                 continue;
             }
@@ -406,6 +415,21 @@ int scs_flat_tree_newick(int64_t num_nodes, const int32_t *parent, const int32_t
     *text_out = buf;
     *text_bytes = text.size();
     return SCS_OK;
+}
+
+int scs_flat_tree_newick(int64_t num_nodes, const int32_t *parent, const int32_t *taxon, const char *names,
+                         size_t names_bytes, int num_taxa, char **text_out, size_t *text_bytes) {
+    return flat_tree_newick(num_nodes, parent, taxon, names, names_bytes, num_taxa, nullptr, 0, text_out, text_bytes);
+}
+
+/* The same with a numeric label after every internal non-root node whose value is finite: the support values of an
+ * annotated supertree (scs_supertree_support), written as "%.*f" so that scs_forest_parse_newick reads them back as
+ * supports. */
+int scs_flat_tree_newick_values(int64_t num_nodes, const int32_t *parent, const int32_t *taxon, const char *names,
+                                size_t names_bytes, int num_taxa, const double *value, int digits, char **text_out,
+                                size_t *text_bytes) {
+    if (!value) return SCS_ERR_INVALID;
+    return flat_tree_newick(num_nodes, parent, taxon, names, names_bytes, num_taxa, value, digits, text_out, text_bytes);
 }
 
 void scs_free(void *ptr) { std::free(ptr); }

@@ -238,6 +238,24 @@ class Engine:
         _check(status, self._ctx)
         return self._collect_supertree(handle, record)
 
+    def supertree_support(self, forest: "Forest", parent, taxon) -> tuple[np.ndarray, np.ndarray, np.ndarray]:
+        """``scs_supertree_support``: per node of the flat supertree (``parent[i] < i``, ``taxon`` = the forest's taxon
+        id on tips) the support / conflict / permitted counts ``[n, 3]`` (int32) and their sums over the tree weights
+        ``[n, 3]``; per source tree ``[T, 4]``: shared, source and supertree clusters, Robinson-Foulds distance."""
+        parent = np.ascontiguousarray(parent, dtype=np.int32)
+        taxon = np.ascontiguousarray(taxon, dtype=np.int32)
+        n = len(parent)
+        if len(taxon) != n:
+            msg = "parent and taxon must have the same length"
+            raise ValueError(msg)
+        counts = np.zeros((n, 3), dtype=np.int32)
+        weighted = np.zeros((n, 3), dtype=np.float64)
+        per_tree = np.zeros((forest.num_trees, 4), dtype=np.int32)
+        status = self._lib.scs_supertree_support(self._ctx, forest.handle, n, ptr(parent), ptr(taxon), ptr(counts),
+                                                 ptr(weighted), ptr(per_tree))  # fmt: skip
+        _check(status, self._ctx)
+        return counts, weighted, per_tree
+
     def _collect_supertree(self, handle, record: bool) -> dict:
         try:
             count = self._lib.scs_supertree_num_nodes(handle)
