@@ -408,6 +408,16 @@ int scs_supertree_record(const scs_supertree *tree, int64_t index, int32_t *taxa
 int scs_supertree_support(scs_ctx *ctx, const scs_forest *sources, int64_t num_nodes, const int32_t *parent,
                           const int32_t *taxon, int32_t *counts, double *weighted, int32_t *per_tree);
 
+/* Rooted triplet fit of the same supertree (validated as in scs_supertree_support; SCS_ERR_INPUT if malformed)
+ * against every source tree t, both restricted to the k taxa X_t they share.  A triplet {a, b, c} of X_t is resolved
+ * as ab|c when LCA(a, b) lies strictly below LCA(a, b, c), a fan otherwise.  per_tree[5 * T], int64 per tree: k,
+ * triplets resolved in the restricted source tree, triplets resolved in the restricted supertree, triplets resolved
+ * the same way in both (agree) and resolved differently (contradict); all but k are 0 when k < 3.  SCS_ERR_INVALID if
+ * a leaf of the supertree lies deeper than its shared-memory Fenwick tree allows (about 29 000 levels).  Returns
+ * after the results landed. */
+int scs_supertree_triplets(scs_ctx *ctx, const scs_forest *sources, int64_t num_nodes, const int32_t *parent,
+                           const int32_t *taxon, int64_t *per_tree);
+
 /* ---- one recursion node over several GPUs of one NVLink box (one process per GPU) ------------- *
  * The reference is single-process (scs.py:239 n_jobs=1); this is the B200 answer to its largest
  * recursion nodes.  A node with >= min_n taxa is ROW-SHARDED: rank r builds and keeps rows

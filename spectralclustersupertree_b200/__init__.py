@@ -2,7 +2,8 @@
 
 ``construct_supertree`` and ``load_trees`` keep the reference's signatures
 (ref: src/sc_supertree/__init__.py:6-12); the ``scs`` command lives in ``.cli``.  ``clade_support`` scores a
-supertree against its source trees (per-clade support and conflict, per-tree Robinson-Foulds distance).
+supertree against its source trees (per-clade support and conflict, per-tree Robinson-Foulds distance), and
+``triplet_fit`` compares their rooted triplets.
 Importing the package does not touch the GPU; the first ``construct_supertree`` call loads
 ``libscs_b200.so`` and raises if it (or a CUDA device) is missing -- there is no CPU fallback.
 """
@@ -12,5 +13,7 @@ __version__ = "2025.12.9+b200.1"
 from .load import load_trees  # noqa: E402
 from .scs import construct_supertree  # noqa: E402
 from .support import CladeSupport, clade_support  # noqa: E402
+from .triplets import TripletFit, triplet_fit  # noqa: E402
 
-__all__ = ["CladeSupport", "__version__", "clade_support", "construct_supertree", "load_trees"]
+__all__ = ["CladeSupport", "TripletFit", "__version__", "clade_support", "construct_supertree", "load_trees",
+           "triplet_fit"]

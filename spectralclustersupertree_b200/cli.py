@@ -19,26 +19,32 @@ from .load import load_forest
 from .engine import default_engine
 from .scs import flat_newick, supertree_newick_of_forest
 from .support import flat_clade_support
+from .triplets import flat_triplet_fit
 
 
 def run(in_file: str, out_file: str, weighting: str = "branch", contract_edges: bool = True,
-        support_out: str | None = None) -> None:
+        support_out: str | None = None, triplets_out: str | None = None) -> None:
     """``load_trees`` + ``construct_supertree`` + ``write`` of the reference's command (ref: cli.py:33-39).  With
     ``support_out`` the supertree is also written there with the V support index of every internal non-root node
-    (``support.flat_clade_support``) as its label."""
+    (``support.flat_clade_support``) as its label; with ``triplets_out`` the triplet fit of every source tree
+    (``triplets.flat_triplet_fit``) is written there as TSV.  The supertree is built once either way."""
     forest = load_forest(in_file)
     if forest.num_trees == 0:  # what construct_supertree says about an empty list (ref: scs.py:63-65)
         msg = "There must be at least one tree to make a supertree."
         raise ValueError(msg)
-    if support_out is None:
+    if support_out is None and triplets_out is None:
         text = supertree_newick_of_forest(forest, weighting.lower(), contract_edges=contract_edges)
         Path(out_file).write_text(text + "\n")
         return
     engine = default_engine()
     built = engine.supertree_build(forest, weighting.lower(), contract_edges=contract_edges)
     Path(out_file).write_text(flat_newick(built["parent"], built["taxon"], forest.names) + "\n")
-    scored = flat_clade_support(forest, built["parent"], built["taxon"], engine=engine)
-    Path(support_out).write_text(scored.newick + "\n")
+    if support_out is not None:
+        scored = flat_clade_support(forest, built["parent"], built["taxon"], engine=engine)
+        Path(support_out).write_text(scored.newick + "\n")
+    if triplets_out is not None:
+        fit = flat_triplet_fit(forest, built["parent"], built["taxon"], engine=engine)
+        Path(triplets_out).write_text(fit.tsv())
 
 
 @click.command(no_args_is_help=True)
@@ -63,6 +69,11 @@ def run(in_file: str, out_file: str, weighting: str = "branch", contract_edges: 
     help="Also write the supertree with the V support index of each clade from the source trees.",
     default=None,
 )
+@click.option(
+    "--triplets-out",
+    help="Also write, per source tree, the rooted triplets the supertree agrees with and contradicts (TSV).",
+    default=None,
+)
 def scs(
     in_file: str,
     out_file: str,
@@ -70,9 +81,11 @@ def scs(
     *,
     disable_contraction: bool,
     support_out: str | None,
+    triplets_out: str | None,
 ) -> None:
     """Run spectral cluster supertree over the given set of source trees."""
-    run(in_file, out_file, pcg_weighting, contract_edges=not disable_contraction, support_out=support_out)
+    run(in_file, out_file, pcg_weighting, contract_edges=not disable_contraction, support_out=support_out,
+        triplets_out=triplets_out)
 
 
 if __name__ == "__main__":

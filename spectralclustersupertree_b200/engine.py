@@ -256,6 +256,20 @@ class Engine:
         _check(status, self._ctx)
         return counts, weighted, per_tree
 
+    def supertree_triplets(self, forest: "Forest", parent, taxon) -> np.ndarray:
+        """``scs_supertree_triplets``: per source tree ``[T, 5]`` (int64): shared taxa, triplets resolved in the
+        restricted source tree, triplets resolved in the restricted supertree, agreeing and contradicting triplets."""
+        parent = np.ascontiguousarray(parent, dtype=np.int32)
+        taxon = np.ascontiguousarray(taxon, dtype=np.int32)
+        n = len(parent)
+        if len(taxon) != n:
+            msg = "parent and taxon must have the same length"
+            raise ValueError(msg)
+        per_tree = np.zeros((forest.num_trees, 5), dtype=np.int64)
+        status = self._lib.scs_supertree_triplets(self._ctx, forest.handle, n, ptr(parent), ptr(taxon), ptr(per_tree))
+        _check(status, self._ctx)
+        return per_tree
+
     def _collect_supertree(self, handle, record: bool) -> dict:
         try:
             count = self._lib.scs_supertree_num_nodes(handle)

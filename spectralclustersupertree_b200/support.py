@@ -111,6 +111,20 @@ class CladeSupport:
         return copy
 
 
+def _flat_supertree(supertree: PhyloNode, trees: Sequence[PhyloNode]) -> tuple[list, list[str], np.ndarray, np.ndarray]:
+    """The supertree as flat pre-order arrays (parent before child) over one joint sorted name list of its tips and
+    those of ``trees``: (nodes, names, parent, taxon)."""
+    nodes = list(supertree.preorder())
+    names = sorted({n.name for n in nodes if not n.children}.union(*(tree.get_tip_names() for tree in trees)))
+    taxon_id = {name: i for i, name in enumerate(names)}
+    index = {id(node): i for i, node in enumerate(nodes)}
+    parent = np.array([-1 if node.parent is None or id(node.parent) not in index else index[id(node.parent)]
+                       for node in nodes], dtype=np.int32)  # fmt: skip
+    parent[0] = -1
+    taxon = np.array([-1 if node.children else taxon_id[node.name] for node in nodes], dtype=np.int32)
+    return nodes, names, parent, taxon
+
+
 def clade_support(supertree: PhyloNode, trees: Sequence, weights: Sequence[float] | None = None, *,
                   engine: Engine | None = None) -> CladeSupport:  # fmt: skip
     """Score ``supertree`` against its source ``trees`` (see the module docstring).  ``NotCompleted`` entries are
@@ -121,15 +135,7 @@ def clade_support(supertree: PhyloNode, trees: Sequence, weights: Sequence[float
         msg = f"The number of trees ({len(trees)}) and tree weights ({len(weights)}) must match."
         raise ValueError(msg)
     kept = [i for i, tree in enumerate(trees) if not _is_not_completed(tree)]
-    # the supertree as flat pre-order arrays (parent before child) over one joint sorted name list
-    nodes = list(supertree.preorder())
-    names = sorted({n.name for n in nodes if not n.children}.union(*(trees[i].get_tip_names() for i in kept)))
-    taxon_id = {name: i for i, name in enumerate(names)}
-    index = {id(node): i for i, node in enumerate(nodes)}
-    parent = np.array([-1 if node.parent is None or id(node.parent) not in index else index[id(node.parent)]
-                       for node in nodes], dtype=np.int32)  # fmt: skip
-    parent[0] = -1
-    taxon = np.array([-1 if node.children else taxon_id[node.name] for node in nodes], dtype=np.int32)
+    nodes, names, parent, taxon = _flat_supertree(supertree, [trees[i] for i in kept])
     internal = np.array([i for i, node in enumerate(nodes) if node.children], dtype=np.int64)
 
     T = len(trees)
