@@ -291,6 +291,11 @@ int components(scs_ctx *ctx, int n, const uint32_t *bits, int32_t *label, int32_
 
 int components_async(scs_ctx *ctx, int n, const uint32_t *bits, int32_t *label, int32_t *count_dev);
 
+// The same labels from the node's leaf tours, without its graph; *bad_dev is raised for a malformed tour.
+int tour_components_async(scs_ctx *ctx, int n, int T, int64_t L, const int64_t *leaf_offsets,
+                          const int32_t *leaf_taxon, const int32_t *adj_depth, const int32_t *root_depth,
+                          int32_t *label, int32_t *count_dev, int32_t *bad_dev);
+
 int contract(scs_ctx *ctx, int n, const double *W, const uint32_t *adj_bits, const uint32_t *max_bits,
              int32_t *group, int32_t *m_host, double *Wc, double *degree_c);
 // `rows` (sharded): only contracted rows [row0, row1) are produced, into the row block Wc; W is then read
@@ -345,10 +350,19 @@ int small_cycles(scs_ctx *ctx, unsigned long long *out2, int reset);
 
 // One recursion node on device-resident tours.  part_dev[n] receives the component index or side;
 // if part_host is not null the result is also copied there before the function returns.
+// tour_components (the recursion drivers): a node above the small limit is first split into the components
+// of its tours, and a disconnected one returns without building its graph.  Off, the graph is always built,
+// so that scs_node_last_buffers shows W and the bits of every node.
 int node_split(scs_ctx *ctx, int n, int T, int64_t L, const int64_t *leaf_offsets, const int32_t *leaf_taxon,
                const int32_t *adj_depth, const double *adj_val, const int32_t *root_depth,
                const double *tree_weight, int contract_edges, uint64_t seed, int32_t *part_dev,
-               int32_t *part_host, scs_node_stats *stats);
+               int32_t *part_host, scs_node_stats *stats, bool tour_components = false);
+
+// scs_node_split_host with the choice above (driver.cu's host-forest recursion passes true).
+int node_split_host(scs_ctx *ctx, int n, int T, int64_t L, const int64_t *leaf_offsets, const int32_t *leaf_taxon,
+                    const int32_t *adj_depth, const double *adj_val, const int32_t *root_depth,
+                    const double *tree_weight, int contract_edges, uint64_t seed, int32_t *part,
+                    scs_node_stats *stats_out, bool tour_components);
 
 // ---- sharded nodes (shard.cu) -----------------------------------------------------------------------
 bool shard_applies(const scs_ctx *ctx, int n);

@@ -1,4 +1,5 @@
-// Connected components of a graph given as a bit adjacency matrix.
+// Connected components of a graph given as a bit adjacency matrix, or of a node's proper-cluster graph given
+// by its leaf tours (tour_components_async: no graph needed).
 //
 // Replaces _get_graph_components of the reference (/root/reference/src/sc_supertree/scs.py:458-492).
 // The reference explores the `edges` sets, i.e. "the pair co-occurred in some tree", which is the
@@ -128,6 +129,35 @@ __global__ void uf_flatten(int n, int32_t *parent, int32_t *label, int32_t *n_ro
     if (r == i) atomicAdd(n_roots, 1);
 }
 
+// Components straight from the leaf tours.  Taxa a and b are adjacent iff some tree holds both with their
+// LCA below its root; the leaves under one child of a root are a contiguous run of the tour whose
+// consecutive LCAs all lie below the root.  So hooking every consecutive pair i, i + 1 of a tree whose
+// adj_depth differs from the tree's root depth (the root test of the graph build) yields the same
+// components.  One thread per tour entry.  As on the bits, hooking every pair of a giant component is contention for
+// nothing: a first launch hooks every kTourSample-th pair only (snapshot == nullptr), then the roots are
+// snapshotted and the second launch hooks only the pairs whose snapshot roots still differ.
+constexpr int kTourSample = 16;
+__global__ void uf_hook_tours(int n, int T, int64_t L, const int64_t *__restrict__ leaf_offsets,
+                              const int32_t *__restrict__ leaf_taxon, const int32_t *__restrict__ adj_depth,
+                              const int32_t *__restrict__ root_depth, const int32_t *__restrict__ snapshot,
+                              int32_t *parent, int32_t *__restrict__ bad) {
+    const int64_t g = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
+    if (g >= L || (!snapshot && g % kTourSample != 0)) return;
+    int lo = 0, hi = T;  // largest t with leaf_offsets[t] <= g
+    while (hi - lo > 1) {
+        const int mid = (lo + hi) >> 1;
+        if (leaf_offsets[mid] <= g) lo = mid; else hi = mid;
+    }
+    const int64_t end = leaf_offsets[lo + 1];
+    const int a = leaf_taxon[g];
+    // out of range, or more leaves than taxa (a repeated taxon): rejected like the graph build rejects it
+    if (a < 0 || a >= n || end - leaf_offsets[lo] > n) { *bad = 1; return; }
+    if (g + 1 >= end || adj_depth[g] == root_depth[lo]) return;
+    const int b = leaf_taxon[g + 1];
+    if (b < 0 || b >= n || (snapshot && snapshot[a] == snapshot[b])) return;
+    uf_union(parent, a, b);
+}
+
 }  // namespace
 
 // Enqueue only: label[v] = smallest vertex of v's component, *count_dev = number of components.
@@ -151,6 +181,34 @@ int components_async(scs_ctx *ctx, int n, const uint32_t *bits, int32_t *label, 
     SCS_LAUNCHED(ctx, "uf_pick_giant");
     uf_hook_rest<<<row_blocks, 256, 0, ctx->stream>>>(n, words, bits, label, giant, parent);
     SCS_LAUNCHED(ctx, "uf_hook_rest");
+    uf_flatten<<<ceil_div(n, 256), 256, 0, ctx->stream>>>(n, parent, label, count_dev);
+    SCS_LAUNCHED(ctx, "uf_flatten");
+    return SCS_OK;
+}
+
+// Enqueue only: the components of the node's proper-cluster graph from its tours, labelled as components_async
+// labels them; *bad_dev is raised for a malformed tour.  Neither counter is cleared here.
+int tour_components_async(scs_ctx *ctx, int n, int T, int64_t L, const int64_t *leaf_offsets,
+                          const int32_t *leaf_taxon, const int32_t *adj_depth, const int32_t *root_depth,
+                          int32_t *label, int32_t *count_dev, int32_t *bad_dev) {
+    if (n <= 0 || T < 0 || L < 0 || !label || !count_dev || !bad_dev)
+        return fail(ctx, SCS_ERR_INVALID, "tour components: bad argument");
+    int32_t *parent;
+    int rc;
+    if ((rc = reserve_as(ctx, SLOT_UF_PARENT, static_cast<size_t>(n), &parent))) return rc;
+    uf_init<<<ceil_div(n, 256), 256, 0, ctx->stream>>>(n, parent);
+    SCS_LAUNCHED(ctx, "uf_init");
+    if (L > 0 && T > 0) {
+        // the snapshot lives in `label` until the final flatten overwrites it
+        uf_hook_tours<<<ceil_div(L, 256), 256, 0, ctx->stream>>>(n, T, L, leaf_offsets, leaf_taxon, adj_depth,
+                                                                 root_depth, nullptr, parent, bad_dev);
+        SCS_LAUNCHED(ctx, "uf_hook_tours");
+        uf_snapshot<<<ceil_div(n, 256), 256, 0, ctx->stream>>>(n, parent, label);
+        SCS_LAUNCHED(ctx, "uf_snapshot");
+        uf_hook_tours<<<ceil_div(L, 256), 256, 0, ctx->stream>>>(n, T, L, leaf_offsets, leaf_taxon, adj_depth,
+                                                                 root_depth, label, parent, bad_dev);
+        SCS_LAUNCHED(ctx, "uf_hook_tours");
+    }
     uf_flatten<<<ceil_div(n, 256), 256, 0, ctx->stream>>>(n, parent, label, count_dev);
     SCS_LAUNCHED(ctx, "uf_flatten");
     return SCS_OK;

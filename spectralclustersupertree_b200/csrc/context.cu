@@ -147,7 +147,51 @@ void clear_stats(scs_node_stats *s) {
 int node_split(scs_ctx *ctx, int n, int T, int64_t L, const int64_t *leaf_offsets, const int32_t *leaf_taxon,
                const int32_t *adj_depth, const double *adj_val, const int32_t *root_depth,
                const double *tree_weight, int contract_edges, uint64_t seed, int32_t *part_dev,
-               int32_t *part_host, scs_node_stats *stats) {
+               int32_t *part_host, scs_node_stats *stats, bool tour_components) {
+    auto number_components = [&](const int32_t *label) -> int {
+        // number the components by smallest member (scs.py:139 iterates them in arbitrary order)
+        int32_t *flag, *rank;
+        int rc;
+        if ((rc = reserve_as(ctx, SLOT_GROUP_PTR, 4 * static_cast<size_t>(n) + 8, &flag))) return rc;
+        rank = flag + n;
+        const int blocks = ceil_div(n, 256);
+        mark_roots<<<blocks, 256, 0, ctx->stream>>>(n, label, flag);
+        SCS_LAUNCHED(ctx, "mark_roots");
+        if ((rc = exclusive_scan(ctx, n, flag, rank))) return rc;
+        relabel_components<<<blocks, 256, 0, ctx->stream>>>(n, label, rank, part_dev);
+        SCS_LAUNCHED(ctx, "relabel_components");
+        if (part_host) {
+            SCS_CUDA(ctx, cudaMemcpyAsync(part_host, part_dev, sizeof(int32_t) * n, cudaMemcpyDeviceToHost, ctx->stream));
+            ctx->d2h_bytes += static_cast<int64_t>(sizeof(int32_t)) * n;
+            SCS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        }
+        return SCS_OK;
+    };
+    if (tour_components && n > ctx->small_limit) {
+        // A disconnected node needs no graph: its components come from the tours, one pass over the leaves.
+        // Every rank of a sharded build sees the same tours, so all of them leave here together.
+        const auto t0 = std::chrono::steady_clock::now();
+        int32_t *label, *scalars;
+        void *pin_v;
+        int rc;
+        if ((rc = reserve_as(ctx, SLOT_LABEL, static_cast<size_t>(n), &label))) return rc;
+        if ((rc = reserve_as(ctx, SLOT_SCALARS, 64, &scalars))) return rc;
+        if ((rc = reserve_pinned(ctx, 512, &pin_v))) return rc;
+        SCS_CUDA(ctx, cudaMemsetAsync(scalars, 0, 16 * sizeof(int32_t), ctx->stream));
+        if ((rc = tour_components_async(ctx, n, T, L, leaf_offsets, leaf_taxon, adj_depth, root_depth, label,
+                                        scalars + 8, scalars)))
+            return rc;
+        int32_t *host_scalars = reinterpret_cast<int32_t *>(static_cast<unsigned char *>(pin_v) + 256);
+        SCS_CUDA(ctx, cudaMemcpyAsync(host_scalars, scalars, 16 * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
+        SCS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        ctx->stage_seconds[6] += std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
+        if (host_scalars[0] != 0) return fail(ctx, SCS_ERR_INPUT, "leaf tour: taxon id out of range");
+        if (host_scalars[8] != 1) {
+            stats->n_components = host_scalars[8];
+            stats->contracted_size = n;
+            return number_components(label);
+        }
+    }
     if (shard_applies(ctx, n))
         return node_split_sharded(ctx, n, T, L, leaf_offsets, leaf_taxon, adj_depth, adj_val, root_depth, tree_weight,
                                   contract_edges, seed, part_dev, part_host, stats);
@@ -229,20 +273,7 @@ int node_split(scs_ctx *ctx, int n, int T, int64_t L, const int64_t *leaf_offset
     stats->contracted_size = n;
     const int blocks = ceil_div(n, 256);
 
-    if (ncomp != 1) {
-        // number the components by smallest member (scs.py:139 iterates them in arbitrary order)
-        int32_t *flag, *rank;
-        if ((rc = reserve_as(ctx, SLOT_GROUP_PTR, 4 * static_cast<size_t>(n) + 8, &flag))) return rc;
-        rank = flag + n;
-        mark_roots<<<blocks, 256, 0, ctx->stream>>>(n, label, flag);
-        SCS_LAUNCHED(ctx, "mark_roots");
-        if ((rc = exclusive_scan(ctx, n, flag, rank))) return rc;
-        relabel_components<<<blocks, 256, 0, ctx->stream>>>(n, label, rank, part_dev);
-        SCS_LAUNCHED(ctx, "relabel_components");
-        if ((rc = fetch_part())) return rc;
-        if (part_host) SCS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-        return SCS_OK;
-    }
+    if (ncomp != 1) return number_components(label);
 
     int m = n;
     const double *Wm = W;
@@ -319,6 +350,82 @@ int prewarm_node(scs_ctx *ctx, int n, int T, int64_t L) {
     if ((rc = reserve(ctx, SLOT_BUCKET_COUNT, 448 * (nL + 1), &p))) return rc;  // LeafStairs (pcg.cu)
     if ((rc = reserve(ctx, SLOT_START16, 64 * (nL + 1), &p))) return rc;
     return SCS_OK;
+}
+}  // namespace scs
+
+namespace scs {
+int node_split_host(scs_ctx *ctx, int n, int T, int64_t L, const int64_t *leaf_offsets, const int32_t *leaf_taxon,
+                    const int32_t *adj_depth, const double *adj_val, const int32_t *root_depth,
+                    const double *tree_weight, int contract_edges, uint64_t seed, int32_t *part,
+                    scs_node_stats *stats_out, bool tour_components) {
+    if (!ctx) return SCS_ERR_INVALID;
+    if (n <= 0 || T < 0 || L < 0 || !part) return fail(ctx, SCS_ERR_INVALID, "node_split: bad argument");
+    if (T > 0 && (!leaf_offsets || !root_depth || !tree_weight))
+        return fail(ctx, SCS_ERR_INVALID, "node_split: null tour array");
+    if (L > 0 && (!leaf_taxon || !adj_depth || !adj_val))
+        return fail(ctx, SCS_ERR_INVALID, "node_split: null tour array");
+    DeviceGuard guard(ctx->device);
+    scs_node_stats local;
+    scs_node_stats *stats = stats_out ? stats_out : &local;
+    clear_stats(stats);
+
+    // stage the tours through one pinned buffer so the copies are truly asynchronous
+    const size_t nT = static_cast<size_t>(T), nL = static_cast<size_t>(L);
+    const size_t b_off = (nT + 1) * sizeof(int64_t);
+    const size_t b_val = nL * sizeof(double);
+    const size_t b_w = nT * sizeof(double);
+    const size_t b_tax = nL * sizeof(int32_t);
+    const size_t b_dep = nL * sizeof(int32_t);
+    const size_t b_root = nT * sizeof(int32_t);
+    const size_t total = b_off + b_val + b_w + b_tax + b_dep + b_root + 64;
+    int rc;
+    if (ctx->pinned_io_bytes < total) {
+        if (ctx->pinned_io) {
+            SCS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+            SCS_CUDA(ctx, cudaFreeHost(ctx->pinned_io));
+            ctx->pinned_io = nullptr;
+            ctx->pinned_io_bytes = 0;
+        }
+        const size_t want = 2 * total + 4096;  // pinned allocations synchronise the device: grow rarely
+        SCS_CUDA(ctx, cudaMallocHost(&ctx->pinned_io, want));
+        ctx->pinned_io_bytes = want;
+    }
+    unsigned char *stage = static_cast<unsigned char *>(ctx->pinned_io);
+    unsigned char *dev_stage;
+    if ((rc = reserve_as(ctx, SLOT_TOUR_OFFSETS, total, &dev_stage))) return rc;
+    size_t o_off = 0, o_val = o_off + b_off, o_w = o_val + b_val, o_tax = o_w + b_w, o_dep = o_tax + b_tax,
+           o_root = o_dep + b_dep;
+    if (T > 0) {
+        std::memcpy(stage + o_off, leaf_offsets, b_off);
+        std::memcpy(stage + o_w, tree_weight, b_w);
+        std::memcpy(stage + o_root, root_depth, b_root);
+    } else {
+        std::memset(stage + o_off, 0, b_off);
+    }
+    if (L > 0) {
+        std::memcpy(stage + o_val, adj_val, b_val);
+        std::memcpy(stage + o_tax, leaf_taxon, b_tax);
+        std::memcpy(stage + o_dep, adj_depth, b_dep);
+    }
+    SCS_CUDA(ctx, cudaMemcpyAsync(dev_stage, stage, total - 64, cudaMemcpyHostToDevice, ctx->stream));
+    ctx->h2d_bytes += static_cast<int64_t>(total - 64);
+    ctx->pending_units = 0.0;
+    for (int t = 0; t < T; ++t) {
+        const double k = static_cast<double>(leaf_offsets[t + 1] - leaf_offsets[t]);
+        ctx->pending_units += k * (k - 1.0);
+    }
+
+    int32_t *part_dev;
+    if ((rc = reserve_as(ctx, SLOT_PART, static_cast<size_t>(n), &part_dev))) return rc;
+    rc = node_split(ctx, n, T, L, reinterpret_cast<const int64_t *>(dev_stage + o_off),
+                    reinterpret_cast<const int32_t *>(dev_stage + o_tax),
+                    reinterpret_cast<const int32_t *>(dev_stage + o_dep),
+                    reinterpret_cast<const double *>(dev_stage + o_val),
+                    reinterpret_cast<const int32_t *>(dev_stage + o_root),
+                    reinterpret_cast<const double *>(dev_stage + o_w), contract_edges, seed, part_dev, part, stats,
+                    tour_components);
+    ctx->pending_units = 0.0;
+    return rc;
 }
 }  // namespace scs
 
@@ -632,73 +739,8 @@ int scs_node_split_host(scs_ctx *ctx, int n, int T, int64_t L, const int64_t *le
                         const int32_t *leaf_taxon, const int32_t *adj_depth, const double *adj_val,
                         const int32_t *root_depth, const double *tree_weight, int contract_edges, uint64_t seed,
                         int32_t *part, scs_node_stats *stats_out) {
-    if (!ctx) return SCS_ERR_INVALID;
-    if (n <= 0 || T < 0 || L < 0 || !part) return fail(ctx, SCS_ERR_INVALID, "node_split: bad argument");
-    if (T > 0 && (!leaf_offsets || !root_depth || !tree_weight))
-        return fail(ctx, SCS_ERR_INVALID, "node_split: null tour array");
-    if (L > 0 && (!leaf_taxon || !adj_depth || !adj_val))
-        return fail(ctx, SCS_ERR_INVALID, "node_split: null tour array");
-    DeviceGuard guard(ctx->device);
-    scs_node_stats local;
-    scs_node_stats *stats = stats_out ? stats_out : &local;
-    clear_stats(stats);
-
-    // stage the tours through one pinned buffer so the copies are truly asynchronous
-    const size_t nT = static_cast<size_t>(T), nL = static_cast<size_t>(L);
-    const size_t b_off = (nT + 1) * sizeof(int64_t);
-    const size_t b_val = nL * sizeof(double);
-    const size_t b_w = nT * sizeof(double);
-    const size_t b_tax = nL * sizeof(int32_t);
-    const size_t b_dep = nL * sizeof(int32_t);
-    const size_t b_root = nT * sizeof(int32_t);
-    const size_t total = b_off + b_val + b_w + b_tax + b_dep + b_root + 64;
-    int rc;
-    if (ctx->pinned_io_bytes < total) {
-        if (ctx->pinned_io) {
-            SCS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-            SCS_CUDA(ctx, cudaFreeHost(ctx->pinned_io));
-            ctx->pinned_io = nullptr;
-            ctx->pinned_io_bytes = 0;
-        }
-        const size_t want = 2 * total + 4096;  // pinned allocations synchronise the device: grow rarely
-        SCS_CUDA(ctx, cudaMallocHost(&ctx->pinned_io, want));
-        ctx->pinned_io_bytes = want;
-    }
-    unsigned char *stage = static_cast<unsigned char *>(ctx->pinned_io);
-    unsigned char *dev_stage;
-    if ((rc = reserve_as(ctx, SLOT_TOUR_OFFSETS, total, &dev_stage))) return rc;
-    size_t o_off = 0, o_val = o_off + b_off, o_w = o_val + b_val, o_tax = o_w + b_w, o_dep = o_tax + b_tax,
-           o_root = o_dep + b_dep;
-    if (T > 0) {
-        std::memcpy(stage + o_off, leaf_offsets, b_off);
-        std::memcpy(stage + o_w, tree_weight, b_w);
-        std::memcpy(stage + o_root, root_depth, b_root);
-    } else {
-        std::memset(stage + o_off, 0, b_off);
-    }
-    if (L > 0) {
-        std::memcpy(stage + o_val, adj_val, b_val);
-        std::memcpy(stage + o_tax, leaf_taxon, b_tax);
-        std::memcpy(stage + o_dep, adj_depth, b_dep);
-    }
-    SCS_CUDA(ctx, cudaMemcpyAsync(dev_stage, stage, total - 64, cudaMemcpyHostToDevice, ctx->stream));
-    ctx->h2d_bytes += static_cast<int64_t>(total - 64);
-    ctx->pending_units = 0.0;
-    for (int t = 0; t < T; ++t) {
-        const double k = static_cast<double>(leaf_offsets[t + 1] - leaf_offsets[t]);
-        ctx->pending_units += k * (k - 1.0);
-    }
-
-    int32_t *part_dev;
-    if ((rc = reserve_as(ctx, SLOT_PART, static_cast<size_t>(n), &part_dev))) return rc;
-    rc = node_split(ctx, n, T, L, reinterpret_cast<const int64_t *>(dev_stage + o_off),
-                    reinterpret_cast<const int32_t *>(dev_stage + o_tax),
-                    reinterpret_cast<const int32_t *>(dev_stage + o_dep),
-                    reinterpret_cast<const double *>(dev_stage + o_val),
-                    reinterpret_cast<const int32_t *>(dev_stage + o_root),
-                    reinterpret_cast<const double *>(dev_stage + o_w), contract_edges, seed, part_dev, part, stats);
-    ctx->pending_units = 0.0;
-    return rc;
+    return node_split_host(ctx, n, T, L, leaf_offsets, leaf_taxon, adj_depth, adj_val, root_depth, tree_weight,
+                           contract_edges, seed, part, stats_out, false);
 }
 
 int scs_node_last_buffers(scs_ctx *ctx, int *n, int *m, double **W_dev, uint32_t **adj_bits_dev,

@@ -410,7 +410,7 @@ class DeviceDriver {
                         tours_.adj_depth.as<int32_t>() + job.where.leaf_begin, tours_.adj_val.as<double>() + job.where.leaf_begin,
                         tours_.root_depth.as<int32_t>() + job.where.tree_begin, forest.weight.as<double>() + job.where.tree_begin,
                         contract_, node_seed(seed_, job.taxa[0], job.taxa.size()), part_dev_.as<int32_t>() + s.part_at, nullptr,
-                        &s.stats);
+                        &s.stats, true);
         ctx_->pending_units = 0.0;
         ctx_->shard.engaged = false;
         return rc;

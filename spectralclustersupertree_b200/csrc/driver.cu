@@ -509,9 +509,9 @@ class Driver {
         if (rc) return rc;
         res.part.resize(n);
         // the seed only picks the Lanczos start vector; it is a function of the node's taxa (driver.hpp)
-        return scs_node_split_host(ctx, n, T, L, buf.off.data(), buf.tax.data(), buf.dep.data(), buf.val.data(),
-                                   buf.root.data(), buf.wgt.data(), contract_, node_seed(seed_, taxa[0], taxa.size()),
-                                   res.part.data(), &res.stats);
+        return node_split_host(ctx, n, T, L, buf.off.data(), buf.tax.data(), buf.dep.data(), buf.val.data(),
+                               buf.root.data(), buf.wgt.data(), contract_, node_seed(seed_, taxa[0], taxa.size()),
+                               res.part.data(), &res.stats, true);
     }
 
     // The staged path is a chain of small launches and a few host round trips per node: latency, not

@@ -22,6 +22,8 @@
 #include "shard.cuh"
 #include "spectral_dev.cuh"
 
+#include <cooperative_groups.h>
+
 #include <algorithm>
 #include <chrono>
 #include <cmath>
@@ -31,6 +33,7 @@ namespace scs {
 namespace {
 
 using namespace specdev;
+namespace cg = cooperative_groups;
 
 // ---- degree and scaling ---------------------------------------------------------------------
 // one warp per row: d[a] = sum_b W[a][b]   (scipy _laplacian.py:543: column sums of a symmetric matrix)
@@ -223,69 +226,117 @@ __global__ void random_start(int m, uint64_t seed, double *__restrict__ w) {
     w[i] = 2.0 * (static_cast<double>(r >> 11) * (1.0 / 9007199254740992.0)) - 1.0;
 }
 
-// h[k] = basis[k] . w   for k in [0, nb); one CTA per basis vector, fixed summation order
-__global__ void __launch_bounds__(kVecThreads)
-multi_dot(int m, const double *__restrict__ basis, const double *__restrict__ w, double *__restrict__ h) {
-    __shared__ double scratch[33];
-    const double *b = basis + static_cast<size_t>(blockIdx.x) * m;
-    double acc = 0.0;
-    for (int i = threadIdx.x; i < m; i += kVecThreads) acc = fma(b[i], w[i], acc);
-    acc = block_sum(acc, scratch);
-    if (threadIdx.x == 0) h[blockIdx.x] = acc;
-}
+// ---- Lanczos step tail of a large node (m > kFusedMax): one launch of a thread-block cluster ------------------
+// Everything of a step except the operator application: both classical Gram-Schmidt passes against the nb leading
+// basis vectors, the norm, the next basis vector v_{j+1} and z = isd .* v_{j+1}, alpha_j / beta_j and, at check
+// steps, the projected eigenproblem.  Its verdict is latched in state[1] (state[2] = the step), so that the
+// launches queued behind it fall through, as lanczos_tail does for m <= kFusedMax.  The basis (a few MB) stays in
+// L2; kStepCluster CTAs share the work and meet at cluster barriers, which also make the global stores of one
+// phase visible to the next.  No cooperative launch and no grid-wide sync: the cluster is co-scheduled.
+// The summation order of every value is fixed by the decomposition below, whatever the cluster size:
+//   h[k] = basis[k] . w     by one CTA of kVecThreads threads (thread stride, then block_sum);
+//   w[i] -= h[k] basis[k]i  one thread per element, k ascending;
+//   |w|^2                   kOneCta virtual threads (stride kOneCta, warp sums, then the 32 warp sums), computed
+//                           by every CTA from the whole of w, so that all of them scale by the same bits;
+//   projected problem       tridiag_solve by kVecThreads threads of CTA 0.
+// state: [0] breakdown step, [1] done, [2] step at which done was raised.
+constexpr int kStepCluster = 8;
+constexpr int kDots = 4;  // basis vectors a CTA dots with w in one sweep
 
-// w -= sum_k h[k] basis[k]
-__global__ void __launch_bounds__(kVecThreads)
-multi_axpy(int m, int nb, const double *__restrict__ basis, const double *__restrict__ h, double *__restrict__ w) {
-    extern __shared__ double hs[];
-    for (int k = threadIdx.x; k < nb; k += kVecThreads) hs[k] = h[k];
+__global__ void __cluster_dims__(kStepCluster, 1, 1) __launch_bounds__(kVecThreads, 1)
+lanczos_step(int m, int j, int nb, int hj, int check, const double *__restrict__ basis, double *w,
+             const double *__restrict__ isd, double *h1, double *h2, double *alpha, double *beta, double *next,
+             double *z, int32_t *state, double *coef, double *ritz) {
+    extern __shared__ double step_smem[];
+    double *hs = step_smem;                 // [kMaxBasis + 8] coefficients of the current pass
+    double *tri = hs + (kMaxBasis + 8);     // 5 (j + 2) doubles for the projected problem
+    __shared__ double scratch[33];
+    __shared__ int counts[kVecThreads];
+    __shared__ double pair[4];
+    if (state[1]) return;  // converged earlier in this chunk (written by an earlier launch: the same in every CTA)
+    cg::cluster_group cluster = cg::this_cluster();
+    const int rank = static_cast<int>(cluster.block_rank());
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int first = rank * kVecThreads + tid, stride = kStepCluster * kVecThreads;
+    for (int pass = 0; pass < 2; ++pass) {
+        double *h = pass ? h2 : h1;
+        // this CTA's vectors k = rank + q kStepCluster, kDots at a time in one sweep over w (independent sums)
+        for (int k0 = rank; k0 < nb; k0 += kDots * kStepCluster) {
+            const double *b[kDots];
+            double acc[kDots];
+#pragma unroll
+            for (int q = 0; q < kDots; ++q) {
+                const int k = min(k0 + q * kStepCluster, nb - 1);  // past the end: a duplicate, never stored
+                b[q] = basis + static_cast<size_t>(k) * m;
+                acc[q] = 0.0;
+            }
+#pragma unroll 2
+            for (int i = tid; i < m; i += kVecThreads) {
+                const double wi = w[i];
+#pragma unroll
+                for (int q = 0; q < kDots; ++q) acc[q] = fma(b[q][i], wi, acc[q]);
+            }
+#pragma unroll
+            for (int q = 0; q < kDots; ++q) {
+                const double sum = block_sum(acc[q], scratch);
+                if (tid == 0 && k0 + q * kStepCluster < nb) h[k0 + q * kStepCluster] = sum;
+            }
+        }
+        cluster.sync();
+        for (int k = tid; k < nb; k += kVecThreads) hs[k] = h[k];
+        __syncthreads();
+        for (int i = first; i < m; i += stride) {
+            double acc = w[i];
+#pragma unroll 8
+            for (int k = 0; k < nb; ++k) acc = fma(-hs[k], basis[static_cast<size_t>(k) * m + i], acc);
+            w[i] = acc;
+        }
+        cluster.sync();
+    }
+    // |w|^2 as one CTA of kOneCta threads sums it: virtual thread q * kVecThreads + tid, warp q * 8 + warp
+    constexpr int kVirtual = kOneCta / kVecThreads;
+    static_assert(kOneCta == 32 * 32 && kVirtual * kVecThreads == kOneCta, "32 virtual warps of 32 threads");
+#pragma unroll
+    for (int q = 0; q < kVirtual; ++q) {
+        double ss = 0.0;
+        for (int i = q * kVecThreads + tid; i < m; i += kOneCta) ss = fma(w[i], w[i], ss);
+        ss = warp_sum(ss);
+        if (lane == 0) scratch[q * (kVecThreads / 32) + warp] = ss;
+    }
     __syncthreads();
-    const int i = blockIdx.x * kVecThreads + threadIdx.x;
-    if (i >= m) return;
-    double acc = w[i];
-    for (int k = 0; k < nb; ++k) acc = fma(-hs[k], basis[static_cast<size_t>(k) * m + i], acc);
-    w[i] = acc;
-}
-
-// beta = |w|; next = w / beta; z = isd .* next; records alpha_j = h1[hj] + h2[hj] (hj = position of
-// v_j in the basis) and beta_j.  j == 0 is the normalisation of the start vector (nothing recorded).
-// The first j whose beta_j is negligible (the Krylov space is invariant: later vectors are noise)
-// is latched in state[0]; the projected problem is then solved on the leading block only.  One CTA.
-__global__ void __launch_bounds__(kOneCta)
-normalize_step(int m, int j, int hj, const double *__restrict__ w, const double *__restrict__ isd,
-               const double *__restrict__ h1, const double *__restrict__ h2, double *__restrict__ alpha,
-               double *__restrict__ beta, double *__restrict__ next, double *__restrict__ z,
-               int32_t *__restrict__ state) {
-    __shared__ double scratch[33];
-    double ss = 0.0;
-    for (int i = threadIdx.x; i < m; i += blockDim.x) ss = fma(w[i], w[i], ss);
-    ss = block_sum(ss, scratch);
-    const double b = sqrt(ss);
-    if (threadIdx.x == 0) {
-        beta[j] = b;
+    if (warp == 0) {
+        const double t = warp_sum(scratch[lane]);
+        if (lane == 0) scratch[32] = t;
+    }
+    __syncthreads();
+    const double bnorm = sqrt(scratch[32]);
+    if (rank == 0 && tid == 0) {
+        beta[j] = bnorm;
         if (j > 0) {
             alpha[j] = h1[hj] + h2[hj];
-            if (b <= kBreakdown && state[0] == 0) state[0] = j;
+            if (bnorm <= kBreakdown && state[0] == 0) state[0] = j;
         } else {
             state[0] = 0;
         }
     }
-    const double inv = b > 0.0 ? 1.0 / b : 0.0;
-    for (int i = threadIdx.x; i < m; i += blockDim.x) {
+    const double inv = bnorm > 0.0 ? 1.0 / bnorm : 0.0;
+    for (int i = first; i < m; i += stride) {
         const double v = w[i] * inv;
         next[i] = v;
         z[i] = isd[i] * v;
     }
+    if (rank != 0 || !check || j == 0) return;
+    __syncthreads();  // alpha / beta / state written by thread 0 are read below
+    tridiag_solve(j, alpha, beta, state, coef, ritz, tri, counts, pair);
+    if (tid == 0) {
+        ritz[5] = static_cast<double>(j);
+        if (ritz[3] <= kBreakdown || ritz[2] <= kResidualTol) {
+            state[1] = 1;
+            state[2] = j;
+        }
+    }
 }
-
-__global__ void __launch_bounds__(256)
-tridiag_ritz(int jrun, const double *__restrict__ alpha, const double *__restrict__ beta,
-             const int32_t *__restrict__ state, double *__restrict__ coef, double *__restrict__ out) {
-    extern __shared__ double sm[];
-    __shared__ int counts[256];
-    __shared__ double pair[4];
-    tridiag_solve(jrun, alpha, beta, state, coef, out, sm, counts, pair);
-}
+constexpr size_t kStepSmem = (kMaxBasis + 8 + 5 * (kMaxBasis + 2)) * sizeof(double);
 
 // ---- fused Lanczos step tail (m <= kFusedMax) -----------------------------------------------------
 // Everything of a Lanczos step except the operator application, in one single-CTA launch: both
@@ -446,13 +497,6 @@ int lanczos_largest(scs_ctx *ctx, int m, const double *W, const LanczosBuffers &
     const int vec_blocks = ceil_div(m, kVecThreads);
     double *v0 = b.basis + static_cast<size_t>(ndefl - 1) * m;  // v_k lives at v0 + k m
     double *w = b.w;  // the vector being orthogonalised: b.w, or the window buffer a sharded matvec filled
-    auto orthogonalise = [&](int nb, double *h) -> int {
-        multi_dot<<<nb, kVecThreads, 0, ctx->stream>>>(m, b.basis, w, h);
-        SCS_LAUNCHED(ctx, "multi_dot");
-        multi_axpy<<<vec_blocks, kVecThreads, nb * sizeof(double), ctx->stream>>>(m, nb, b.basis, h, w);
-        SCS_LAUNCHED(ctx, "multi_axpy");
-        return SCS_OK;
-    };
     int rc;
     int jdone = 0;
     const bool fused = m <= kFusedMax;
@@ -462,6 +506,23 @@ int lanczos_largest(scs_ctx *ctx, int m, const double *W, const LanczosBuffers &
         ctx->tail_configured = true;
     }
     const size_t tail_smem = (static_cast<size_t>(m) + 6 * (kMaxBasis + 8)) * sizeof(double);
+    // everything of step j but the matvec: one CTA up to kFusedMax, one cluster above
+    auto step_tail = [&](int j, int check) -> int {
+        const int nb = j == 0 ? ndefl : ndefl + j;
+        const int hj = j == 0 ? 0 : ndefl - 1 + j;
+        double *next = v0 + static_cast<size_t>(j + 1) * m;
+        if (fused) {
+            lanczos_tail<<<1, kOneCta, tail_smem, ctx->stream>>>(m, j, nb, hj, check, b.basis, w, b.isd, b.alpha, b.beta,
+                                                                next, b.z, b.state, b.coef, b.ritz);
+            SCS_LAUNCHED(ctx, "lanczos_tail");
+        } else {
+            lanczos_step<<<kStepCluster, kVecThreads, kStepSmem, ctx->stream>>>(m, j, nb, hj, check, b.basis, w, b.isd,
+                                                                               b.h1, b.h2, b.alpha, b.beta, next, b.z,
+                                                                               b.state, b.coef, b.ritz);
+            SCS_LAUNCHED(ctx, "lanczos_step");
+        }
+        return SCS_OK;
+    };
     for (int attempt = 0; attempt <= kMaxRestarts && !out->converged; ++attempt) {
         w = b.w;
         if (attempt == 0) {
@@ -472,82 +533,38 @@ int lanczos_largest(scs_ctx *ctx, int m, const double *W, const LanczosBuffers &
             SCS_CUDA(ctx, cudaMemcpyAsync(b.w, y, sizeof(double) * m, cudaMemcpyDeviceToDevice, ctx->stream));
             out->restarts = attempt;
         }
-        if (fused) {
-            SCS_CUDA(ctx, cudaMemsetAsync(b.state, 0, 4 * sizeof(int32_t), ctx->stream));
-            lanczos_tail<<<1, kOneCta, tail_smem, ctx->stream>>>(m, 0, ndefl, 0, 0, b.basis, b.w, b.isd, b.alpha, b.beta,
-                                                                v0 + m, b.z, b.state, b.coef, b.ritz);
-            SCS_LAUNCHED(ctx, "lanczos_tail");
-            // steps are queued a chunk at a time; the tail of a check step latches convergence on the
-            // device and everything queued behind it falls through
-            int j = 1;
-            int attempt_matvecs = 0;
-            bool done = false;
-            while (j <= jmax && !done) {
-                const int chunk_end = std::min(jmax, j == 1 ? 16 : j + 3);  // chunks end on check steps
-                for (; j <= chunk_end; ++j) {
-                    if ((rc = launch_matvec(ctx, m, W, b.isd, b.z, &w, b.state + 1, rows))) return rc;
-                    const int check = j == jmax || (j % 4) == 0;
-                    lanczos_tail<<<1, kOneCta, tail_smem, ctx->stream>>>(
-                        m, j, ndefl + j, ndefl - 1 + j, check, b.basis, w, b.isd, b.alpha, b.beta,
-                        v0 + static_cast<size_t>(j + 1) * m, b.z, b.state, b.coef, b.ritz);
-                    SCS_LAUNCHED(ctx, "lanczos_tail");
-                }
-                SCS_CUDA(ctx, cudaMemcpyAsync(b.pin, b.ritz, 6 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-                SCS_CUDA(ctx, cudaMemcpyAsync(b.pin + 6, b.state, 4 * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
-                SCS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-                const int32_t *st = reinterpret_cast<const int32_t *>(b.pin + 6);
-                out->theta1 = b.pin[0];
-                out->theta2 = b.pin[1];
-                out->estimate = b.pin[2];
-                out->steps = static_cast<int>(b.pin[4]);
-                jdone = static_cast<int>(b.pin[5]);  // the step of the last check that ran
-                if (st[1]) {
-                    done = true;
-                    out->converged = true;
-                    out->invariant = b.pin[3] <= kBreakdown;
-                    attempt_matvecs = st[2];  // steps actually applied before the flag went up
-                } else {
-                    attempt_matvecs = chunk_end;
-                }
+        SCS_CUDA(ctx, cudaMemsetAsync(b.state, 0, 4 * sizeof(int32_t), ctx->stream));
+        if ((rc = step_tail(0, 0))) return rc;
+        // steps are queued a chunk at a time; the tail of a check step latches convergence on the
+        // device and everything queued behind it falls through
+        int j = 1;
+        int attempt_matvecs = 0;
+        bool done = false;
+        while (j <= jmax && !done) {
+            const int chunk_end = std::min(jmax, j == 1 ? 16 : j + 3);  // chunks end on check steps
+            for (; j <= chunk_end; ++j) {
+                if ((rc = launch_matvec(ctx, m, W, b.isd, b.z, &w, b.state + 1, rows))) return rc;
+                if ((rc = step_tail(j, j == jmax || (j % 4) == 0))) return rc;
             }
-            out->matvecs += attempt_matvecs;
-        } else {
-            if ((rc = orthogonalise(ndefl, b.h1))) return rc;
-            if ((rc = orthogonalise(ndefl, b.h2))) return rc;
-            normalize_step<<<1, kOneCta, 0, ctx->stream>>>(m, 0, 0, w, b.isd, b.h1, b.h2, b.alpha, b.beta, v0 + m, b.z,
-                                                           b.state);
-            SCS_LAUNCHED(ctx, "normalize_step");
-            for (int j = 1; j <= jmax; ++j) {
-                if ((rc = launch_matvec(ctx, m, W, b.isd, b.z, &w, nullptr, rows))) return rc;
-                out->matvecs += 1;
-                if ((rc = orthogonalise(ndefl + j, b.h1))) return rc;
-                if ((rc = orthogonalise(ndefl + j, b.h2))) return rc;
-                normalize_step<<<1, kOneCta, 0, ctx->stream>>>(m, j, ndefl - 1 + j, w, b.isd, b.h1, b.h2, b.alpha,
-                                                               b.beta, v0 + static_cast<size_t>(j + 1) * m, b.z, b.state);
-                SCS_LAUNCHED(ctx, "normalize_step");
-                jdone = j;
-                const bool check = j == jmax || (j % 4) == 0;
-                if (!check) continue;
-                tridiag_ritz<<<1, 256, 5 * (j + 2) * sizeof(double), ctx->stream>>>(j, b.alpha, b.beta, b.state, b.coef,
-                                                                                   b.ritz);
-                SCS_LAUNCHED(ctx, "tridiag_ritz");
-                SCS_CUDA(ctx, cudaMemcpyAsync(b.pin, b.ritz, 5 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-                SCS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-                out->theta1 = b.pin[0];
-                out->theta2 = b.pin[1];
-                out->estimate = b.pin[2];
-                out->steps = static_cast<int>(b.pin[4]);
-                if (b.pin[3] <= kBreakdown) {
-                    out->converged = true;
-                    out->invariant = true;
-                    break;
-                }
-                if (out->estimate <= kResidualTol) {
-                    out->converged = true;
-                    break;
-                }
+            SCS_CUDA(ctx, cudaMemcpyAsync(b.pin, b.ritz, 6 * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+            SCS_CUDA(ctx, cudaMemcpyAsync(b.pin + 6, b.state, 4 * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
+            SCS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+            const int32_t *st = reinterpret_cast<const int32_t *>(b.pin + 6);
+            out->theta1 = b.pin[0];
+            out->theta2 = b.pin[1];
+            out->estimate = b.pin[2];
+            out->steps = static_cast<int>(b.pin[4]);
+            jdone = static_cast<int>(b.pin[5]);  // the step of the last check that ran
+            if (st[1]) {
+                done = true;
+                out->converged = true;
+                out->invariant = b.pin[3] <= kBreakdown;
+                attempt_matvecs = st[2];  // steps actually applied before the flag went up
+            } else {
+                attempt_matvecs = chunk_end;
             }
         }
+        out->matvecs += attempt_matvecs;
         // Ritz vector of the current basis (also the restart vector); coefficients past a breakdown are 0
         ritz_vector<<<1, kOneCta, (jdone + 1) * sizeof(double), ctx->stream>>>(m, jdone, v0, b.coef, b.isd, y, b.z);
         SCS_LAUNCHED(ctx, "ritz_vector");

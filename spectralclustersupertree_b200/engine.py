@@ -122,8 +122,9 @@ class Engine:
         """Host wall clock per stage of the staged node path (``scs_ctx_stage_seconds``)."""
         out = np.zeros(8)
         _check(self._lib.scs_ctx_stage_seconds(self._ctx, ptr(out), int(reset)), self._ctx)
-        keys = ("enqueue_graph", "wait_graph", "enqueue_contract", "spectral", "result_copy", "lanczos_in_spectral")
-        return dict(zip(keys, out[:6].tolist(), strict=True))
+        keys = ("enqueue_graph", "wait_graph", "enqueue_contract", "spectral", "result_copy", "lanczos_in_spectral",
+                "tour_components")  # fmt: skip
+        return dict(zip(keys, out[:7].tolist(), strict=True))
 
     def flush_l2(self) -> None:
         _check(self._lib.scs_ctx_flush_l2(self._ctx), self._ctx)
