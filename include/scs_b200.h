@@ -418,6 +418,18 @@ int scs_supertree_support(scs_ctx *ctx, const scs_forest *sources, int64_t num_n
 int scs_supertree_triplets(scs_ctx *ctx, const scs_forest *sources, int64_t num_nodes, const int32_t *parent,
                            const int32_t *taxon, int64_t *per_tree);
 
+/* The same triplets credited to their taxa (validated and failing as scs_supertree_triplets).  For every taxon p,
+ * summed over the source trees t with p in X_t and k = |X_t| >= 3, int64 per_taxon[6 * num_taxa], row p: the number
+ * of such trees, the triplets of X_t that contain p (sum of C(k - 1, 2)), and those of them resolved in the restricted
+ * source tree, resolved in the restricted supertree, resolved the same way in both (agree) and resolved differently
+ * (contradict).  Rows are indexed by the forest's taxon id; taxa that are not tips of the supertree are all zero, and
+ * a tree of one tip adds nothing.  weighted (may be NULL) [3 * num_taxa], row p: resolved source, agree and
+ * contradict summed over the same trees in tree order as acc = acc + w_t * count, without fused multiply-add.
+ * SCS_ERR_INVALID if a leaf of the supertree lies deeper than the three shared-memory arrays of a row allow (about
+ * 19 000 levels).  Returns after the results landed. */
+int scs_supertree_taxon_triplets(scs_ctx *ctx, const scs_forest *sources, int64_t num_nodes, const int32_t *parent,
+                                 const int32_t *taxon, int64_t *per_taxon, double *weighted);
+
 /* ---- one recursion node over several GPUs of one NVLink box (one process per GPU) ------------- *
  * The reference is single-process (scs.py:239 n_jobs=1); this is the B200 answer to its largest
  * recursion nodes.  A node with >= min_n taxa is ROW-SHARDED: rank r builds and keeps rows

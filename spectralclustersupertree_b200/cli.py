@@ -19,20 +19,22 @@ from .load import load_forest
 from .engine import default_engine
 from .scs import flat_newick, supertree_newick_of_forest
 from .support import flat_clade_support
-from .triplets import flat_triplet_fit
+from .triplets import flat_taxon_triplet_fit, flat_triplet_fit
 
 
 def run(in_file: str, out_file: str, weighting: str = "branch", contract_edges: bool = True,
-        support_out: str | None = None, triplets_out: str | None = None) -> None:
+        support_out: str | None = None, triplets_out: str | None = None,
+        taxon_triplets_out: str | None = None) -> None:
     """``load_trees`` + ``construct_supertree`` + ``write`` of the reference's command (ref: cli.py:33-39).  With
     ``support_out`` the supertree is also written there with the V support index of every internal non-root node
     (``support.flat_clade_support``) as its label; with ``triplets_out`` the triplet fit of every source tree
-    (``triplets.flat_triplet_fit``) is written there as TSV.  The supertree is built once either way."""
+    (``triplets.flat_triplet_fit``) is written there as TSV, and with ``taxon_triplets_out`` that of every tip of the
+    supertree (``triplets.flat_taxon_triplet_fit``).  The supertree is built once either way."""
     forest = load_forest(in_file)
     if forest.num_trees == 0:  # what construct_supertree says about an empty list (ref: scs.py:63-65)
         msg = "There must be at least one tree to make a supertree."
         raise ValueError(msg)
-    if support_out is None and triplets_out is None:
+    if support_out is None and triplets_out is None and taxon_triplets_out is None:
         text = supertree_newick_of_forest(forest, weighting.lower(), contract_edges=contract_edges)
         Path(out_file).write_text(text + "\n")
         return
@@ -45,6 +47,9 @@ def run(in_file: str, out_file: str, weighting: str = "branch", contract_edges: 
     if triplets_out is not None:
         fit = flat_triplet_fit(forest, built["parent"], built["taxon"], engine=engine)
         Path(triplets_out).write_text(fit.tsv())
+    if taxon_triplets_out is not None:
+        per_taxon = flat_taxon_triplet_fit(forest, built["parent"], built["taxon"], engine=engine)
+        Path(taxon_triplets_out).write_text(per_taxon.tsv())
 
 
 @click.command(no_args_is_help=True)
@@ -74,6 +79,12 @@ def run(in_file: str, out_file: str, weighting: str = "branch", contract_edges: 
     help="Also write, per source tree, the rooted triplets the supertree agrees with and contradicts (TSV).",
     default=None,
 )
+@click.option(
+    "--taxon-triplets-out",
+    help="Also write, per supertree taxon, the rooted triplets containing it that the source trees agree with and "
+    "contradict (TSV).",
+    default=None,
+)
 def scs(
     in_file: str,
     out_file: str,
@@ -82,10 +93,11 @@ def scs(
     disable_contraction: bool,
     support_out: str | None,
     triplets_out: str | None,
+    taxon_triplets_out: str | None,
 ) -> None:
     """Run spectral cluster supertree over the given set of source trees."""
     run(in_file, out_file, pcg_weighting, contract_edges=not disable_contraction, support_out=support_out,
-        triplets_out=triplets_out)
+        triplets_out=triplets_out, taxon_triplets_out=taxon_triplets_out)
 
 
 if __name__ == "__main__":

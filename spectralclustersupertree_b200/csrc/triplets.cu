@@ -22,8 +22,20 @@
 //
 // Integer counts are exact; every row writes its own partial counts and a second kernel adds a tree's rows in tour
 // order.  Trees are processed in chunks that bound the per-leaf scratch.
+//
+// Per taxon (scs_supertree_taxon_triplets).  Each triplet is also credited to its three taxa.  For a point x of row a
+// let f_alpha(x) / f_beta(x) be the other points y whose alpha / beta differs from x's, and c(x) / d(x) those with
+// (alpha(x) - alpha(y)) (beta(x) - beta(y)) > 0 / < 0.  With R_p the sums over the points of row p and C_p the sums of
+// the values of point p over the other rows of the tree, taxon p has (R_p[f_alpha] / 2 + C_p[f_alpha]) / 2 resolved
+// source triplets, likewise with f_beta resolved supertree triplets and with c agreeing ones, and R_p[d] / 2 + C_p[d]
+// contradicting ones: a resolved or agreeing triplet ab|x is seen from rows a and b and each of its taxa collects it
+// twice (as the row or as one of its pair), a contradicting one is seen from one row and each taxon collects it once.
+// The row warp regrows the window, now with every point's beta known in advance (a histogram over the row), and
+// adds each point's four values into the column of its t' position; the columns go to a [chunk trees x taxa] matrix,
+// which a last kernel adds up per taxon in tree order.
 
 #include <algorithm>
+#include <string>
 #include <vector>
 
 #include "devforest.cuh"
@@ -37,6 +49,7 @@ constexpr int kPrepThreads = 256;
 constexpr int kMaxRowWarps = 8;
 constexpr size_t kScratchBytes = size_t(1024) << 20;         // per-leaf scratch of one chunk
 constexpr size_t kLeafScratch = 3 * sizeof(int32_t) + 4 * sizeof(int64_t);  // qpos, spos, td + four row counts
+constexpr size_t kMatrixBytes = size_t(256) << 20;           // per-taxon counts of one chunk's trees
 
 struct TripletArgs {
     // supertree: taxon -> leaf position (-1 if S lacks it), depth of every leaf, sparse table over the depths of the
@@ -53,8 +66,15 @@ struct TripletArgs {
     int32_t *spos;   // [chunk leaves]: per tree, at its first tour position: S leaf position of t' position q
     int32_t *td;     // [chunk leaves]: per tree, likewise: depth in t of the LCA of t' positions q and q + 1
     int32_t *k;      // [chunk trees]
-    int64_t *rows;   // [chunk leaves][4]: per row a: R1, R2, AG, CO
+    int64_t *rows;   // per tree: [chunk leaves][4]: per row a: R1, R2, AG, CO; per taxon: [4][chunk leaves]: the
+                     // columns of f_alpha, f_beta, c, d at each tree's t' positions, with R / 2 added at the row's own
     int64_t *per_tree;
+    // per taxon
+    const int32_t *s_taxon;  // S leaf position -> taxon
+    const double *weight;    // [trees]
+    int64_t *matrix;         // [chunk trees][4][taxa]: the four counts of every taxon in X_t, -1 for the others
+    int64_t *per_taxon;      // [taxa][6]: trees, triplets, resolved source, resolved supertree, agree, contradict
+    double *weighted;        // [taxa][3]: resolved source, agree, contradict summed with the tree weights
 };
 
 // One CTA per tree: t' positions, the S positions of its taxa and the depths between t'-neighbours.
@@ -92,6 +112,55 @@ __device__ __forceinline__ int s_lca_depth(const TripletArgs &a, int p, int r) {
     return min(__ldg(level + lo), __ldg(level + hi - (1 << l)));
 }
 
+// The tree of chunk tour position g: the last t with leaf_off[t] <= leaf0 + g.
+__device__ __forceinline__ int tree_of(const TripletArgs &a, int64_t g) {
+    int lo = a.t0, hi = a.t1;
+    while (hi - lo > 1) {
+        const int mid = (lo + hi) >> 1;
+        if (a.leaf_off[mid] <= a.leaf0 + g) lo = mid; else hi = mid;
+    }
+    return lo;
+}
+
+// The next depth level of the window [L, R] of t' positions around a (-1 once the window is the whole tree), and the
+// window [nL, nR] grown by it: its new positions are the taxa x with alpha(x) = level.  Called by the whole warp.
+__device__ __forceinline__ int grow_window(const int32_t *td, int k, int lane, int L, int R, int &nL, int &nR) {
+    const int eL = L > 0 ? td[L - 1] : -1, eR = R < k - 1 ? td[R] : -1;
+    const int level = max(eL, eR);
+    nL = L;
+    nR = R;
+    if (level < 0) return level;
+    if (eL == level) {  // q joins while td[q .. L - 1] >= level
+        for (;;) {
+            const int q = nL - 1 - lane;
+            const unsigned bad = __ballot_sync(0xffffffffu, !(q >= 0 && td[q] >= level));
+            const int run = bad ? __ffs(bad) - 1 : 32;
+            nL -= run;
+            if (run < 32) break;
+        }
+    }
+    if (eR == level) {  // q joins while td[R .. q - 1] >= level
+        for (;;) {
+            const int q = nR + 1 + lane;
+            const unsigned bad = __ballot_sync(0xffffffffu, !(q < k && td[q - 1] >= level));
+            const int run = bad ? __ffs(bad) - 1 : 32;
+            nR += run;
+            if (run < 32) break;
+        }
+    }
+    return level;
+}
+
+// Fenwick tree over [1, m] in shared memory: the sum of entries [1, f], and v added at f.
+__device__ __forceinline__ int fenwick_prefix(const int32_t *fw, int f) {
+    int s = 0;
+    for (; f > 0; f -= f & -f) s += fw[f];
+    return s;
+}
+__device__ __forceinline__ void fenwick_add(int32_t *fw, int f, int m, int v) {
+    for (; f <= m; f += f & -f) atomicAdd(&fw[f], v);
+}
+
 // One warp per row: tour position g of the chunk.  Shared memory per warp: Fenwick tree over beta + 1 in [1, m] and
 // a histogram of beta in [0, m), m = depth of a in S (beta < m).
 __global__ void __launch_bounds__(kMaxRowWarps * 32, 1) tp_rows(TripletArgs a, int stride) {
@@ -100,11 +169,7 @@ __global__ void __launch_bounds__(kMaxRowWarps * 32, 1) tp_rows(TripletArgs a, i
     const int64_t g = static_cast<int64_t>(blockIdx.x) * (blockDim.x >> 5) + warp;
     if (g >= a.chunk_leaves) return;
     int64_t *out = a.rows + 4 * g;
-    int lo = a.t0, hi = a.t1;  // the tree of g: the last t with leaf_off[t] <= leaf0 + g
-    while (hi - lo > 1) {
-        const int mid = (lo + hi) >> 1;
-        if (a.leaf_off[mid] <= a.leaf0 + g) lo = mid; else hi = mid;
-    }
+    const int lo = tree_of(a, g);
     const int64_t rel = a.leaf_off[lo] - a.leaf0;
     const int nl = static_cast<int>(a.leaf_off[lo + 1] - a.leaf_off[lo]), j = static_cast<int>(g - rel);
     const int k = a.k[lo - a.t0];
@@ -124,42 +189,21 @@ __global__ void __launch_bounds__(kMaxRowWarps * 32, 1) tp_rows(TripletArgs a, i
     long long r1 = 0, ag = 0, co = 0;
     int L = qa, R = qa, inside = 0;  // t' positions [L, R] are inside the window (a itself is no point)
     for (;;) {
-        const int eL = L > 0 ? td[L - 1] : -1, eR = R < k - 1 ? td[R] : -1;
-        const int level = max(eL, eR);
-        if (level < 0) break;
-        int nL = L, nR = R;
-        if (eL == level) {  // q joins while td[q .. L - 1] >= level
-            for (;;) {
-                const int q = nL - 1 - lane;
-                const unsigned bad = __ballot_sync(0xffffffffu, !(q >= 0 && td[q] >= level));
-                const int run = bad ? __ffs(bad) - 1 : 32;
-                nL -= run;
-                if (run < 32) break;
-            }
-        }
-        if (eR == level) {  // q joins while td[R .. q - 1] >= level
-            for (;;) {
-                const int q = nR + 1 + lane;
-                const unsigned bad = __ballot_sync(0xffffffffu, !(q < k && td[q - 1] >= level));
-                const int run = bad ? __ffs(bad) - 1 : 32;
-                nR += run;
-                if (run < 32) break;
-            }
-        }
+        int nL, nR;
+        if (grow_window(td, k, lane, L, R, nL, nR) < 0) break;
         const int left = L - nL, added = left + nR - R;
         // the new taxa x (alpha(x) = level) against the y inside (alpha(y) > level): concordant when beta(y) >
         // beta(x), discordant when beta(y) < beta(x)
         for (int i = lane; i < added; i += 32) {
             const int b = s_lca_depth(a, pa, sp[i < left ? nL + i : R + 1 + (i - left)]);
-            int below = 0;
-            for (int f = b; f > 0; f -= f & -f) below += fw[f];
+            const int below = fenwick_prefix(fw, b);
             co += below;
             ag += inside - below - hist[b];
         }
         __syncwarp();
         for (int i = lane; i < added; i += 32) {
             const int b = s_lca_depth(a, pa, sp[i < left ? nL + i : R + 1 + (i - left)]);
-            for (int f = b + 1; f <= m; f += f & -f) atomicAdd(&fw[f], 1);
+            fenwick_add(fw, b + 1, m, 1);
             atomicAdd(&hist[b], 1);
         }
         __syncwarp();
@@ -208,6 +252,277 @@ __global__ void tp_reduce(TripletArgs a) {
     }
 }
 
+// One warp per row, for the per-taxon counts.  Every point x gets f_alpha(x), f_beta(x), c(x), d(x) (see the top of
+// the file), added to the column of its t' position; half the row's sums go to the column of a.  Shared memory per
+// warp, three arrays over [0, m]: lt[b] = points with beta < b (from a histogram of the whole row), a Fenwick tree
+// over beta + 1 of the points inside the window (deeper in t than the level being added) and one of that level.
+__global__ void __launch_bounds__(kMaxRowWarps * 32, 1) tx_rows(TripletArgs a, int stride) {
+    extern __shared__ int32_t smem[];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int64_t g = static_cast<int64_t>(blockIdx.x) * (blockDim.x >> 5) + warp;
+    if (g >= a.chunk_leaves) return;
+    const int lo = tree_of(a, g);
+    const int64_t rel = a.leaf_off[lo] - a.leaf0;
+    const int nl = static_cast<int>(a.leaf_off[lo + 1] - a.leaf_off[lo]), j = static_cast<int>(g - rel);
+    const int k = a.k[lo - a.t0];
+    const int32_t *qp = a.qpos + rel;
+    const int qa = qp[j];
+    if (k < 3 || (j + 1 < nl ? qp[j + 1] : k) == qa) return;  // fewer than three shared taxa, or a is not shared
+    const int32_t *sp = a.spos + rel, *td = a.td + rel;
+    const int pa = sp[qa], m = a.leaf_depth[pa];
+    int32_t *lt = smem + warp * 3 * stride, *deep = lt + stride, *lev = deep + stride;
+    for (int i = lane; i <= m; i += 32) lt[i] = deep[i] = lev[i] = 0;
+    __syncwarp();
+    for (int q = lane; q < k; q += 32)
+        if (q != qa) atomicAdd(&lt[s_lca_depth(a, pa, sp[q]) + 1], 1);
+    __syncwarp();
+    for (int base = 0, carry = 0; base <= m; base += 32) {  // inclusive scan of the shifted histogram
+        const int i = base + lane;
+        int v = i <= m ? lt[i] : 0;
+#pragma unroll
+        for (int off = 1; off < 32; off <<= 1) {
+            const int o = __shfl_up_sync(0xffffffffu, v, off);
+            if (lane >= off) v += o;
+        }
+        if (i <= m) lt[i] = carry + v;
+        carry += __shfl_sync(0xffffffffu, v, 31);
+    }
+    __syncwarp();
+
+    unsigned long long *col = reinterpret_cast<unsigned long long *>(a.rows) + rel;
+    const int64_t cs = a.chunk_leaves;
+    long long s_fa = 0, s_fb = 0, s_c = 0, s_d = 0;
+    int L = qa, R = qa, inside = 0;
+    for (;;) {
+        int nL, nR;
+        if (grow_window(td, k, lane, L, R, nL, nR) < 0) break;
+        const int left = L - nL, added = left + nR - R;
+        auto point = [&](int i) { return i < left ? nL + i : R + 1 + (i - left); };
+        for (int i = lane; i < added; i += 32) fenwick_add(lev, s_lca_depth(a, pa, sp[point(i)]) + 1, m, 1);
+        __syncwarp();
+        for (int i = lane; i < added; i += 32) {
+            const int q = point(i), b = s_lca_depth(a, pa, sp[q]);
+            // the other points with beta below / above x's: all of them, those inside (deeper), those of the level
+            const int lt_all = lt[b], gt_all = k - 1 - lt[b + 1];
+            const int lt_in = fenwick_prefix(deep, b), gt_in = inside - fenwick_prefix(deep, b + 1);
+            const int lt_lv = fenwick_prefix(lev, b), gt_lv = added - fenwick_prefix(lev, b + 1);
+            const int fa = k - 1 - added, fb = k - 1 - (lt[b + 1] - lt[b]);
+            const int c = gt_in + (lt_all - lt_in - lt_lv);  // deeper with beta above, shallower with beta below
+            const int d = lt_in + (gt_all - gt_in - gt_lv);  // deeper with beta below, shallower with beta above
+            atomicAdd(col + q, static_cast<unsigned long long>(fa));
+            atomicAdd(col + cs + q, static_cast<unsigned long long>(fb));
+            atomicAdd(col + 2 * cs + q, static_cast<unsigned long long>(c));
+            atomicAdd(col + 3 * cs + q, static_cast<unsigned long long>(d));
+            s_fa += fa;
+            s_fb += fb;
+            s_c += c;
+            s_d += d;
+        }
+        __syncwarp();
+        for (int i = lane; i < added; i += 32) {
+            const int f = s_lca_depth(a, pa, sp[point(i)]) + 1;
+            fenwick_add(lev, f, m, -1);
+            fenwick_add(deep, f, m, 1);
+        }
+        __syncwarp();
+        inside += added;
+        L = nL;
+        R = nR;
+    }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) {
+        s_fa += __shfl_down_sync(0xffffffffu, s_fa, off);
+        s_fb += __shfl_down_sync(0xffffffffu, s_fb, off);
+        s_c += __shfl_down_sync(0xffffffffu, s_c, off);
+        s_d += __shfl_down_sync(0xffffffffu, s_d, off);
+    }
+    if (lane == 0) {  // every pair of points is in the sums twice
+        atomicAdd(col + qa, static_cast<unsigned long long>(s_fa / 2));
+        atomicAdd(col + cs + qa, static_cast<unsigned long long>(s_fb / 2));
+        atomicAdd(col + 2 * cs + qa, static_cast<unsigned long long>(s_c / 2));
+        atomicAdd(col + 3 * cs + qa, static_cast<unsigned long long>(s_d / 2));
+    }
+}
+
+// One warp per tree of the chunk with at least three shared taxa: its columns as the four counts of each of its taxa,
+// into the tree's rows of the matrix.
+__global__ void tx_tree(TripletArgs a) {
+    const int64_t w = (static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (w >= a.t1 - a.t0) return;
+    const int k = a.k[w];
+    if (k < 3) return;
+    const int64_t rel = a.leaf_off[a.t0 + w] - a.leaf0, cs = a.chunk_leaves, taxa = a.taxa;
+    const int64_t *col = a.rows + rel;
+    const int32_t *sp = a.spos + rel;
+    int64_t *out = a.matrix + w * 4 * taxa;
+    for (int q = lane; q < k; q += 32) {
+        const int x = a.s_taxon[sp[q]];
+        out[x] = col[q] / 2;                       // resolved in t'
+        out[taxa + x] = col[cs + q] / 2;           // resolved in s'
+        out[2 * taxa + x] = col[2 * cs + q] / 2;   // agree
+        out[3 * taxa + x] = col[3 * cs + q];       // contradict
+    }
+}
+
+// One thread per taxon: the chunk's trees in order added to its counts, and to its weighted sums as acc + w * count
+// without contraction, so the sums are those of the same loop on the host.
+__global__ void tx_reduce(TripletArgs a) {
+    const int x = blockIdx.x * blockDim.x + threadIdx.x;
+    if (x >= a.taxa) return;
+    const int64_t taxa = a.taxa;
+    int64_t *cnt = a.per_taxon + 6 * static_cast<int64_t>(x);
+    double *sum = a.weighted + 3 * static_cast<int64_t>(x);
+    long long c[6] = {cnt[0], cnt[1], cnt[2], cnt[3], cnt[4], cnt[5]};
+    double s[3] = {sum[0], sum[1], sum[2]};
+    for (int w = 0; w < a.t1 - a.t0; ++w) {
+        const int64_t *m = a.matrix + w * 4 * taxa + x;
+        const long long rs = m[0];
+        if (rs < 0) continue;  // x is not in X_t, or k < 3
+        const long long k = a.k[w], ag = m[2 * taxa], co = m[3 * taxa];
+        const double wt = a.weight[a.t0 + w];
+        c[0] += 1;
+        c[1] += (k - 1) * (k - 2) / 2;
+        c[2] += rs;
+        c[3] += m[taxa];
+        c[4] += ag;
+        c[5] += co;
+        s[0] = __dadd_rn(s[0], __dmul_rn(wt, static_cast<double>(rs)));
+        s[1] = __dadd_rn(s[1], __dmul_rn(wt, static_cast<double>(ag)));
+        s[2] = __dadd_rn(s[2], __dmul_rn(wt, static_cast<double>(co)));
+    }
+    for (int f = 0; f < 6; ++f) cnt[f] = c[f];
+    for (int f = 0; f < 3; ++f) sum[f] = s[f];
+}
+
+// What both entry points share: the supertree validated and in pre-order, the depth of its leaves and the sparse
+// table over the depths between consecutive leaves, the chunk plan, and on the device the source forest, its tours,
+// those supertree arrays and the per-leaf scratch of a chunk.
+struct TripletPass {
+    PreorderTree s;
+    int taxa = 0, T = 0, stride = 0, warps = 0;
+    size_t row_smem = 0;
+    std::vector<int32_t> leaf_depth, stab;
+    std::vector<int> chunk_begin{0};
+    int64_t most_leaves = 0, most_trees = 0;
+    DevForest forest;
+    DevTours tours;
+    GrowBuf ident, flags, pos, d_leaf_depth, d_stab, qpos, spos, td, kbuf, rows;
+
+    // Host side; returns the failure status (message set) or SCS_OK.  arrays: ints of (max depth + 1) per row warp
+    // in shared memory; tree_bytes: device bytes per tree of a chunk on top of the per-leaf scratch.
+    int prepare(scs_ctx *ctx, const char *name, const scs_forest *sources, int64_t num_nodes, const int32_t *parent,
+                const int32_t *taxon, int arrays, size_t tree_bytes) {
+        taxa = sources->num_taxa;
+        if (preorder_supertree(num_nodes, parent, taxon, taxa, &s))
+            return fail(ctx, SCS_ERR_INPUT, (std::string(name) + ": malformed supertree (parent[i] >= i, a tip without a "
+                                             "taxon of the forest, or a repeated taxon)").c_str());
+        const int n = static_cast<int>(num_nodes), NL = s.leaves;
+        T = sources->num_trees();
+        // depth of every leaf and of the LCA of consecutive leaves: in pre-order the node after a tip hangs off that LCA
+        std::vector<int32_t> depth(static_cast<size_t>(n), 0), adj(static_cast<size_t>(std::max(NL - 1, 1)), 0);
+        leaf_depth.assign(static_cast<size_t>(NL), 0);
+        int max_depth = 0;
+        for (int u = 1; u < n; ++u) depth[u] = depth[s.parent[u]] + 1;
+        for (int u = 0; u < n; ++u) {
+            if (u + 1 < n && s.parent[u + 1] == u) continue;  // not a tip
+            leaf_depth[s.first[u]] = depth[u];
+            max_depth = std::max(max_depth, depth[u]);
+            if (u + 1 < n) adj[s.first[u]] = depth[s.parent[u + 1]];
+        }
+        int levels = 1;
+        while ((int64_t(1) << levels) <= NL - 1) ++levels;
+        stab.assign(static_cast<size_t>(levels) * NL, 0);
+        std::copy(adj.begin(), adj.begin() + std::max(NL - 1, 0), stab.begin());
+        for (int l = 1; l < levels; ++l)
+            for (int i = 0; i + (1 << l) <= NL - 1; ++i)
+                stab[static_cast<size_t>(l) * NL + i] = std::min(stab[static_cast<size_t>(l - 1) * NL + i],
+                                                                 stab[static_cast<size_t>(l - 1) * NL + i + (1 << (l - 1))]);
+        // per row warp: `arrays` arrays of max_depth + 1 ints in shared memory (Fenwick trees, histograms)
+        stride = max_depth + 1;
+        const size_t warp_smem = static_cast<size_t>(arrays) * stride * sizeof(int32_t);
+        warps = static_cast<int>(std::min<size_t>(kMaxRowWarps, ctx->smem_optin / warp_smem));
+        if (warps < 1)
+            return fail(ctx, SCS_ERR_INVALID, (std::string(name) + ": the supertree is too deep for the shared-memory "
+                                               "Fenwick tree of a row").c_str());
+        row_smem = static_cast<size_t>(warps) * warp_smem;
+
+        const std::vector<int64_t> &loff = sources->leaf_offsets;
+        for (int t = 0; t < T;) {
+            const int b = chunk_begin.back();
+            int e = t + 1;
+            while (e < T && static_cast<size_t>(loff[e + 1] - loff[b]) * kLeafScratch <= kScratchBytes &&
+                   static_cast<size_t>(e + 1 - b) * tree_bytes <= kMatrixBytes)
+                ++e;
+            most_leaves = std::max(most_leaves, loff[e] - loff[b]);
+            most_trees = std::max<int64_t>(most_trees, e - b);
+            chunk_begin.push_back(e);
+            t = e;
+        }
+        return SCS_OK;
+    }
+
+    // Uploads and scratch; fills the fields of `args` that do not change from chunk to chunk.
+    int upload(scs_ctx *ctx, const scs_forest *sources, TripletArgs *args) {
+        int rc;
+        if ((rc = devforest_upload(ctx, sources, 0, &forest))) return rc;
+        std::vector<int32_t> identity(static_cast<size_t>(taxa > 0 ? taxa : 1));
+        for (size_t x = 0; x < identity.size(); ++x) identity[x] = static_cast<int32_t>(x);
+        if ((rc = put(ctx, ident, identity.data(), identity.size() * sizeof(int32_t))) ||
+            (rc = put(ctx, pos, s.pos.data(), s.pos.size() * sizeof(int32_t))) ||
+            (rc = put(ctx, d_leaf_depth, leaf_depth.data(), leaf_depth.size() * sizeof(int32_t))) ||
+            (rc = put(ctx, d_stab, stab.data(), stab.size() * sizeof(int32_t))))
+            return rc;
+        if ((rc = grow(ctx, flags, 2 * sizeof(int32_t)))) return rc;
+        SCS_CUDA(ctx, cudaMemsetAsync(flags.ptr, 0, 2 * sizeof(int32_t), ctx->stream));
+        if ((rc = devforest_tours(ctx, forest, 0, ident.as<int32_t>(), &tours, flags.as<int32_t>()))) return rc;
+        const size_t L = static_cast<size_t>(most_leaves) + 1;
+        if ((rc = grow(ctx, qpos, L * 4)) || (rc = grow(ctx, spos, L * 4)) || (rc = grow(ctx, td, L * 4)) ||
+            (rc = grow(ctx, rows, L * 4 * sizeof(int64_t))) || (rc = grow(ctx, kbuf, static_cast<size_t>(most_trees) * 4)))
+            return rc;
+        args->taxa = taxa;
+        args->n_leaves = s.leaves;
+        args->pos = pos.as<int32_t>();
+        args->leaf_depth = d_leaf_depth.as<int32_t>();
+        args->stab = d_stab.as<int32_t>();
+        args->leaf_off = forest.leaf_off.as<int64_t>();
+        args->leaf_taxon = tours.leaf_taxon.as<int32_t>();
+        args->adj_depth = tours.adj_depth.as<int32_t>();
+        args->qpos = qpos.as<int32_t>();
+        args->spos = spos.as<int32_t>();
+        args->td = td.as<int32_t>();
+        args->k = kbuf.as<int32_t>();
+        args->rows = rows.as<int64_t>();
+        return SCS_OK;
+    }
+
+    // Points `args` at chunk c and runs tp_prep on it.
+    int prep_chunk(scs_ctx *ctx, const scs_forest *sources, size_t c, TripletArgs *args) {
+        const std::vector<int64_t> &loff = sources->leaf_offsets;
+        const int b = chunk_begin[c], e = chunk_begin[c + 1];
+        args->t0 = b;
+        args->t1 = e;
+        args->leaf0 = loff[b];
+        args->chunk_leaves = loff[e] - loff[b];
+        tp_prep<<<e - b, kPrepThreads, 0, ctx->stream>>>(*args);
+        SCS_LAUNCHED(ctx, "tp_prep");
+        return SCS_OK;
+    }
+
+    static int put(scs_ctx *ctx, GrowBuf &buf, const void *src, size_t bytes) {
+        int r;
+        if ((r = grow(ctx, buf, bytes))) return r;
+        SCS_CUDA(ctx, cudaMemcpyAsync(buf.ptr, src, bytes, cudaMemcpyHostToDevice, ctx->stream));
+        return SCS_OK;
+    }
+
+    void release_all(scs_ctx *ctx) {
+        forest.free_all(ctx);
+        tours.free_all(ctx);
+        for (GrowBuf *b : {&ident, &flags, &pos, &d_leaf_depth, &d_stab, &qpos, &spos, &td, &kbuf, &rows}) release(ctx, *b);
+    }
+};
+
 }  // namespace
 }  // namespace scs
 
@@ -218,120 +533,28 @@ extern "C" int scs_supertree_triplets(scs_ctx *ctx, const scs_forest *sources, i
     if (!ctx) return SCS_ERR_INVALID;
     if (!sources || !parent || !taxon || !per_tree || num_nodes <= 0 || num_nodes >= (int64_t(1) << 31))
         return fail(ctx, SCS_ERR_INVALID, "scs_supertree_triplets: bad argument");
-    const int taxa = sources->num_taxa;
-    PreorderTree s;
-    if (preorder_supertree(num_nodes, parent, taxon, taxa, &s))
-        return fail(ctx, SCS_ERR_INPUT, "scs_supertree_triplets: malformed supertree (parent[i] >= i, a tip without a "
-                                        "taxon of the forest, or a repeated taxon)");
-    const int n = static_cast<int>(num_nodes), T = sources->num_trees(), NL = s.leaves;
-    // depth of every leaf and of the LCA of consecutive leaves: in pre-order the node after a tip hangs off that LCA
-    std::vector<int32_t> depth(static_cast<size_t>(n), 0), leaf_depth(static_cast<size_t>(NL), 0);
-    std::vector<int32_t> adj(static_cast<size_t>(std::max(NL - 1, 1)), 0);
-    int max_depth = 0;
-    for (int u = 1; u < n; ++u) depth[u] = depth[s.parent[u]] + 1;
-    for (int u = 0; u < n; ++u) {
-        if (u + 1 < n && s.parent[u + 1] == u) continue;  // not a tip
-        leaf_depth[s.first[u]] = depth[u];
-        max_depth = std::max(max_depth, depth[u]);
-        if (u + 1 < n) adj[s.first[u]] = depth[s.parent[u + 1]];
-    }
-    int levels = 1;
-    while ((int64_t(1) << levels) <= NL - 1) ++levels;
-    std::vector<int32_t> stab(static_cast<size_t>(levels) * NL, 0);
-    std::copy(adj.begin(), adj.begin() + std::max(NL - 1, 0), stab.begin());
-    for (int l = 1; l < levels; ++l)
-        for (int i = 0; i + (1 << l) <= NL - 1; ++i)
-            stab[static_cast<size_t>(l) * NL + i] = std::min(stab[static_cast<size_t>(l - 1) * NL + i],
-                                                             stab[static_cast<size_t>(l - 1) * NL + i + (1 << (l - 1))]);
-    // per row warp: a Fenwick tree (max_depth + 1 ints) and a histogram (max_depth ints) in shared memory
-    const int stride = max_depth + 1;
-    const size_t warp_smem = 2 * static_cast<size_t>(stride) * sizeof(int32_t);
-    const int warps = static_cast<int>(std::min<size_t>(kMaxRowWarps, ctx->smem_optin / warp_smem));
-    if (warps < 1)
-        return fail(ctx, SCS_ERR_INVALID, "scs_supertree_triplets: the supertree is too deep for the shared-memory "
-                                          "Fenwick tree of a row");
+    TripletPass p;
+    int rc = p.prepare(ctx, "scs_supertree_triplets", sources, num_nodes, parent, taxon, 2, 0);
+    if (rc) return rc;
+    const int T = p.T, taxa = p.taxa;
     std::fill(per_tree, per_tree + 5 * static_cast<int64_t>(T), 0);
     if (T == 0) return SCS_OK;
 
-    const std::vector<int64_t> &loff = sources->leaf_offsets;
-    std::vector<int> chunk_begin{0};
-    int64_t most_leaves = 0, most_trees = 0;
-    for (int t = 0; t < T;) {
-        const int b = chunk_begin.back();
-        int e = t + 1;
-        while (e < T && static_cast<size_t>(loff[e + 1] - loff[b]) * kLeafScratch <= kScratchBytes) ++e;
-        most_leaves = std::max(most_leaves, loff[e] - loff[b]);
-        most_trees = std::max<int64_t>(most_trees, e - b);
-        chunk_begin.push_back(e);
-        t = e;
-    }
-
-    DevForest forest;
-    DevTours tours;
-    GrowBuf ident, flags, pos, d_leaf_depth, d_stab, qpos, spos, td, kbuf, rows, d_per_tree;
-    auto cleanup = [&] {
-        forest.free_all(ctx);
-        tours.free_all(ctx);
-        for (GrowBuf *b : {&ident, &flags, &pos, &d_leaf_depth, &d_stab, &qpos, &spos, &td, &kbuf, &rows, &d_per_tree})
-            release(ctx, *b);
-        cudaStreamSynchronize(ctx->stream);
-    };
+    GrowBuf d_per_tree;
     auto run = [&]() -> int {
-        int rc;
-        if ((rc = devforest_upload(ctx, sources, 0, &forest))) return rc;
-        std::vector<int32_t> identity(static_cast<size_t>(taxa > 0 ? taxa : 1));
-        for (size_t x = 0; x < identity.size(); ++x) identity[x] = static_cast<int32_t>(x);
-        auto put = [&](GrowBuf &buf, const void *src, size_t bytes) -> int {
-            int r;
-            if ((r = grow(ctx, buf, bytes))) return r;
-            SCS_CUDA(ctx, cudaMemcpyAsync(buf.ptr, src, bytes, cudaMemcpyHostToDevice, ctx->stream));
-            return SCS_OK;
-        };
-        if ((rc = put(ident, identity.data(), identity.size() * sizeof(int32_t))) ||
-            (rc = put(pos, s.pos.data(), s.pos.size() * sizeof(int32_t))) ||
-            (rc = put(d_leaf_depth, leaf_depth.data(), leaf_depth.size() * sizeof(int32_t))) ||
-            (rc = put(d_stab, stab.data(), stab.size() * sizeof(int32_t))))
-            return rc;
-        if ((rc = grow(ctx, flags, 2 * sizeof(int32_t)))) return rc;
-        SCS_CUDA(ctx, cudaMemsetAsync(flags.ptr, 0, 2 * sizeof(int32_t), ctx->stream));
-        if ((rc = devforest_tours(ctx, forest, 0, ident.as<int32_t>(), &tours, flags.as<int32_t>()))) return rc;
-        const size_t L = static_cast<size_t>(most_leaves) + 1;
-        if ((rc = grow(ctx, qpos, L * 4)) || (rc = grow(ctx, spos, L * 4)) || (rc = grow(ctx, td, L * 4)) ||
-            (rc = grow(ctx, rows, L * 4 * sizeof(int64_t))) || (rc = grow(ctx, kbuf, static_cast<size_t>(most_trees) * 4)) ||
-            (rc = grow(ctx, d_per_tree, 5 * static_cast<size_t>(T) * sizeof(int64_t))))
-            return rc;
-        const size_t row_smem = static_cast<size_t>(warps) * warp_smem;
-        if (row_smem > 48 * 1024)
-            SCS_CUDA(ctx, cudaFuncSetAttribute(tp_rows, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(row_smem)));
-
         TripletArgs args{};
-        args.taxa = taxa;
-        args.n_leaves = NL;
-        args.pos = pos.as<int32_t>();
-        args.leaf_depth = d_leaf_depth.as<int32_t>();
-        args.stab = d_stab.as<int32_t>();
-        args.leaf_off = forest.leaf_off.as<int64_t>();
-        args.leaf_taxon = tours.leaf_taxon.as<int32_t>();
-        args.adj_depth = tours.adj_depth.as<int32_t>();
-        args.qpos = qpos.as<int32_t>();
-        args.spos = spos.as<int32_t>();
-        args.td = td.as<int32_t>();
-        args.k = kbuf.as<int32_t>();
-        args.rows = rows.as<int64_t>();
+        if ((rc = p.upload(ctx, sources, &args))) return rc;
+        if ((rc = grow(ctx, d_per_tree, 5 * static_cast<size_t>(T) * sizeof(int64_t)))) return rc;
+        if (p.row_smem > 48 * 1024)
+            SCS_CUDA(ctx, cudaFuncSetAttribute(tp_rows, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(p.row_smem)));
         args.per_tree = d_per_tree.as<int64_t>();
-        for (size_t c = 0; c + 1 < chunk_begin.size(); ++c) {
-            const int b = chunk_begin[c], e = chunk_begin[c + 1];
-            args.t0 = b;
-            args.t1 = e;
-            args.leaf0 = loff[b];
-            args.chunk_leaves = loff[e] - loff[b];
-            tp_prep<<<e - b, kPrepThreads, 0, ctx->stream>>>(args);
-            SCS_LAUNCHED(ctx, "tp_prep");
+        for (size_t c = 0; c + 1 < p.chunk_begin.size(); ++c) {
+            if ((rc = p.prep_chunk(ctx, sources, c, &args))) return rc;
             if (args.chunk_leaves > 0) {
-                tp_rows<<<ceil_div(args.chunk_leaves, warps), warps * 32, row_smem, ctx->stream>>>(args, stride);
+                tp_rows<<<ceil_div(args.chunk_leaves, p.warps), p.warps * 32, p.row_smem, ctx->stream>>>(args, p.stride);
                 SCS_LAUNCHED(ctx, "tp_rows");
             }
-            tp_reduce<<<ceil_div(e - b, 8), 256, 0, ctx->stream>>>(args);
+            tp_reduce<<<ceil_div(args.t1 - args.t0, 8), 256, 0, ctx->stream>>>(args);
             SCS_LAUNCHED(ctx, "tp_reduce");
         }
         const size_t out_bytes = 5 * static_cast<size_t>(T) * sizeof(int64_t);
@@ -343,11 +566,78 @@ extern "C" int scs_supertree_triplets(scs_ctx *ctx, const scs_forest *sources, i
         for (int t = 0; t < T; ++t)
             if (noff[t + 1] - noff[t] == 1) {
                 const int x = sources->taxon[noff[t]];
-                per_tree[5 * static_cast<int64_t>(t)] = x >= 0 && x < taxa && s.pos[x] >= 0;
+                per_tree[5 * static_cast<int64_t>(t)] = x >= 0 && x < taxa && p.s.pos[x] >= 0;
             }
         return SCS_OK;
     };
-    const int rc = run();
-    cleanup();
+    rc = run();
+    p.release_all(ctx);
+    release(ctx, d_per_tree);
+    cudaStreamSynchronize(ctx->stream);
+    return rc;
+}
+
+extern "C" int scs_supertree_taxon_triplets(scs_ctx *ctx, const scs_forest *sources, int64_t num_nodes,
+                                            const int32_t *parent, const int32_t *taxon, int64_t *per_taxon,
+                                            double *weighted) {
+    if (!ctx) return SCS_ERR_INVALID;
+    if (!sources || !parent || !taxon || !per_taxon || num_nodes <= 0 || num_nodes >= (int64_t(1) << 31))
+        return fail(ctx, SCS_ERR_INVALID, "scs_supertree_taxon_triplets: bad argument");
+    const int64_t taxa = sources->num_taxa;
+    TripletPass p;
+    int rc = p.prepare(ctx, "scs_supertree_taxon_triplets", sources, num_nodes, parent, taxon, 3,
+                       4 * static_cast<size_t>(taxa) * sizeof(int64_t));
+    if (rc) return rc;
+    const int T = p.T;
+    std::fill(per_taxon, per_taxon + 6 * taxa, 0);
+    if (weighted) std::fill(weighted, weighted + 3 * taxa, 0.0);
+    if (T == 0 || taxa == 0) return SCS_OK;
+
+    GrowBuf s_taxon, matrix, d_per_taxon, d_weighted;
+    auto run = [&]() -> int {
+        TripletArgs args{};
+        if ((rc = p.upload(ctx, sources, &args))) return rc;
+        std::vector<int32_t> taxon_at(static_cast<size_t>(std::max(p.s.leaves, 1)), 0);
+        for (int64_t x = 0; x < taxa; ++x)
+            if (p.s.pos[x] >= 0) taxon_at[p.s.pos[x]] = static_cast<int32_t>(x);
+        const size_t matrix_bytes = static_cast<size_t>(p.most_trees) * 4 * taxa * sizeof(int64_t);
+        if ((rc = TripletPass::put(ctx, s_taxon, taxon_at.data(), taxon_at.size() * sizeof(int32_t))) ||
+            (rc = grow(ctx, matrix, matrix_bytes)) || (rc = grow(ctx, d_per_taxon, 6 * taxa * sizeof(int64_t))) ||
+            (rc = grow(ctx, d_weighted, 3 * taxa * sizeof(double))))
+            return rc;
+        SCS_CUDA(ctx, cudaMemsetAsync(d_per_taxon.ptr, 0, 6 * taxa * sizeof(int64_t), ctx->stream));
+        SCS_CUDA(ctx, cudaMemsetAsync(d_weighted.ptr, 0, 3 * taxa * sizeof(double), ctx->stream));
+        if (p.row_smem > 48 * 1024)
+            SCS_CUDA(ctx, cudaFuncSetAttribute(tx_rows, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(p.row_smem)));
+        args.s_taxon = s_taxon.as<int32_t>();
+        args.weight = p.forest.weight.as<double>();
+        args.matrix = matrix.as<int64_t>();
+        args.per_taxon = d_per_taxon.as<int64_t>();
+        args.weighted = d_weighted.as<double>();
+        for (size_t c = 0; c + 1 < p.chunk_begin.size(); ++c) {
+            if ((rc = p.prep_chunk(ctx, sources, c, &args))) return rc;
+            const int trees = args.t1 - args.t0;
+            SCS_CUDA(ctx, cudaMemsetAsync(matrix.ptr, 0xff, static_cast<size_t>(trees) * 4 * taxa * sizeof(int64_t), ctx->stream));
+            if (args.chunk_leaves > 0) {
+                SCS_CUDA(ctx, cudaMemsetAsync(p.rows.ptr, 0, 4 * static_cast<size_t>(args.chunk_leaves) * sizeof(int64_t), ctx->stream));
+                tx_rows<<<ceil_div(args.chunk_leaves, p.warps), p.warps * 32, p.row_smem, ctx->stream>>>(args, p.stride);
+                SCS_LAUNCHED(ctx, "tx_rows");
+                tx_tree<<<ceil_div(trees, 8), 256, 0, ctx->stream>>>(args);
+                SCS_LAUNCHED(ctx, "tx_tree");
+            }
+            tx_reduce<<<ceil_div(taxa, 256), 256, 0, ctx->stream>>>(args);
+            SCS_LAUNCHED(ctx, "tx_reduce");
+        }
+        SCS_CUDA(ctx, cudaMemcpyAsync(per_taxon, d_per_taxon.ptr, 6 * taxa * sizeof(int64_t), cudaMemcpyDeviceToHost, ctx->stream));
+        if (weighted)
+            SCS_CUDA(ctx, cudaMemcpyAsync(weighted, d_weighted.ptr, 3 * taxa * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+        SCS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        ctx->d2h_bytes += static_cast<int64_t>(6 * taxa * sizeof(int64_t) + (weighted ? 3 * taxa * sizeof(double) : 0));
+        return SCS_OK;
+    };
+    rc = run();
+    p.release_all(ctx);
+    for (GrowBuf *b : {&s_taxon, &matrix, &d_per_taxon, &d_weighted}) release(ctx, *b);
+    cudaStreamSynchronize(ctx->stream);
     return rc;
 }

@@ -271,6 +271,24 @@ class Engine:
         _check(status, self._ctx)
         return per_tree
 
+    def supertree_taxon_triplets(self, forest: "Forest", parent, taxon) -> tuple[np.ndarray, np.ndarray]:
+        """``scs_supertree_taxon_triplets``: per taxon id of ``forest`` ``[num_taxa, 6]`` (int64): source trees sharing
+        it with at least two other taxa, triplets containing it, and those of them resolved in the restricted source
+        tree, resolved in the restricted supertree, agreeing and contradicting; ``[num_taxa, 3]``: the resolved-source,
+        agreeing and contradicting counts summed with the tree weights in tree order."""
+        parent = np.ascontiguousarray(parent, dtype=np.int32)
+        taxon = np.ascontiguousarray(taxon, dtype=np.int32)
+        n = len(parent)
+        if len(taxon) != n:
+            msg = "parent and taxon must have the same length"
+            raise ValueError(msg)
+        per_taxon = np.zeros((forest.num_taxa, 6), dtype=np.int64)
+        weighted = np.zeros((forest.num_taxa, 3), dtype=np.float64)
+        status = self._lib.scs_supertree_taxon_triplets(self._ctx, forest.handle, n, ptr(parent), ptr(taxon),
+                                                        ptr(per_taxon), ptr(weighted))  # fmt: skip
+        _check(status, self._ctx)
+        return per_taxon, weighted
+
     def _collect_supertree(self, handle, record: bool) -> dict:
         try:
             count = self._lib.scs_supertree_num_nodes(handle)
