@@ -430,6 +430,19 @@ int scs_supertree_triplets(scs_ctx *ctx, const scs_forest *sources, int64_t num_
 int scs_supertree_taxon_triplets(scs_ctx *ctx, const scs_forest *sources, int64_t num_nodes, const int32_t *parent,
                                  const int32_t *taxon, int64_t *per_taxon, double *weighted);
 
+/* MRP (matrix representation with parsimony) score of the same supertree (validated as in scs_supertree_support;
+ * SCS_ERR_INPUT if malformed).  Every non-trivial cluster c (2 <= |c| < k) of source tree t restricted to the k taxa
+ * X_t it shares with the supertree is one binary character: 1 on c, 0 on X_t \ c, missing on the other tips.  Its
+ * length is the minimum number of state changes on the supertree (Fitch/Hartigan; polytomies are hard, unary nodes
+ * pass their child's set up) with an all-0 outgroup above the root.  per_tree[4 * T], int64 per tree: k, characters,
+ * their summed length (steps) and the characters of length 1 (exactly the clusters of the restricted supertree); all
+ * but k are 0 when k < 3.  SCS_ERR_INVALID if a leaf of the supertree lies deeper than the shared-memory stack of a
+ * character allows (about 29 000 levels, as scs_supertree_triplets), or if the supertree has more tips than the
+ * shared-memory bitmap of a tree allows (about 925 000, as scs_supertree_support).  Returns after the results
+ * landed. */
+int scs_supertree_mrp(scs_ctx *ctx, const scs_forest *sources, int64_t num_nodes, const int32_t *parent,
+                      const int32_t *taxon, int64_t *per_tree);
+
 /* ---- one recursion node over several GPUs of one NVLink box (one process per GPU) ------------- *
  * The reference is single-process (scs.py:239 n_jobs=1); this is the B200 answer to its largest
  * recursion nodes.  A node with >= min_n taxa is ROW-SHARDED: rank r builds and keeps rows

@@ -3,7 +3,8 @@
 ``construct_supertree`` and ``load_trees`` keep the reference's signatures
 (ref: src/sc_supertree/__init__.py:6-12); the ``scs`` command lives in ``.cli``.  ``clade_support`` scores a
 supertree against its source trees (per-clade support and conflict, per-tree Robinson-Foulds distance),
-``triplet_fit`` compares their rooted triplets and ``taxon_triplet_fit`` credits those triplets to the taxa.
+``triplet_fit`` compares their rooted triplets, ``taxon_triplet_fit`` credits those triplets to the taxa and
+``mrp_score`` gives the parsimony length of the supertree on the matrix representation of the source trees.
 Importing the package does not touch the GPU; the first ``construct_supertree`` call loads
 ``libscs_b200.so`` and raises if it (or a CUDA device) is missing -- there is no CPU fallback.
 """
@@ -11,9 +12,10 @@ Importing the package does not touch the GPU; the first ``construct_supertree`` 
 __version__ = "2025.12.9+b200.1"
 
 from .load import load_trees  # noqa: E402
+from .mrp import MrpScore, mrp_score  # noqa: E402
 from .scs import construct_supertree  # noqa: E402
 from .support import CladeSupport, clade_support  # noqa: E402
 from .triplets import TaxonTripletFit, TripletFit, taxon_triplet_fit, triplet_fit  # noqa: E402
 
-__all__ = ["CladeSupport", "TaxonTripletFit", "TripletFit", "__version__", "clade_support", "construct_supertree",
-           "load_trees", "taxon_triplet_fit", "triplet_fit"]
+__all__ = ["CladeSupport", "MrpScore", "TaxonTripletFit", "TripletFit", "__version__", "clade_support",
+           "construct_supertree", "load_trees", "mrp_score", "taxon_triplet_fit", "triplet_fit"]

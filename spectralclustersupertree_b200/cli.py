@@ -17,6 +17,7 @@ import click
 from . import __version__
 from .load import load_forest
 from .engine import default_engine
+from .mrp import flat_mrp_score
 from .scs import flat_newick, supertree_newick_of_forest
 from .support import flat_clade_support
 from .triplets import flat_taxon_triplet_fit, flat_triplet_fit
@@ -24,17 +25,18 @@ from .triplets import flat_taxon_triplet_fit, flat_triplet_fit
 
 def run(in_file: str, out_file: str, weighting: str = "branch", contract_edges: bool = True,
         support_out: str | None = None, triplets_out: str | None = None,
-        taxon_triplets_out: str | None = None) -> None:
+        taxon_triplets_out: str | None = None, mrp_out: str | None = None) -> None:
     """``load_trees`` + ``construct_supertree`` + ``write`` of the reference's command (ref: cli.py:33-39).  With
     ``support_out`` the supertree is also written there with the V support index of every internal non-root node
     (``support.flat_clade_support``) as its label; with ``triplets_out`` the triplet fit of every source tree
     (``triplets.flat_triplet_fit``) is written there as TSV, and with ``taxon_triplets_out`` that of every tip of the
-    supertree (``triplets.flat_taxon_triplet_fit``).  The supertree is built once either way."""
+    supertree (``triplets.flat_taxon_triplet_fit``); with ``mrp_out`` the MRP score of every source tree
+    (``mrp.flat_mrp_score``) is written there as TSV.  The supertree is built once either way."""
     forest = load_forest(in_file)
     if forest.num_trees == 0:  # what construct_supertree says about an empty list (ref: scs.py:63-65)
         msg = "There must be at least one tree to make a supertree."
         raise ValueError(msg)
-    if support_out is None and triplets_out is None and taxon_triplets_out is None:
+    if support_out is None and triplets_out is None and taxon_triplets_out is None and mrp_out is None:
         text = supertree_newick_of_forest(forest, weighting.lower(), contract_edges=contract_edges)
         Path(out_file).write_text(text + "\n")
         return
@@ -50,6 +52,9 @@ def run(in_file: str, out_file: str, weighting: str = "branch", contract_edges: 
     if taxon_triplets_out is not None:
         per_taxon = flat_taxon_triplet_fit(forest, built["parent"], built["taxon"], engine=engine)
         Path(taxon_triplets_out).write_text(per_taxon.tsv())
+    if mrp_out is not None:
+        score = flat_mrp_score(forest, built["parent"], built["taxon"], engine=engine)
+        Path(mrp_out).write_text(score.tsv())
 
 
 @click.command(no_args_is_help=True)
@@ -85,6 +90,11 @@ def run(in_file: str, out_file: str, weighting: str = "branch", contract_edges: 
     "contradict (TSV).",
     default=None,
 )
+@click.option(
+    "--mrp-out",
+    help="Also write, per source tree, the parsimony steps its clusters need on the supertree (MRP score, TSV).",
+    default=None,
+)
 def scs(
     in_file: str,
     out_file: str,
@@ -94,10 +104,11 @@ def scs(
     support_out: str | None,
     triplets_out: str | None,
     taxon_triplets_out: str | None,
+    mrp_out: str | None,
 ) -> None:
     """Run spectral cluster supertree over the given set of source trees."""
     run(in_file, out_file, pcg_weighting, contract_edges=not disable_contraction, support_out=support_out,
-        triplets_out=triplets_out, taxon_triplets_out=taxon_triplets_out)
+        triplets_out=triplets_out, taxon_triplets_out=taxon_triplets_out, mrp_out=mrp_out)
 
 
 if __name__ == "__main__":

@@ -1,5 +1,6 @@
 // Pieces shared by the passes that score a supertree against its source trees (support.cu, triplets.cu): the
-// supertree in depth-first pre-order with the leaf range of every node, and a CTA-wide exclusive scan.
+// supertree in depth-first pre-order with the leaf range of every node, a CTA-wide exclusive scan and the rank of a
+// leaf position in a bitmap.
 #pragma once
 
 #include <vector>
@@ -44,6 +45,12 @@ __device__ inline int block_scan(int32_t *data, int n, int32_t *sums) {
     const int total = sums[32];
     __syncthreads();
     return total;
+}
+
+// Rank of bit p among the set bits of a bitmap, given the exclusive prefix of its word popcounts (wpre): how a tree's
+// taxa get their order in S from a bitmap over S's leaf positions.
+__device__ __forceinline__ int bitmap_rank(const uint32_t *bits, const int32_t *wpre, int p) {
+    return wpre[p >> 5] + __popc(bits[p >> 5] & ((1u << (p & 31)) - 1u));
 }
 
 // The supertree in depth-first pre-order (children in index order) with the leaf range of every node.

@@ -86,9 +86,7 @@ __global__ void __launch_bounds__(kThreads) sp_tree(SupportArgs a) {
     for (int w = threadIdx.x; w < a.words; w += blockDim.x) wpre[w] = __popc(bits[w]);
     __syncthreads();
     block_scan(wpre, a.words, sums);
-    auto rank = [&](int p) {
-        return p >= a.n_leaves ? k : wpre[p >> 5] + __popc(bits[p >> 5] & ((1u << (p & 31)) - 1u));
-    };
+    auto rank = [&](int p) { return p >= a.n_leaves ? k : bitmap_rank(bits, wpre, p); };
 
     int32_t *sq = a.sq + rel, *sr = a.sr + rel, *td = a.table + rel;
     for (int j = threadIdx.x; j < nl; j += blockDim.x) {

@@ -33,8 +33,24 @@
 // The row warp regrows the window, now with every point's beta known in advance (a histogram over the row), and
 // adds each point's four values into the column of its t' position; the columns go to a [chunk trees x taxa] matrix,
 // which a last kernel adds up per taxon in tree order.
+//
+// MRP score (scs_supertree_mrp).  Every non-trivial cluster c of t' is a binary character (1 on c, 0 on X_t \ c,
+// missing elsewhere) whose Fitch/Hartigan length on S equals its length on s' (a missing tip changes neither cost nor
+// set at its parent).  The clusters of t' are the windows of t' positions around a gap q that hold every gap with
+// td >= td[q]; gap q names its window's cluster when no gap left of it in the window has the same depth.  s' is the
+// same kind of order: the shared taxa by S leaf position (S-rank r, from a bitmap over S's leaves) and sdep[r] = depth
+// in S of the LCA of ranks r and r + 1.  Write x / y for the children of a node whose set is {0} / {1}: Hartigan's
+// cost m - max(n_0, n_1) is min(x, y) and the set follows the sign of x - y, so a node needs only that difference
+// (its balance), and a child adds one to the cost when it moves the balance towards 0.  Let w be the LCA in s' of the
+// character's taxa: its ancestors each have one child holding the character and the rest all 0, so together with
+// the all-0 outgroup they add 1 exactly when w's set is {1}.  One warp per gap finds the cluster and w's leaf range
+// [lw, rw] with ballots, and one lane runs the stack-based Hartigan pass over that range, the ranks streamed in 32 at
+// a time.  The stack holds (depth, balance) of the open nodes, at most one per level of S, in shared memory: the same
+// two ints per level as the per-tree triplet row.  A character costs O(rw - lw + 1): |c| when S agrees with it, k at
+// worst.
 
 #include <algorithm>
+#include <climits>
 #include <string>
 #include <vector>
 
@@ -75,6 +91,12 @@ struct TripletArgs {
     int64_t *matrix;         // [chunk trees][4][taxa]: the four counts of every taxon in X_t, -1 for the others
     int64_t *per_taxon;      // [taxa][6]: trees, triplets, resolved source, resolved supertree, agree, contradict
     double *weighted;        // [taxa][3]: resolved source, agree, contradict summed with the tree weights
+    // MRP score, per tree at its first tour position (in the scratch of `rows`)
+    int32_t words;           // 32-bit words of a bitmap over S's leaf positions
+    int32_t *sq;             // [chunk leaves]: t' position of the shared taxon of S-rank r
+    int32_t *sr;             // [chunk leaves]: S-rank of t' position q
+    int32_t *sdep;           // [chunk leaves]: depth in S of the LCA of S-ranks r and r + 1
+    int32_t *len;            // [chunk leaves]: length of the character of gap q, 0 if gap q names no character
 };
 
 // One CTA per tree: t' positions, the S positions of its taxa and the depths between t'-neighbours.
@@ -395,6 +417,183 @@ __global__ void tx_reduce(TripletArgs a) {
     for (int f = 0; f < 3; ++f) sum[f] = s[f];
 }
 
+// One CTA per tree with at least three shared taxa: S-ranks of its taxa and the depths between S-rank neighbours.
+// Shared memory: a bitmap over S's leaf positions and the exclusive prefix of its word popcounts.
+__global__ void __launch_bounds__(kPrepThreads) mp_rank(TripletArgs a) {
+    extern __shared__ uint32_t bits[];
+    int32_t *wpre = reinterpret_cast<int32_t *>(bits + a.words);
+    __shared__ int32_t sums[33];
+    const int w = blockIdx.x;
+    const int k = a.k[w];
+    if (k < 3) return;
+    const int64_t rel = a.leaf_off[a.t0 + w] - a.leaf0;
+    const int32_t *sp = a.spos + rel;
+    int32_t *sq = a.sq + rel, *sr = a.sr + rel, *sd = a.sdep + rel;
+    for (int i = threadIdx.x; i < a.words; i += blockDim.x) bits[i] = 0;
+    __syncthreads();
+    for (int q = threadIdx.x; q < k; q += blockDim.x) atomicOr(&bits[sp[q] >> 5], 1u << (sp[q] & 31));
+    __syncthreads();
+    for (int i = threadIdx.x; i < a.words; i += blockDim.x) wpre[i] = __popc(bits[i]);
+    __syncthreads();
+    block_scan(wpre, a.words, sums);
+    for (int q = threadIdx.x; q < k; q += blockDim.x) {
+        const int r = bitmap_rank(bits, wpre, sp[q]);
+        sq[r] = q;
+        sr[q] = r;
+    }
+    __syncthreads();
+    for (int r = threadIdx.x; r < k - 1; r += blockDim.x) sd[r] = s_lca_depth(a, sp[sq[r]], sp[sq[r + 1]]);
+}
+
+// Hartigan: child of sign s (+1 set {0}, -1 set {1}, 0 set {0, 1}) added to a node of balance bal; returns the cost.
+__device__ __forceinline__ int mp_attach(int &bal, int s) {
+    const int cost = (s > 0 && bal < 0) || (s < 0 && bal > 0);
+    bal += s;
+    return cost;
+}
+
+// One warp per tour position of the chunk, for the gap q between t' positions q and q + 1 of its taxon: the length
+// of the character that gap names, or 0.  Shared memory per warp: the stack of (depth, balance) of `stride` levels.
+__global__ void __launch_bounds__(kMaxRowWarps * 32, 1) mp_chars(TripletArgs a, int stride) {
+    extern __shared__ int32_t smem[];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int64_t g = static_cast<int64_t>(blockIdx.x) * (blockDim.x >> 5) + warp;
+    if (g >= a.chunk_leaves) return;
+    const int lo_t = tree_of(a, g);
+    const int64_t rel = a.leaf_off[lo_t] - a.leaf0;
+    const int nl = static_cast<int>(a.leaf_off[lo_t + 1] - a.leaf_off[lo_t]), j = static_cast<int>(g - rel);
+    const int k = a.k[lo_t - a.t0];
+    const int32_t *qp = a.qpos + rel;
+    const int q = qp[j];
+    if (k < 3 || (j + 1 < nl ? qp[j + 1] : k) == q || q >= k - 1) return;  // no gap of a tree with characters
+    const int32_t *td = a.td + rel, *sq = a.sq + rel, *sr = a.sr + rel, *sd = a.sdep + rel;
+    int32_t *len = a.len + rel;
+    const unsigned full = 0xffffffffu;
+    const int d = td[q];
+    // the cluster: t' positions [lo, hi] around gap q with every gap inside at depth >= d
+    int lo = q;
+    for (;;) {
+        const int i = lo - 1 - lane;
+        const unsigned stop = __ballot_sync(full, i < 0 || td[i] <= d);
+        if (!stop) {
+            lo -= 32;
+            continue;
+        }
+        const int i0 = lo - __ffs(stop);
+        if (i0 >= 0 && td[i0] == d) {  // an earlier gap of the same node names it
+            if (lane == 0) len[q] = 0;
+            return;
+        }
+        lo = i0 + 1;
+        break;
+    }
+    int hi = q + 1;
+    for (;;) {
+        const int i = hi + lane;
+        const unsigned stop = __ballot_sync(full, i >= k - 1 || td[i] < d);
+        if (stop) {
+            hi += __ffs(stop) - 1;
+            break;
+        }
+        hi += 32;
+    }
+    if (lo == 0 && hi == k - 1) {  // X_t itself
+        if (lane == 0) len[q] = 0;
+        return;
+    }
+    // the S-ranks of the character's taxa, and w = their LCA in s': its depth dw and leaf range [lw, rw]
+    int rmin = INT_MAX, rmax = -1;
+    for (int i = lo + lane; i <= hi; i += 32) {
+        const int r = sr[i];
+        rmin = min(rmin, r);
+        rmax = max(rmax, r);
+    }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) {
+        rmin = min(rmin, __shfl_xor_sync(full, rmin, off));
+        rmax = max(rmax, __shfl_xor_sync(full, rmax, off));
+    }
+    int dw = INT_MAX;
+    for (int r = rmin + lane; r < rmax; r += 32) dw = min(dw, sd[r]);
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) dw = min(dw, __shfl_xor_sync(full, dw, off));
+    int lw = rmin;
+    for (;;) {
+        const int i = lw - 1 - lane;
+        const unsigned stop = __ballot_sync(full, i < 0 || sd[i] < dw);
+        if (stop) {
+            lw -= __ffs(stop) - 1;
+            break;
+        }
+        lw -= 32;
+    }
+    int rw = rmax;
+    for (;;) {
+        const int i = rw + lane;
+        const unsigned stop = __ballot_sync(full, i >= k - 1 || sd[i] < dw);
+        if (stop) {
+            rw += __ffs(stop) - 1;
+            break;
+        }
+        rw += 32;
+    }
+    // Hartigan over the leaves [lw, rw] of w, left to right: leaf r, then the gap after it closes the open nodes
+    // deeper than it and joins or opens the node at its depth; the gap after rw closes them all
+    int2 *stk = reinterpret_cast<int2 *>(smem) + static_cast<int64_t>(warp) * stride;
+    int top = -1, cost = 0, cur = 0;
+    for (int base = lw; base <= rw; base += 32) {
+        const int r = base + lane;
+        int dep = -1, one = 0;
+        if (r <= rw) {
+            const int qr = sq[r];
+            one = qr >= lo && qr <= hi;
+            if (r < rw) dep = sd[r];
+        }
+        const int n = min(32, rw - base + 1);
+        for (int i = 0; i < n; ++i) {
+            const int dg = __shfl_sync(full, dep, i), s1 = __shfl_sync(full, one, i);
+            if (lane != 0) continue;
+            cur = s1 ? -1 : 1;
+            while (top >= 0 && stk[top].x > dg) {
+                cost += mp_attach(stk[top].y, cur);
+                cur = (stk[top].y > 0) - (stk[top].y < 0);
+                --top;
+            }
+            if (dg < 0) break;  // past rw: cur is w's sign
+            if (top < 0 || stk[top].x < dg) stk[++top] = make_int2(dg, 0);
+            cost += mp_attach(stk[top].y, cur);
+        }
+    }
+    if (lane == 0) len[q] = cost + (cur < 0);
+}
+
+// One warp per tree of the chunk: k, and over its gaps the characters, their summed length and those of length 1.
+__global__ void mp_reduce(TripletArgs a) {
+    const int64_t w = (static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (w >= a.t1 - a.t0) return;
+    const int k = a.k[w];
+    const int32_t *len = a.len + (a.leaf_off[a.t0 + w] - a.leaf0);
+    long long s[3] = {0, 0, 0};
+    if (k >= 3)
+        for (int q = lane; q < k - 1; q += 32) {
+            const int l = len[q];
+            s[0] += l > 0;
+            s[1] += l;
+            s[2] += l == 1;
+        }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1)
+        for (int c = 0; c < 3; ++c) s[c] += __shfl_down_sync(0xffffffffu, s[c], off);
+    if (lane == 0) {
+        int64_t *o = a.per_tree + 4 * static_cast<int64_t>(a.t0 + w);
+        o[0] = k;
+        o[1] = s[0];
+        o[2] = s[1];
+        o[3] = s[2];
+    }
+}
+
 // What both entry points share: the supertree validated and in pre-order, the depth of its leaves and the sparse
 // table over the depths between consecutive leaves, the chunk plan, and on the device the source forest, its tours,
 // those supertree arrays and the per-leaf scratch of a chunk.
@@ -410,9 +609,11 @@ struct TripletPass {
     GrowBuf ident, flags, pos, d_leaf_depth, d_stab, qpos, spos, td, kbuf, rows;
 
     // Host side; returns the failure status (message set) or SCS_OK.  arrays: ints of (max depth + 1) per row warp
-    // in shared memory; tree_bytes: device bytes per tree of a chunk on top of the per-leaf scratch.
+    // in shared memory, which `what` names in the message for a supertree too deep for them; tree_bytes: device bytes
+    // per tree of a chunk on top of the per-leaf scratch.
     int prepare(scs_ctx *ctx, const char *name, const scs_forest *sources, int64_t num_nodes, const int32_t *parent,
-                const int32_t *taxon, int arrays, size_t tree_bytes) {
+                const int32_t *taxon, int arrays, size_t tree_bytes,
+                const char *what = "the shared-memory Fenwick tree of a row") {
         taxa = sources->num_taxa;
         if (preorder_supertree(num_nodes, parent, taxon, taxa, &s))
             return fail(ctx, SCS_ERR_INPUT, (std::string(name) + ": malformed supertree (parent[i] >= i, a tip without a "
@@ -443,8 +644,7 @@ struct TripletPass {
         const size_t warp_smem = static_cast<size_t>(arrays) * stride * sizeof(int32_t);
         warps = static_cast<int>(std::min<size_t>(kMaxRowWarps, ctx->smem_optin / warp_smem));
         if (warps < 1)
-            return fail(ctx, SCS_ERR_INVALID, (std::string(name) + ": the supertree is too deep for the shared-memory "
-                                               "Fenwick tree of a row").c_str());
+            return fail(ctx, SCS_ERR_INVALID, (std::string(name) + ": the supertree is too deep for " + what).c_str());
         row_smem = static_cast<size_t>(warps) * warp_smem;
 
         const std::vector<int64_t> &loff = sources->leaf_offsets;
@@ -638,6 +838,72 @@ extern "C" int scs_supertree_taxon_triplets(scs_ctx *ctx, const scs_forest *sour
     rc = run();
     p.release_all(ctx);
     for (GrowBuf *b : {&s_taxon, &matrix, &d_per_taxon, &d_weighted}) release(ctx, *b);
+    cudaStreamSynchronize(ctx->stream);
+    return rc;
+}
+
+extern "C" int scs_supertree_mrp(scs_ctx *ctx, const scs_forest *sources, int64_t num_nodes, const int32_t *parent,
+                                 const int32_t *taxon, int64_t *per_tree) {
+    if (!ctx) return SCS_ERR_INVALID;
+    if (!sources || !parent || !taxon || !per_tree || num_nodes <= 0 || num_nodes >= (int64_t(1) << 31))
+        return fail(ctx, SCS_ERR_INVALID, "scs_supertree_mrp: bad argument");
+    TripletPass p;
+    int rc = p.prepare(ctx, "scs_supertree_mrp", sources, num_nodes, parent, taxon, 2, 0,
+                       "the shared-memory stack of a character");
+    if (rc) return rc;
+    const int T = p.T, taxa = p.taxa;
+    const int words = (p.s.leaves + 31) / 32;
+    const size_t rank_smem = static_cast<size_t>(words) * 8;
+    if (rank_smem + 1024 > ctx->smem_optin)  // room for the static shared arrays
+        return fail(ctx, SCS_ERR_INVALID, "scs_supertree_mrp: the supertree has too many tips for the shared-memory bitmap");
+    std::fill(per_tree, per_tree + 4 * static_cast<int64_t>(T), 0);
+    if (T == 0) return SCS_OK;
+
+    GrowBuf d_per_tree;
+    auto run = [&]() -> int {
+        TripletArgs args{};
+        if ((rc = p.upload(ctx, sources, &args))) return rc;
+        if ((rc = grow(ctx, d_per_tree, 4 * static_cast<size_t>(T) * sizeof(int64_t)))) return rc;
+        if (p.row_smem > 48 * 1024)
+            SCS_CUDA(ctx, cudaFuncSetAttribute(mp_chars, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(p.row_smem)));
+        if (rank_smem > 48 * 1024)
+            SCS_CUDA(ctx, cudaFuncSetAttribute(mp_rank, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(rank_smem)));
+        // four ints per tour position in the scratch of the triplet rows
+        const int64_t L = p.most_leaves + 1;
+        int32_t *scratch = p.rows.as<int32_t>();
+        args.words = words;
+        args.sq = scratch;
+        args.sr = scratch + L;
+        args.sdep = scratch + 2 * L;
+        args.len = scratch + 3 * L;
+        args.per_tree = d_per_tree.as<int64_t>();
+        for (size_t c = 0; c + 1 < p.chunk_begin.size(); ++c) {
+            if ((rc = p.prep_chunk(ctx, sources, c, &args))) return rc;
+            if (args.chunk_leaves > 0) {
+                mp_rank<<<args.t1 - args.t0, kPrepThreads, rank_smem, ctx->stream>>>(args);
+                SCS_LAUNCHED(ctx, "mp_rank");
+                mp_chars<<<ceil_div(args.chunk_leaves, p.warps), p.warps * 32, p.row_smem, ctx->stream>>>(args, p.stride);
+                SCS_LAUNCHED(ctx, "mp_chars");
+            }
+            mp_reduce<<<ceil_div(args.t1 - args.t0, 8), 256, 0, ctx->stream>>>(args);
+            SCS_LAUNCHED(ctx, "mp_reduce");
+        }
+        const size_t out_bytes = 4 * static_cast<size_t>(T) * sizeof(int64_t);
+        SCS_CUDA(ctx, cudaMemcpyAsync(per_tree, d_per_tree.ptr, out_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+        SCS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        ctx->d2h_bytes += static_cast<int64_t>(out_bytes);
+        // a lone tip has no tour: it shares one taxon with S or none
+        const std::vector<int64_t> &noff = sources->node_offsets;
+        for (int t = 0; t < T; ++t)
+            if (noff[t + 1] - noff[t] == 1) {
+                const int x = sources->taxon[noff[t]];
+                per_tree[4 * static_cast<int64_t>(t)] = x >= 0 && x < taxa && p.s.pos[x] >= 0;
+            }
+        return SCS_OK;
+    };
+    rc = run();
+    p.release_all(ctx);
+    release(ctx, d_per_tree);
     cudaStreamSynchronize(ctx->stream);
     return rc;
 }

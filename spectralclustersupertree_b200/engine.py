@@ -289,6 +289,21 @@ class Engine:
         _check(status, self._ctx)
         return per_taxon, weighted
 
+    def supertree_mrp(self, forest: "Forest", parent, taxon) -> np.ndarray:
+        """``scs_supertree_mrp``: per source tree ``[T, 4]`` (int64): shared taxa, MRP characters (the non-trivial
+        clusters of the restricted source tree), their summed parsimony length on the supertree (steps), and the
+        characters of length 1."""
+        parent = np.ascontiguousarray(parent, dtype=np.int32)
+        taxon = np.ascontiguousarray(taxon, dtype=np.int32)
+        n = len(parent)
+        if len(taxon) != n:
+            msg = "parent and taxon must have the same length"
+            raise ValueError(msg)
+        per_tree = np.zeros((forest.num_trees, 4), dtype=np.int64)
+        status = self._lib.scs_supertree_mrp(self._ctx, forest.handle, n, ptr(parent), ptr(taxon), ptr(per_tree))
+        _check(status, self._ctx)
+        return per_tree
+
     def _collect_supertree(self, handle, record: bool) -> dict:
         try:
             count = self._lib.scs_supertree_num_nodes(handle)
