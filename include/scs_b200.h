@@ -443,6 +443,19 @@ int scs_supertree_taxon_triplets(scs_ctx *ctx, const scs_forest *sources, int64_
 int scs_supertree_mrp(scs_ctx *ctx, const scs_forest *sources, int64_t num_nodes, const int32_t *parent,
                       const int32_t *taxon, int64_t *per_tree);
 
+/* Rooted Robinson-Foulds distances between every pair of source trees of the forest, each pair restricted to the k
+ * taxa X it shares (as scs_forest_induce restricts; no supertree is involved).  Three caller-owned T x T row-major
+ * int32 arrays: shared_taxa[i][j] = k (symmetric; the diagonal is the tree's tip count); clusters[i][j] = the
+ * non-trivial clusters (2 <= |c| < k) of tree i restricted to X (not symmetric: row i counts tree i's clusters); common
+ * = the clusters the two restrictions have in common (symmetric).  clusters and common are 0 where k < 3.  The rooted
+ * RF distance is clusters[i][j] + clusters[j][i] - 2 common[i][j]; with tree i as the supertree, scs_supertree_support
+ * gives for source tree j: shared clusters = common[i][j], source clusters = clusters[j][i], supertree clusters =
+ * clusters[i][j].  Tree weights do not enter.  SCS_ERR_INVALID if the forest has more taxa than the shared-memory
+ * bitmap of a pair allows (about 925 000) or more trees than the grid of 64 x 64 pair tiles allows (about 4 million).
+ * Returns after the results landed. */
+int scs_forest_pairwise_rf(scs_ctx *ctx, const scs_forest *forest, int32_t *shared_taxa, int32_t *clusters,
+                           int32_t *common);
+
 /* ---- one recursion node over several GPUs of one NVLink box (one process per GPU) ------------- *
  * The reference is single-process (scs.py:239 n_jobs=1); this is the B200 answer to its largest
  * recursion nodes.  A node with >= min_n taxa is ROW-SHARDED: rank r builds and keeps rows

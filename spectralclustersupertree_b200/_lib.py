@@ -124,6 +124,7 @@ SIGNATURES: dict[str, tuple] = {
     "scs_supertree_triplets": (c_int, [_P, _P, c_int64, _P, _P, _P]),
     "scs_supertree_taxon_triplets": (c_int, [_P, _P, c_int64, _P, _P, _P, _P]),
     "scs_supertree_mrp": (c_int, [_P, _P, c_int64, _P, _P, _P]),
+    "scs_forest_pairwise_rf": (c_int, [_P, _P, _P, _P, _P]),
     "scs_profiler_range": (c_int, [c_int]),
     "scs_debug_small_cycles": (c_int, [_P, _P, c_int]),
     "scs_free": (None, [_P]),

@@ -15,6 +15,7 @@ from typing import Literal
 import click
 
 from . import __version__
+from .distances import flat_source_tree_distances
 from .load import load_forest
 from .engine import default_engine
 from .mrp import flat_mrp_score
@@ -25,18 +26,22 @@ from .triplets import flat_taxon_triplet_fit, flat_triplet_fit
 
 def run(in_file: str, out_file: str, weighting: str = "branch", contract_edges: bool = True,
         support_out: str | None = None, triplets_out: str | None = None,
-        taxon_triplets_out: str | None = None, mrp_out: str | None = None) -> None:
+        taxon_triplets_out: str | None = None, mrp_out: str | None = None,
+        source_rf_out: str | None = None) -> None:
     """``load_trees`` + ``construct_supertree`` + ``write`` of the reference's command (ref: cli.py:33-39).  With
     ``support_out`` the supertree is also written there with the V support index of every internal non-root node
     (``support.flat_clade_support``) as its label; with ``triplets_out`` the triplet fit of every source tree
     (``triplets.flat_triplet_fit``) is written there as TSV, and with ``taxon_triplets_out`` that of every tip of the
     supertree (``triplets.flat_taxon_triplet_fit``); with ``mrp_out`` the MRP score of every source tree
-    (``mrp.flat_mrp_score``) is written there as TSV.  The supertree is built once either way."""
+    (``mrp.flat_mrp_score``) is written there as TSV; with ``source_rf_out`` the Robinson-Foulds distance of every pair
+    of source trees that share at least three taxa (``distances.flat_source_tree_distances``) is written there as
+    TSV.  The supertree is built once either way."""
     forest = load_forest(in_file)
     if forest.num_trees == 0:  # what construct_supertree says about an empty list (ref: scs.py:63-65)
         msg = "There must be at least one tree to make a supertree."
         raise ValueError(msg)
-    if support_out is None and triplets_out is None and taxon_triplets_out is None and mrp_out is None:
+    extras = (support_out, triplets_out, taxon_triplets_out, mrp_out, source_rf_out)
+    if all(path is None for path in extras):
         text = supertree_newick_of_forest(forest, weighting.lower(), contract_edges=contract_edges)
         Path(out_file).write_text(text + "\n")
         return
@@ -55,6 +60,9 @@ def run(in_file: str, out_file: str, weighting: str = "branch", contract_edges: 
     if mrp_out is not None:
         score = flat_mrp_score(forest, built["parent"], built["taxon"], engine=engine)
         Path(mrp_out).write_text(score.tsv())
+    if source_rf_out is not None:
+        distances = flat_source_tree_distances(forest, engine=engine)
+        Path(source_rf_out).write_text(distances.tsv())
 
 
 @click.command(no_args_is_help=True)
@@ -95,6 +103,12 @@ def run(in_file: str, out_file: str, weighting: str = "branch", contract_edges: 
     help="Also write, per source tree, the parsimony steps its clusters need on the supertree (MRP score, TSV).",
     default=None,
 )
+@click.option(
+    "--source-rf-out",
+    help="Also write the rooted Robinson-Foulds distance between every pair of source trees on the taxa they share "
+    "(TSV).",
+    default=None,
+)
 def scs(
     in_file: str,
     out_file: str,
@@ -105,10 +119,12 @@ def scs(
     triplets_out: str | None,
     taxon_triplets_out: str | None,
     mrp_out: str | None,
+    source_rf_out: str | None,
 ) -> None:
     """Run spectral cluster supertree over the given set of source trees."""
     run(in_file, out_file, pcg_weighting, contract_edges=not disable_contraction, support_out=support_out,
-        triplets_out=triplets_out, taxon_triplets_out=taxon_triplets_out, mrp_out=mrp_out)
+        triplets_out=triplets_out, taxon_triplets_out=taxon_triplets_out, mrp_out=mrp_out,
+        source_rf_out=source_rf_out)
 
 
 if __name__ == "__main__":

@@ -304,6 +304,18 @@ class Engine:
         _check(status, self._ctx)
         return per_tree
 
+    def forest_pairwise_rf(self, forest: "Forest") -> tuple[np.ndarray, np.ndarray, np.ndarray]:
+        """``scs_forest_pairwise_rf``: for every pair of source trees, restricted to the taxa they share, three
+        ``[T, T]`` int32 matrices: the shared taxa, the non-trivial clusters of row tree i's restriction (not
+        symmetric) and the clusters the two restrictions have in common."""
+        T = forest.num_trees
+        shared = np.zeros((T, T), dtype=np.int32)
+        clusters = np.zeros((T, T), dtype=np.int32)
+        common = np.zeros((T, T), dtype=np.int32)
+        status = self._lib.scs_forest_pairwise_rf(self._ctx, forest.handle, ptr(shared), ptr(clusters), ptr(common))
+        _check(status, self._ctx)
+        return shared, clusters, common
+
     def _collect_supertree(self, handle, record: bool) -> dict:
         try:
             count = self._lib.scs_supertree_num_nodes(handle)
