@@ -456,6 +456,22 @@ int scs_supertree_mrp(scs_ctx *ctx, const scs_forest *sources, int64_t num_nodes
 int scs_forest_pairwise_rf(scs_ctx *ctx, const scs_forest *forest, int32_t *shared_taxa, int32_t *clusters,
                            int32_t *common);
 
+/* Rooted triplet distances between every pair of source trees of the forest, each pair restricted to the k taxa X it
+ * shares (as scs_forest_pairwise_rf restricts).  A triplet {a, b, c} of X is resolved as ab|c in a restricted tree
+ * when LCA(a, b) lies strictly below LCA(a, b, c), a fan otherwise.  Caller-owned T x T row-major arrays:
+ * shared_taxa[i][j] = k (int32, the same matrix as scs_forest_pairwise_rf); int64 resolved[i][j] = the triplets of X
+ * resolved in tree i restricted to X (not symmetric: row i counts tree i); agree = those resolved the same way in both
+ * restrictions and contradict = those resolved in both but differently (both symmetric).  All three are 0 where
+ * k < 3; the diagonal has resolved = agree and contradict = 0.  The triplet distance is resolved[i][j] +
+ * resolved[j][i] - 2 agree[i][j] - contradict[i][j]; with tree i as the supertree, scs_supertree_triplets gives for
+ * source tree j: shared = shared_taxa[i][j], resolved source = resolved[j][i], resolved supertree = resolved[i][j],
+ * agree = agree[i][j], contradict = contradict[i][j].  Tree weights do not enter.  SCS_ERR_INVALID if a tip of a tree
+ * lies deeper than the shared-memory Fenwick tree of a row allows (about 29 000 levels, as scs_supertree_triplets),
+ * or for the taxa and tree limits of scs_forest_pairwise_rf; all are checked before anything runs on the device.
+ * Returns after the results landed. */
+int scs_forest_pairwise_triplets(scs_ctx *ctx, const scs_forest *forest, int32_t *shared_taxa, int64_t *resolved,
+                                 int64_t *agree, int64_t *contradict);
+
 /* ---- one recursion node over several GPUs of one NVLink box (one process per GPU) ------------- *
  * The reference is single-process (scs.py:239 n_jobs=1); this is the B200 answer to its largest
  * recursion nodes.  A node with >= min_n taxa is ROW-SHARDED: rank r builds and keeps rows

@@ -20,7 +20,7 @@ INCLUDE = PKG.parent / "include"
 LIB = PKG / "libscs_b200.so"
 
 SOURCES = ["context.cu", "pcg.cu", "components.cu", "contract.cu", "spectral.cu", "medium.cu", "small.cu", "shard.cu", "driver.cu", "devforest.cu", "devdriver.cu", "support.cu", "triplets.cu", "pairwise.cu", "forest.cpp", "newick.cpp"]
-HEADERS = ["common.cuh", "shard.cuh", "forest.hpp", "spectral_dev.cuh", "uf.cuh", "devforest.cuh", "driver.hpp", "supertree.cuh"]
+HEADERS = ["common.cuh", "shard.cuh", "forest.hpp", "spectral_dev.cuh", "uf.cuh", "devforest.cuh", "driver.hpp", "supertree.cuh", "dominance.cuh"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-std=c++17", "-lineinfo",

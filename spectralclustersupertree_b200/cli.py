@@ -15,7 +15,7 @@ from typing import Literal
 import click
 
 from . import __version__
-from .distances import flat_source_tree_distances
+from .distances import flat_source_tree_distances, flat_source_tree_triplet_distances
 from .load import load_forest
 from .engine import default_engine
 from .mrp import flat_mrp_score
@@ -27,7 +27,7 @@ from .triplets import flat_taxon_triplet_fit, flat_triplet_fit
 def run(in_file: str, out_file: str, weighting: str = "branch", contract_edges: bool = True,
         support_out: str | None = None, triplets_out: str | None = None,
         taxon_triplets_out: str | None = None, mrp_out: str | None = None,
-        source_rf_out: str | None = None) -> None:
+        source_rf_out: str | None = None, source_triplets_out: str | None = None) -> None:
     """``load_trees`` + ``construct_supertree`` + ``write`` of the reference's command (ref: cli.py:33-39).  With
     ``support_out`` the supertree is also written there with the V support index of every internal non-root node
     (``support.flat_clade_support``) as its label; with ``triplets_out`` the triplet fit of every source tree
@@ -35,12 +35,13 @@ def run(in_file: str, out_file: str, weighting: str = "branch", contract_edges: 
     supertree (``triplets.flat_taxon_triplet_fit``); with ``mrp_out`` the MRP score of every source tree
     (``mrp.flat_mrp_score``) is written there as TSV; with ``source_rf_out`` the Robinson-Foulds distance of every pair
     of source trees that share at least three taxa (``distances.flat_source_tree_distances``) is written there as
-    TSV.  The supertree is built once either way."""
+    TSV, and with ``source_triplets_out`` their rooted triplet distance
+    (``distances.flat_source_tree_triplet_distances``).  The supertree is built once either way."""
     forest = load_forest(in_file)
     if forest.num_trees == 0:  # what construct_supertree says about an empty list (ref: scs.py:63-65)
         msg = "There must be at least one tree to make a supertree."
         raise ValueError(msg)
-    extras = (support_out, triplets_out, taxon_triplets_out, mrp_out, source_rf_out)
+    extras = (support_out, triplets_out, taxon_triplets_out, mrp_out, source_rf_out, source_triplets_out)
     if all(path is None for path in extras):
         text = supertree_newick_of_forest(forest, weighting.lower(), contract_edges=contract_edges)
         Path(out_file).write_text(text + "\n")
@@ -63,6 +64,9 @@ def run(in_file: str, out_file: str, weighting: str = "branch", contract_edges: 
     if source_rf_out is not None:
         distances = flat_source_tree_distances(forest, engine=engine)
         Path(source_rf_out).write_text(distances.tsv())
+    if source_triplets_out is not None:
+        triplet_distances = flat_source_tree_triplet_distances(forest, engine=engine)
+        Path(source_triplets_out).write_text(triplet_distances.tsv())
 
 
 @click.command(no_args_is_help=True)
@@ -109,6 +113,11 @@ def run(in_file: str, out_file: str, weighting: str = "branch", contract_edges: 
     "(TSV).",
     default=None,
 )
+@click.option(
+    "--source-triplets-out",
+    help="Also write the rooted triplet distance between every pair of source trees on the taxa they share (TSV).",
+    default=None,
+)
 def scs(
     in_file: str,
     out_file: str,
@@ -120,11 +129,12 @@ def scs(
     taxon_triplets_out: str | None,
     mrp_out: str | None,
     source_rf_out: str | None,
+    source_triplets_out: str | None,
 ) -> None:
     """Run spectral cluster supertree over the given set of source trees."""
     run(in_file, out_file, pcg_weighting, contract_edges=not disable_contraction, support_out=support_out,
         triplets_out=triplets_out, taxon_triplets_out=taxon_triplets_out, mrp_out=mrp_out,
-        source_rf_out=source_rf_out)
+        source_rf_out=source_rf_out, source_triplets_out=source_triplets_out)
 
 
 if __name__ == "__main__":

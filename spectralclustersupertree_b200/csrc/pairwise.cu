@@ -23,12 +23,21 @@
 // g_j[lo, hi), the outer gaps g_j[lo - 1], g_j[hi] are < d (or absent): range minima and maxima over sparse tables of
 // qi and g_j.  A pair costs O(k_i + k_j + k log k) whatever the depth of the trees; every count is an exact integer,
 // written to the pair's own entries, so the order in which CTAs take pairs changes no bit.
+//
+// Rooted triplet distances (scs_forest_pairwise_triplets) share pass 1 (PairPass).  Pass 2 (pw_triplets) is the row
+// pass of triplets.cu with the supertree replaced by t_j: per row a of t_i', alpha comes from the gaps of t_i' and
+// beta(x) = depth in t_j of LCA(a, x) from one range minimum of t_j's unrestricted tour, counted with a Fenwick tree
+// and histogram over beta (dominance.cuh).  Work items are chunks of a pair's rows, so one large pair spreads over
+// many CTAs; the row sums go to per-pair int64 accumulators with integer atomics, which pw_triplet_out halves into
+// both triangles.
 
 #include <algorithm>
 #include <climits>
+#include <string>
 #include <vector>
 
 #include "devforest.cuh"
+#include "dominance.cuh"
 #include "forest.hpp"
 #include "supertree.cuh"
 
@@ -39,6 +48,8 @@ constexpr int kThreads = 256;
 constexpr int kTile = 64;       // trees per side of a pass-1 tile (16 x 16 threads, 4 x 4 pairs each)
 constexpr int kTileWords = 32;  // bitmap words per pass-1 stage
 constexpr size_t kScratchBytes = size_t(4096) << 20;  // per-CTA scratch of pass 2, all resident CTAs together
+constexpr int kRowWarps = kThreads / 32;  // row warps of a pw_triplets CTA when the trees are shallow enough
+constexpr int kChunkRows = 512;           // rows of a pair one pw_triplets work item counts
 
 // Row t of the bitmap: bit x set iff tree t has a tip labelled x (rows zeroed beforehand; one CTA per tree).
 __global__ void pw_bitmap(const int64_t *__restrict__ tree_off, const int32_t *__restrict__ taxon, int taxa, int words,
@@ -157,6 +168,12 @@ struct PairArgs {
     int64_t slot, max_leaves, max_k;
     int32_t levels;
     int32_t *clusters, *common;  // [T][T]
+    // pw_triplets: k of every pair; log2 of the row chunks per listed pair, ints per shared-memory array of a row warp
+    // and row warps per CTA; the doubled row sums of every listed pair ([pairs][4]) and the T x T results
+    const int32_t *shared;
+    int32_t chunk_bits, stride, warps;
+    unsigned long long *acc;
+    int64_t *resolved, *agree, *contradict;
 };
 
 // min of a sparse table (level l at tab + l * ld) over [lo, hi], lo <= hi; likewise the max
@@ -301,6 +318,268 @@ __global__ void __launch_bounds__(kThreads) pw_pairs(PairArgs a) {
     }
 }
 
+// Depth in t of the LCA of the tips at tour positions p != q of tree t (its tour's table at tab = tour_min + leaf_off[t])
+__device__ __forceinline__ int tour_lca_depth(const int32_t *tab, int64_t ld, int p, int q) {
+    const int lo = min(p, q), hi = max(p, q) - 1;  // adj_depth[j] is the LCA depth of tour positions j and j + 1
+    const int l = 31 - __clz(hi - lo + 1);
+    return min(__ldg(tab + l * ld + lo), __ldg(tab + l * ld + hi - (1 << l) + 1));
+}
+
+// Row a = t_i' position qa of a pair, one warp (the triplet row of triplets.cu with S = t_j): alpha(x) = depth in t_i
+// of LCA(a, x) grows out of the gaps td of t_i', beta(x) = depth in t_j of LCA(a, x) is one range minimum over t_j's
+// unrestricted tour between the tour positions jp of a and x.  Every beta is at most one of the two gap depths beside
+// a in t_j's tour, so the Fenwick tree over beta + 1 in [1, m] and the histogram of beta in [0, m) take m + 1 ints
+// each, m = 1 + the larger of those.  Adds to the lane's partial sums of the four doubled counts, except for the
+// C(k - 1, 2) pairs of the row that r2 starts from.
+__device__ __forceinline__ void pair_row(const PairArgs &a, const int32_t *tabj, int nlj, const int32_t *td,
+                                         const int32_t *jp, int k, int qa, int lane, int32_t *fw, int32_t *hist,
+                                         long long &r1, long long &r2, long long &ag, long long &co) {
+    const int pa = jp[qa];
+    const int m = 1 + max(pa > 0 ? tabj[pa - 1] : -1, pa + 1 < nlj ? tabj[pa] : -1);
+    for (int i = lane; i <= m; i += 32) fw[i] = 0;
+    for (int i = lane; i < m; i += 32) hist[i] = 0;
+    __syncwarp();
+    int L = qa, R = qa, inside = 0;  // t_i' positions [L, R] are inside the window (a itself is no point)
+    for (;;) {
+        int nL, nR;
+        if (grow_window(td, k, lane, L, R, nL, nR) < 0) break;
+        const int left = L - nL, added = left + nR - R;
+        // the new taxa x (alpha(x) = level) against the y inside (alpha(y) > level): concordant when beta(y) >
+        // beta(x), discordant when beta(y) < beta(x)
+        for (int i = lane; i < added; i += 32) {
+            const int b = tour_lca_depth(tabj, a.leaves, pa, jp[i < left ? nL + i : R + 1 + (i - left)]);
+            const int below = fenwick_prefix(fw, b);
+            co += below;
+            ag += inside - below - hist[b];
+        }
+        __syncwarp();
+        for (int i = lane; i < added; i += 32) {
+            const int b = tour_lca_depth(tabj, a.leaves, pa, jp[i < left ? nL + i : R + 1 + (i - left)]);
+            fenwick_add(fw, b + 1, m, 1);
+            atomicAdd(&hist[b], 1);
+        }
+        __syncwarp();
+        if (lane == 0) r1 += static_cast<long long>(inside) * added;
+        inside += added;
+        L = nL;
+        R = nR;
+    }
+    // pairs {b, x} with beta(b) = beta(x), taken off the row's C(k - 1, 2) pairs by the caller
+    for (int i = lane; i < m; i += 32) r2 -= static_cast<long long>(hist[i]) * (hist[i] - 1) / 2;
+    __syncwarp();  // the next row clears the arrays
+}
+
+// Persistent CTAs taking work items from a counter: item it is rows [c * kChunkRows, (c + 1) * kChunkRows) of listed
+// pair it >> chunk_bits, c = the low chunk_bits bits of it (none if that is past k).  X and its ranks as in pw_pairs; jtour[r] = position in
+// t_j's unrestricted tour of the taxon of rank r; t_i's tour restricted to X gives, per t_i' position q, the t_j tour
+// position jp[q] of its taxon and td[q], the depth in t_i of the LCA of t_i' positions q and q + 1.  The row warps
+// then reuse the shared memory of the bitmap for their Fenwick trees and histograms; their sums go to the pair's
+// accumulators as exact integer atomics, so the order in which CTAs take items changes no bit.
+__global__ void __launch_bounds__(kThreads) pw_triplets(PairArgs a) {
+    extern __shared__ uint32_t smem[];
+    uint32_t *bits = smem;
+    int32_t *wpre = reinterpret_cast<int32_t *>(smem + a.words);
+    __shared__ int32_t sums[33];
+    __shared__ long long item;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int64_t ld = a.max_k;
+    int32_t *flag = a.scratch + blockIdx.x * a.slot;
+    int32_t *kidx = flag + a.max_leaves + 1, *jtour = kidx + ld, *jp = jtour + ld, *td = jp + ld;
+    int32_t *fw = reinterpret_cast<int32_t *>(smem) + warp * 2 * a.stride, *hist = fw + a.stride;
+    for (;;) {
+        if (threadIdx.x == 0) item = static_cast<long long>(atomicAdd(a.next, 1ull));
+        __syncthreads();
+        const int64_t it = item;
+        if (it >= a.pairs << a.chunk_bits) return;
+        const int64_t pair = it >> a.chunk_bits;
+        const int ti = a.list[pair].x, tj = a.list[pair].y;
+        const int k = a.shared[static_cast<int64_t>(ti) * a.T + tj];
+        const int row0 = static_cast<int>(it & ((int64_t(1) << a.chunk_bits) - 1)) * kChunkRows;
+        if (row0 >= k) {  // past the pair's rows: every thread reads `item` before thread 0 takes the next one
+            __syncthreads();
+            continue;
+        }
+        const uint32_t *ri = a.bits + static_cast<int64_t>(ti) * a.words, *rj = a.bits + static_cast<int64_t>(tj) * a.words;
+        for (int w = threadIdx.x; w < a.words; w += blockDim.x) {
+            bits[w] = ri[w] & rj[w];
+            wpre[w] = __popc(bits[w]);
+        }
+        __syncthreads();
+        block_scan(wpre, a.words, sums);
+
+        // t_j: rank in X -> unrestricted tour position
+        const int64_t lbj = a.leaf_off[tj];
+        const int nlj = static_cast<int>(a.leaf_off[tj + 1] - lbj);
+        {
+            const int32_t *lt = a.leaf_taxon + lbj;
+            for (int j = threadIdx.x; j < nlj; j += blockDim.x) {
+                const int x = lt[j];
+                if ((bits[x >> 5] >> (x & 31)) & 1u) jtour[bitmap_rank(bits, wpre, x)] = j;
+            }
+        }
+        // t_i': the t_j tour position of every t_i' tip, and its gaps (restrict_tour's barriers order jtour)
+        restrict_tour(a, ti, bits, flag, kidx, sums);
+        {
+            const int32_t *lt = a.leaf_taxon + a.leaf_off[ti];
+            for (int p = threadIdx.x; p < k; p += blockDim.x) jp[p] = jtour[bitmap_rank(bits, wpre, lt[kidx[p]])];
+        }
+        gap_depths(a, ti, kidx, k, td);
+        __syncthreads();  // bits and wpre are free from here: the rows' Fenwick trees and histograms take their place
+
+        if (warp < a.warps) {
+            const int32_t *tabj = a.tour_min + lbj;
+            const int row1 = min(k, row0 + kChunkRows);
+            long long r1 = 0, r2 = 0, ag = 0, co = 0;
+            int rows = 0;
+            for (int qa = row0 + warp; qa < row1; qa += a.warps, ++rows)
+                pair_row(a, tabj, nlj, td, jp, k, qa, lane, fw, hist, r1, r2, ag, co);
+            if (lane == 0) r2 += static_cast<long long>(rows) * ((k - 1) * static_cast<long long>(k - 2) / 2);
+#pragma unroll
+            for (int off = 16; off > 0; off >>= 1) {
+                r1 += __shfl_down_sync(0xffffffffu, r1, off);
+                r2 += __shfl_down_sync(0xffffffffu, r2, off);
+                ag += __shfl_down_sync(0xffffffffu, ag, off);
+                co += __shfl_down_sync(0xffffffffu, co, off);
+            }
+            if (lane == 0) {
+                unsigned long long *acc = a.acc + 4 * pair;
+                if (r1) atomicAdd(acc, static_cast<unsigned long long>(r1));
+                if (r2) atomicAdd(acc + 1, static_cast<unsigned long long>(r2));
+                if (ag) atomicAdd(acc + 2, static_cast<unsigned long long>(ag));
+                if (co) atomicAdd(acc + 3, static_cast<unsigned long long>(co));
+            }
+        }
+        // the barrier at the top of the loop keeps the next item's bitmap out of the rows' arrays
+    }
+}
+
+// One thread per listed pair (i, j): its doubled sums halved as tp_reduce halves them (a resolved or agreeing triplet
+// is seen from two rows, a contradicting one from one) into both triangles; row i of `resolved` counts tree i.
+__global__ void pw_triplet_out(PairArgs a) {
+    const int64_t p = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (p >= a.pairs) return;
+    const int64_t i = a.list[p].x, j = a.list[p].y;
+    const unsigned long long *s = a.acc + 4 * p;
+    a.resolved[i * a.T + j] = static_cast<int64_t>(s[0] / 2);
+    a.resolved[j * a.T + i] = static_cast<int64_t>(s[1] / 2);
+    a.agree[i * a.T + j] = a.agree[j * a.T + i] = static_cast<int64_t>(s[2] / 2);
+    a.contradict[i * a.T + j] = a.contradict[j * a.T + i] = static_cast<int64_t>(s[3]);
+}
+
+// Pass 1 and what pass 2 of both entry points reads: the forest's taxon bitmaps, k of every pair, the work list of the
+// pairs i <= j with k >= 3 and the largest such k; when the list is not empty, the forest's tours (weighting one) and
+// the sparse table over them.
+struct PairPass {
+    int T = 0, taxa = 0, words = 0;
+    size_t smem = 0;  // the bitmap of a pair and the prefix of its word popcounts in shared memory
+    int64_t max_leaves = 0, pairs = 0, max_k = 0;
+    DevForest df;
+    DevTours tours;
+    GrowBuf ident, flags, bits, d_shared, list, counters, table;
+
+    // Host side: the limits of the bitmap and of the tile grid (failure status, message set, or SCS_OK).
+    int prepare(scs_ctx *ctx, const char *name, const scs_forest *forest) {
+        T = forest->num_trees();
+        taxa = forest->num_taxa;
+        words = std::max(1, ceil_div(taxa, 32));
+        smem = static_cast<size_t>(words) * 8;
+        if (smem + 1024 > ctx->smem_optin)  // room for the static shared arrays
+            return fail(ctx, SCS_ERR_INVALID, (std::string(name) + ": too many taxa for the shared-memory bitmap of a pair").c_str());
+        const int64_t nb = (static_cast<int64_t>(T) + kTile - 1) / kTile;
+        if (nb * (nb + 1) / 2 > INT_MAX)
+            return fail(ctx, SCS_ERR_INVALID, (std::string(name) + ": too many trees for the grid of pair tiles").c_str());
+        const std::vector<int64_t> &loff = forest->leaf_offsets;
+        for (int t = 0; t < T; ++t) max_leaves = std::max(max_leaves, loff[t + 1] - loff[t]);
+        return SCS_OK;
+    }
+
+    // The device side (T > 0); returns after the work list's length and largest k are on the host.
+    int run(scs_ctx *ctx, const scs_forest *forest) {
+        int rc;
+        if ((rc = devforest_upload(ctx, forest, 0, &df))) return rc;
+        const size_t TT = static_cast<size_t>(T) * static_cast<size_t>(T);
+        const size_t words_bytes = static_cast<size_t>(T) * words * sizeof(uint32_t);
+        const size_t list_bytes = (static_cast<size_t>(T) * (T + 1) / 2) * sizeof(int2);
+        if ((rc = grow(ctx, bits, words_bytes)) || (rc = grow(ctx, d_shared, TT * 4)) || (rc = grow(ctx, list, list_bytes)) ||
+            (rc = grow(ctx, counters, 24)))
+            return rc;
+        SCS_CUDA(ctx, cudaMemsetAsync(bits.ptr, 0, words_bytes, ctx->stream));
+        SCS_CUDA(ctx, cudaMemsetAsync(counters.ptr, 0, 24, ctx->stream));
+        const int nb = (T + kTile - 1) / kTile;
+        pw_bitmap<<<T, kThreads, 0, ctx->stream>>>(df.tree_off.as<int64_t>(), df.taxon.as<int32_t>(), taxa, words,
+                                                   bits.as<uint32_t>());
+        SCS_LAUNCHED(ctx, "pw_bitmap");
+        pw_shared<<<nb * (nb + 1) / 2, kThreads, 0, ctx->stream>>>(T, words, bits.as<uint32_t>(), d_shared.as<int32_t>(),
+                                                                   list.as<int2>(), count(), max_k_dev());
+        SCS_LAUNCHED(ctx, "pw_shared");
+        struct {
+            unsigned long long pairs;
+            int32_t max_k, pad;
+        } head{};
+        SCS_CUDA(ctx, cudaMemcpyAsync(&head, counters.ptr, 16, cudaMemcpyDeviceToHost, ctx->stream));
+        SCS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        pairs = static_cast<int64_t>(head.pairs);
+        max_k = head.max_k;
+        if (pairs == 0) return SCS_OK;
+        std::vector<int32_t> identity(static_cast<size_t>(taxa > 0 ? taxa : 1));
+        for (size_t x = 0; x < identity.size(); ++x) identity[x] = static_cast<int32_t>(x);
+        if ((rc = grow(ctx, ident, identity.size() * sizeof(int32_t))) || (rc = grow(ctx, flags, 2 * sizeof(int32_t))))
+            return rc;
+        SCS_CUDA(ctx, cudaMemcpyAsync(ident.ptr, identity.data(), identity.size() * sizeof(int32_t), cudaMemcpyHostToDevice,
+                                      ctx->stream));
+        SCS_CUDA(ctx, cudaMemsetAsync(flags.ptr, 0, 2 * sizeof(int32_t), ctx->stream));
+        if ((rc = devforest_tours(ctx, df, 0, ident.as<int32_t>(), &tours, flags.as<int32_t>()))) return rc;
+        int tour_levels = 1;
+        while ((int64_t(1) << tour_levels) <= max_leaves) ++tour_levels;
+        if ((rc = grow(ctx, table, static_cast<size_t>(df.leaves) * tour_levels * sizeof(int32_t)))) return rc;
+        SCS_CUDA(ctx, cudaMemcpyAsync(table.ptr, tours.adj_depth.ptr, static_cast<size_t>(df.leaves) * sizeof(int32_t),
+                                      cudaMemcpyDeviceToDevice, ctx->stream));
+        pw_tour_table<<<T, kThreads, 0, ctx->stream>>>(df.leaf_off.as<int64_t>(), df.leaves, table.as<int32_t>());
+        SCS_LAUNCHED(ctx, "pw_tour_table");
+        return SCS_OK;
+    }
+
+    // listed pairs, largest k, next item of pass 2
+    unsigned long long *count() const { return counters.as<unsigned long long>(); }
+    int *max_k_dev() const { return reinterpret_cast<int *>(count() + 1); }
+
+    // The fields of pass 2's arguments that pass 1 gives.
+    void fill(PairArgs *args) const {
+        args->T = T;
+        args->words = words;
+        args->bits = bits.as<uint32_t>();
+        args->leaf_off = df.leaf_off.as<int64_t>();
+        args->leaf_taxon = tours.leaf_taxon.as<int32_t>();
+        args->tour_min = table.as<int32_t>();
+        args->leaves = df.leaves;
+        args->list = list.as<int2>();
+        args->pairs = pairs;
+        args->next = count() + 2;
+        args->max_leaves = max_leaves;
+        args->max_k = max_k;
+    }
+
+    // Resident CTAs of a pass-2 kernel with `dyn` bytes of shared memory, at most `work` and at most what
+    // kScratchBytes of per-CTA scratch of `slot` ints allows.
+    template <typename K>
+    int ctas(scs_ctx *ctx, K kernel, size_t dyn, int64_t slot, int64_t work, int64_t *out) const {
+        if (dyn > 48 * 1024)
+            SCS_CUDA(ctx, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(dyn)));
+        int per_sm = 0;
+        SCS_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kThreads, dyn));
+        int64_t n = static_cast<int64_t>(std::max(per_sm, 1)) * ctx->sm_count;
+        n = std::min<int64_t>(n, std::max<int64_t>(1, static_cast<int64_t>(kScratchBytes / (slot * sizeof(int32_t)))));
+        *out = std::min<int64_t>(n, work);
+        return SCS_OK;
+    }
+
+    void release_all(scs_ctx *ctx) {
+        df.free_all(ctx);
+        tours.free_all(ctx);
+        for (GrowBuf *b : {&ident, &flags, &bits, &d_shared, &list, &counters, &table}) release(ctx, *b);
+    }
+};
+
 }  // namespace
 }  // namespace scs
 
@@ -310,120 +589,149 @@ extern "C" int scs_forest_pairwise_rf(scs_ctx *ctx, const scs_forest *forest, in
                                       int32_t *common) {
     if (!ctx) return SCS_ERR_INVALID;
     if (!forest || !shared_taxa || !clusters || !common) return fail(ctx, SCS_ERR_INVALID, "scs_forest_pairwise_rf: bad argument");
-    const int T = forest->num_trees(), taxa = forest->num_taxa;
-    const int words = std::max(1, ceil_div(taxa, 32));
-    const size_t smem = static_cast<size_t>(words) * 8;
-    if (smem + 1024 > ctx->smem_optin)  // room for the static shared arrays
-        return fail(ctx, SCS_ERR_INVALID, "scs_forest_pairwise_rf: too many taxa for the shared-memory bitmap of a pair");
-    const int64_t nb = (static_cast<int64_t>(T) + kTile - 1) / kTile, tiles = nb * (nb + 1) / 2;
-    if (tiles > INT_MAX)
-        return fail(ctx, SCS_ERR_INVALID, "scs_forest_pairwise_rf: too many trees for the grid of pair tiles");
+    PairPass p;
+    int rc = p.prepare(ctx, "scs_forest_pairwise_rf", forest);
+    if (rc) return rc;
+    const int T = p.T;
     if (T == 0) return SCS_OK;
     const size_t TT = static_cast<size_t>(T) * static_cast<size_t>(T);
-    const std::vector<int64_t> &loff = forest->leaf_offsets;
-    int64_t max_leaves = 0;
-    for (int t = 0; t < T; ++t) max_leaves = std::max(max_leaves, loff[t + 1] - loff[t]);
 
-    DevForest df;
-    DevTours tours;
-    GrowBuf ident, flags, bits, d_shared, d_clusters, d_common, list, counters, table, scratch;
+    GrowBuf d_clusters, d_common, scratch;
     auto cleanup = [&] {
-        df.free_all(ctx);
-        tours.free_all(ctx);
-        for (GrowBuf *b : {&ident, &flags, &bits, &d_shared, &d_clusters, &d_common, &list, &counters, &table, &scratch})
-            release(ctx, *b);
+        p.release_all(ctx);
+        for (GrowBuf *b : {&d_clusters, &d_common, &scratch}) release(ctx, *b);
         cudaStreamSynchronize(ctx->stream);
     };
     auto run = [&]() -> int {
-        int rc;
-        if ((rc = devforest_upload(ctx, forest, 0, &df))) return rc;
-        const size_t words_bytes = static_cast<size_t>(T) * words * sizeof(uint32_t);
-        const size_t list_bytes = (static_cast<size_t>(T) * (T + 1) / 2) * sizeof(int2);
-        if ((rc = grow(ctx, bits, words_bytes)) || (rc = grow(ctx, d_shared, TT * 4)) || (rc = grow(ctx, d_clusters, TT * 4)) ||
-            (rc = grow(ctx, d_common, TT * 4)) || (rc = grow(ctx, list, list_bytes)) || (rc = grow(ctx, counters, 24)))
-            return rc;
-        SCS_CUDA(ctx, cudaMemsetAsync(bits.ptr, 0, words_bytes, ctx->stream));
+        if ((rc = grow(ctx, d_clusters, TT * 4)) || (rc = grow(ctx, d_common, TT * 4))) return rc;
         SCS_CUDA(ctx, cudaMemsetAsync(d_clusters.ptr, 0, TT * 4, ctx->stream));
         SCS_CUDA(ctx, cudaMemsetAsync(d_common.ptr, 0, TT * 4, ctx->stream));
-        SCS_CUDA(ctx, cudaMemsetAsync(counters.ptr, 0, 24, ctx->stream));
-        unsigned long long *count = counters.as<unsigned long long>();  // listed pairs, largest k, next pair of pass 2
-        int *max_k = reinterpret_cast<int *>(count + 1);
+        // pass 1: bitmaps, shared taxa of every pair, the work list, the tours and their sparse table
+        if ((rc = p.run(ctx, forest))) return rc;
 
-        // pass 1: bitmaps, shared taxa of every pair, the work list
-        pw_bitmap<<<T, kThreads, 0, ctx->stream>>>(df.tree_off.as<int64_t>(), df.taxon.as<int32_t>(), taxa, words,
-                                                   bits.as<uint32_t>());
-        SCS_LAUNCHED(ctx, "pw_bitmap");
-        pw_shared<<<static_cast<int>(tiles), kThreads, 0, ctx->stream>>>(T, words, bits.as<uint32_t>(), d_shared.as<int32_t>(),
-                                                                         list.as<int2>(), count, max_k);
-        SCS_LAUNCHED(ctx, "pw_shared");
-        struct {
-            unsigned long long pairs;
-            int32_t max_k, pad;
-        } head{};
-        SCS_CUDA(ctx, cudaMemcpyAsync(&head, counters.ptr, 16, cudaMemcpyDeviceToHost, ctx->stream));
-        SCS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-
-        if (head.pairs > 0) {
-            // pass 2: tours, their sparse table, one CTA per listed pair
-            std::vector<int32_t> identity(static_cast<size_t>(taxa > 0 ? taxa : 1));
-            for (size_t x = 0; x < identity.size(); ++x) identity[x] = static_cast<int32_t>(x);
-            if ((rc = grow(ctx, ident, identity.size() * sizeof(int32_t))) || (rc = grow(ctx, flags, 2 * sizeof(int32_t))))
-                return rc;
-            SCS_CUDA(ctx, cudaMemcpyAsync(ident.ptr, identity.data(), identity.size() * sizeof(int32_t), cudaMemcpyHostToDevice,
-                                          ctx->stream));
-            SCS_CUDA(ctx, cudaMemsetAsync(flags.ptr, 0, 2 * sizeof(int32_t), ctx->stream));
-            if ((rc = devforest_tours(ctx, df, 0, ident.as<int32_t>(), &tours, flags.as<int32_t>()))) return rc;
-            const int64_t leaves = df.leaves;
-            int tour_levels = 1;
-            while ((int64_t(1) << tour_levels) <= max_leaves) ++tour_levels;
-            if ((rc = grow(ctx, table, static_cast<size_t>(leaves) * tour_levels * sizeof(int32_t)))) return rc;
-            SCS_CUDA(ctx, cudaMemcpyAsync(table.ptr, tours.adj_depth.ptr, static_cast<size_t>(leaves) * sizeof(int32_t),
-                                          cudaMemcpyDeviceToDevice, ctx->stream));
-            pw_tour_table<<<T, kThreads, 0, ctx->stream>>>(df.leaf_off.as<int64_t>(), leaves, table.as<int32_t>());
-            SCS_LAUNCHED(ctx, "pw_tour_table");
-
-            const int64_t mk = head.max_k;
+        if (p.pairs > 0) {
+            // pass 2: one CTA per listed pair
+            const int64_t mk = p.max_k;
             int levels = 1;
             while ((int64_t(1) << levels) <= mk) ++levels;
-            const int64_t slot = (max_leaves + 1) + 2 * mk + 4 * static_cast<int64_t>(levels) * mk;
-            if (smem > 48 * 1024)
-                SCS_CUDA(ctx, cudaFuncSetAttribute(pw_pairs, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-            int per_sm = 0;
-            SCS_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, pw_pairs, kThreads, smem));
-            int64_t ctas = static_cast<int64_t>(std::max(per_sm, 1)) * ctx->sm_count;
-            ctas = std::min<int64_t>(ctas, std::max<int64_t>(1, static_cast<int64_t>(kScratchBytes / (slot * sizeof(int32_t)))));
-            ctas = std::min<int64_t>(ctas, static_cast<int64_t>(head.pairs));
+            const int64_t slot = (p.max_leaves + 1) + 2 * mk + 4 * static_cast<int64_t>(levels) * mk;
+            int64_t ctas = 0;
+            if ((rc = p.ctas(ctx, pw_pairs, p.smem, slot, p.pairs, &ctas))) return rc;
             if ((rc = grow(ctx, scratch, static_cast<size_t>(ctas * slot) * sizeof(int32_t)))) return rc;
 
             PairArgs args{};
-            args.T = T;
-            args.words = words;
-            args.bits = bits.as<uint32_t>();
-            args.leaf_off = df.leaf_off.as<int64_t>();
-            args.leaf_taxon = tours.leaf_taxon.as<int32_t>();
-            args.tour_min = table.as<int32_t>();
-            args.leaves = leaves;
-            args.list = list.as<int2>();
-            args.pairs = static_cast<int64_t>(head.pairs);
-            args.next = count + 2;
+            p.fill(&args);
             args.scratch = scratch.as<int32_t>();
             args.slot = slot;
-            args.max_leaves = max_leaves;
-            args.max_k = mk;
             args.levels = levels;
             args.clusters = d_clusters.as<int32_t>();
             args.common = d_common.as<int32_t>();
-            pw_pairs<<<static_cast<int>(ctas), kThreads, smem, ctx->stream>>>(args);
+            pw_pairs<<<static_cast<int>(ctas), kThreads, p.smem, ctx->stream>>>(args);
             SCS_LAUNCHED(ctx, "pw_pairs");
         }
-        SCS_CUDA(ctx, cudaMemcpyAsync(shared_taxa, d_shared.ptr, TT * 4, cudaMemcpyDeviceToHost, ctx->stream));
+        SCS_CUDA(ctx, cudaMemcpyAsync(shared_taxa, p.d_shared.ptr, TT * 4, cudaMemcpyDeviceToHost, ctx->stream));
         SCS_CUDA(ctx, cudaMemcpyAsync(clusters, d_clusters.ptr, TT * 4, cudaMemcpyDeviceToHost, ctx->stream));
         SCS_CUDA(ctx, cudaMemcpyAsync(common, d_common.ptr, TT * 4, cudaMemcpyDeviceToHost, ctx->stream));
         SCS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
         ctx->d2h_bytes += static_cast<int64_t>(3 * TT * 4 + 16);
         return SCS_OK;
     };
-    const int rc = run();
+    rc = run();
+    cleanup();
+    return rc;
+}
+
+extern "C" int scs_forest_pairwise_triplets(scs_ctx *ctx, const scs_forest *forest, int32_t *shared_taxa,
+                                            int64_t *resolved, int64_t *agree, int64_t *contradict) {
+    if (!ctx) return SCS_ERR_INVALID;
+    if (!forest || !shared_taxa || !resolved || !agree || !contradict)
+        return fail(ctx, SCS_ERR_INVALID, "scs_forest_pairwise_triplets: bad argument");
+    PairPass p;
+    int rc = p.prepare(ctx, "scs_forest_pairwise_triplets", forest);
+    if (rc) return rc;
+    const int T = p.T;
+    // the deepest tip of the forest bounds every beta of a row: two arrays of (depth + 1) ints per row warp
+    int max_depth = 0;
+    {
+        const std::vector<int64_t> &noff = forest->node_offsets;
+#pragma omp parallel num_threads(scs_host_threads()) reduction(max : max_depth)
+        {
+            std::vector<int32_t> depth;
+#pragma omp for schedule(dynamic, 16)
+            for (int t = 0; t < T; ++t) {
+                const int64_t b = noff[t], n = noff[t + 1] - b;
+                depth.assign(static_cast<size_t>(n), 0);
+                for (int64_t u = 1; u < n; ++u) {  // parent < child within a tree
+                    depth[u] = depth[forest->parent[b + u]] + 1;
+                    max_depth = std::max(max_depth, depth[u]);
+                }
+            }
+        }
+    }
+    const int stride = max_depth + 1;
+    const size_t warp_smem = 2 * static_cast<size_t>(stride) * sizeof(int32_t);
+    const int warps = static_cast<int>(std::min<size_t>(kRowWarps, (ctx->smem_optin - 1024) / warp_smem));
+    if (warps < 1)
+        return fail(ctx, SCS_ERR_INVALID,
+                    "scs_forest_pairwise_triplets: a source tree is too deep for the shared-memory Fenwick tree of a row");
+    if (T == 0) return SCS_OK;
+    const size_t TT = static_cast<size_t>(T) * static_cast<size_t>(T);
+
+    GrowBuf d_resolved, d_agree, d_contradict, acc, scratch;
+    auto cleanup = [&] {
+        p.release_all(ctx);
+        for (GrowBuf *b : {&d_resolved, &d_agree, &d_contradict, &acc, &scratch}) release(ctx, *b);
+        cudaStreamSynchronize(ctx->stream);
+    };
+    auto run = [&]() -> int {
+        const size_t mat = TT * sizeof(int64_t);
+        if ((rc = grow(ctx, d_resolved, mat)) || (rc = grow(ctx, d_agree, mat)) || (rc = grow(ctx, d_contradict, mat)))
+            return rc;
+        SCS_CUDA(ctx, cudaMemsetAsync(d_resolved.ptr, 0, mat, ctx->stream));
+        SCS_CUDA(ctx, cudaMemsetAsync(d_agree.ptr, 0, mat, ctx->stream));
+        SCS_CUDA(ctx, cudaMemsetAsync(d_contradict.ptr, 0, mat, ctx->stream));
+        if ((rc = p.run(ctx, forest))) return rc;
+
+        if (p.pairs > 0) {
+            // pass 2: persistent CTAs over chunks of rows of the listed pairs
+            const int64_t mk = p.max_k;
+            int chunk_bits = 0;  // a power of two of row chunks per pair covers the largest k
+            while ((int64_t(kChunkRows) << chunk_bits) < mk) ++chunk_bits;
+            const int64_t slot = (p.max_leaves + 1) + 4 * mk;
+            const size_t dyn = std::max(p.smem, static_cast<size_t>(warps) * warp_smem);
+            int64_t ctas = 0;
+            if ((rc = p.ctas(ctx, pw_triplets, dyn, slot, p.pairs << chunk_bits, &ctas))) return rc;
+            const size_t acc_bytes = static_cast<size_t>(p.pairs) * 4 * sizeof(unsigned long long);
+            if ((rc = grow(ctx, scratch, static_cast<size_t>(ctas * slot) * sizeof(int32_t))) || (rc = grow(ctx, acc, acc_bytes)))
+                return rc;
+            SCS_CUDA(ctx, cudaMemsetAsync(acc.ptr, 0, acc_bytes, ctx->stream));
+
+            PairArgs args{};
+            p.fill(&args);
+            args.scratch = scratch.as<int32_t>();
+            args.slot = slot;
+            args.shared = p.d_shared.as<int32_t>();
+            args.chunk_bits = chunk_bits;
+            args.stride = stride;
+            args.warps = warps;
+            args.acc = acc.as<unsigned long long>();
+            args.resolved = d_resolved.as<int64_t>();
+            args.agree = d_agree.as<int64_t>();
+            args.contradict = d_contradict.as<int64_t>();
+            pw_triplets<<<static_cast<int>(ctas), kThreads, dyn, ctx->stream>>>(args);
+            SCS_LAUNCHED(ctx, "pw_triplets");
+            pw_triplet_out<<<static_cast<int>(ceil_div(p.pairs, kThreads)), kThreads, 0, ctx->stream>>>(args);
+            SCS_LAUNCHED(ctx, "pw_triplet_out");
+        }
+        SCS_CUDA(ctx, cudaMemcpyAsync(shared_taxa, p.d_shared.ptr, TT * 4, cudaMemcpyDeviceToHost, ctx->stream));
+        SCS_CUDA(ctx, cudaMemcpyAsync(resolved, d_resolved.ptr, mat, cudaMemcpyDeviceToHost, ctx->stream));
+        SCS_CUDA(ctx, cudaMemcpyAsync(agree, d_agree.ptr, mat, cudaMemcpyDeviceToHost, ctx->stream));
+        SCS_CUDA(ctx, cudaMemcpyAsync(contradict, d_contradict.ptr, mat, cudaMemcpyDeviceToHost, ctx->stream));
+        SCS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        ctx->d2h_bytes += static_cast<int64_t>(TT * 4 + 3 * mat + 16);
+        return SCS_OK;
+    };
+    rc = run();
     cleanup();
     return rc;
 }

@@ -316,6 +316,21 @@ class Engine:
         _check(status, self._ctx)
         return shared, clusters, common
 
+    def forest_pairwise_triplets(self, forest: "Forest") -> tuple[np.ndarray, np.ndarray, np.ndarray, np.ndarray]:
+        """``scs_forest_pairwise_triplets``: for every pair of source trees, restricted to the taxa they share, the
+        ``[T, T]`` int32 matrix of shared taxa and three int64 ones: the triplets resolved in row tree i's restriction
+        (not symmetric), those resolved the same way in both restrictions and those resolved in both but
+        differently."""
+        T = forest.num_trees
+        shared = np.zeros((T, T), dtype=np.int32)
+        resolved = np.zeros((T, T), dtype=np.int64)
+        agree = np.zeros((T, T), dtype=np.int64)
+        contradict = np.zeros((T, T), dtype=np.int64)
+        status = self._lib.scs_forest_pairwise_triplets(self._ctx, forest.handle, ptr(shared), ptr(resolved),
+                                                        ptr(agree), ptr(contradict))  # fmt: skip
+        _check(status, self._ctx)
+        return shared, resolved, agree, contradict
+
     def _collect_supertree(self, handle, record: bool) -> dict:
         try:
             count = self._lib.scs_supertree_num_nodes(handle)
