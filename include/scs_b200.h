@@ -58,14 +58,17 @@ typedef struct {
     int32_t solver;          /* 0 none, 1 trivial (m = 2), 2 dense Jacobi (one CTA), 3 Lanczos */
     int32_t matvecs;         /* operator applications in the Lanczos solver */
     int32_t restarts;
-    int32_t tie_flag;        /* bit 0: eigengap lambda_3 - lambda_2 < 1e-7; bit 1: a vertex within 1e-9
+    int32_t tie_flag;        /* bit 0: eigengap eig[2] - eig[1] < 1e-7 (exact with the dense solver; the Lanczos
+                                solver raises it only for a real tie but misses a repeated lambda_2 unless its
+                                Krylov space closes early); bit 1: a vertex within 1e-9
                                 (relative) of the 2-means boundary; bit 2: eigensolver stopped at its
                                 restart limit; bit 3: a degree is negative or not finite; bit 4: the
                                 1-D 2-means has more than one Lloyd-stable split, i.e. sklearn's
                                 k-means outcome depends on its random initialisation */
     int32_t kmeans_stable_splits; /* number of Lloyd-stable splits of the Fiedler coordinate */
     double eig[3];           /* three smallest eigenvalues of L = I - D^-1/2 W D^-1/2 (eig[0] = 0;
-                                eig[2] is the solver's estimate, NaN if not available) */
+                                eig[2] is the solver's estimate, NaN if not available: exact with the dense
+                                solver, an upper bound on lambda_3 with Lanczos) */
     double residual;         /* || N y - theta y ||_2 of the Fiedler Ritz pair */
     double margin;           /* min_i |u_i - midpoint| / range(u): distance to the 2-means cut */
     double kmeans_runner_up; /* between-cluster score of the best other stable split / the optimum's

@@ -168,6 +168,22 @@ def rf_outside(tree, reference, divergent_sets) -> int:
     return sum(1 for clade in diff if not any(clade <= d for d in divergent_sets))
 
 
+def node_graphs(case: dict) -> dict:
+    """Contracted graph of every spectral node of the oracle's recursion over a golden case (C restatement of the
+    reference), by sorted vertex names.  Below a node where sklearn's k-means depends on the seed the run may leave
+    the recorded one; such nodes are simply not found."""
+    from oracle import scs_oracle
+
+    graphs: dict = {}
+
+    def hook(record, Wc, side, groups):
+        graphs[tuple(record["names"])] = np.array(Wc)
+
+    scs_oracle.construct_supertree(parse(case["lines"]), case["weights"], case["weighting"], use_c=True,
+                                   random_state=np.random.RandomState(0), node_hook=hook)  # fmt: skip
+    return graphs
+
+
 # ---- compact traces of the CPU oracle's whole recursion at full workload size (tools/oracle_run.py) --------
 def ctrace_key(ids: np.ndarray) -> str:
     import hashlib

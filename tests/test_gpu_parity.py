@@ -149,7 +149,7 @@ def test_spectral_tiny_and_degenerate(engine):
         engine.spectral_bipartition(np.zeros((1, 1)))
 
 
-@pytest.mark.parametrize("m", [2, 3, 31, 100, 1001, 2048, 3001])
+@pytest.mark.parametrize("m", [2, 3, 31, 100, 1001, 2047, 2048, 2049, 3001, 4097, 8193])  # warp / CTA per row at 2048
 def test_normalized_matvec(engine, m):
     A = random_affinity(m, 0.7, m)
     d = A.sum(axis=1)
