@@ -446,6 +446,16 @@ int scs_supertree_taxon_triplets(scs_ctx *ctx, const scs_forest *sources, int64_
 int scs_supertree_mrp(scs_ctx *ctx, const scs_forest *sources, int64_t num_nodes, const int32_t *parent,
                       const int32_t *taxon, int64_t *per_tree);
 
+/* Maximum agreement subtree of the same supertree (validated as in scs_supertree_support; SCS_ERR_INPUT if malformed)
+ * and every source tree t, both restricted to the k taxa X_t they share (unary nodes collapse, polytomies stay): the
+ * largest Y in X_t on which the two restrictions are the same rooted tree.  per_tree[2 * T], int64 per tree: k and
+ * |Y| (k when k <= 2).  Each tree needs a table of (k - 1)^2 ints on the device; SCS_ERR_INVALID with a message, before
+ * any launch, if one tree's region passes 4 GiB (k above about 32 700), or if the supertree has more tips than the
+ * shared-memory bitmap of a tree allows (about 925 000, as scs_supertree_support).  Any depth and any degree.  Returns
+ * after the results landed. */
+int scs_supertree_mast(scs_ctx *ctx, const scs_forest *sources, int64_t num_nodes, const int32_t *parent,
+                       const int32_t *taxon, int64_t *per_tree);
+
 /* Rooted Robinson-Foulds distances between every pair of source trees of the forest, each pair restricted to the k
  * taxa X it shares (as scs_forest_induce restricts; no supertree is involved).  Three caller-owned T x T row-major
  * int32 arrays: shared_taxa[i][j] = k (symmetric; the diagonal is the tree's tip count); clusters[i][j] = the

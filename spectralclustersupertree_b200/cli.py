@@ -17,6 +17,7 @@ import click
 from . import __version__
 from .distances import flat_source_tree_distances, flat_source_tree_triplet_distances
 from .load import load_forest
+from .mast import flat_mast_fit
 from .engine import default_engine
 from .mrp import flat_mrp_score
 from .scs import flat_newick, supertree_newick_of_forest
@@ -27,7 +28,8 @@ from .triplets import flat_taxon_triplet_fit, flat_triplet_fit
 def run(in_file: str, out_file: str, weighting: str = "branch", contract_edges: bool = True,
         support_out: str | None = None, triplets_out: str | None = None,
         taxon_triplets_out: str | None = None, mrp_out: str | None = None,
-        source_rf_out: str | None = None, source_triplets_out: str | None = None) -> None:
+        source_rf_out: str | None = None, source_triplets_out: str | None = None,
+        mast_out: str | None = None) -> None:
     """``load_trees`` + ``construct_supertree`` + ``write`` of the reference's command (ref: cli.py:33-39).  With
     ``support_out`` the supertree is also written there with the V support index of every internal non-root node
     (``support.flat_clade_support``) as its label; with ``triplets_out`` the triplet fit of every source tree
@@ -36,12 +38,14 @@ def run(in_file: str, out_file: str, weighting: str = "branch", contract_edges: 
     (``mrp.flat_mrp_score``) is written there as TSV; with ``source_rf_out`` the Robinson-Foulds distance of every pair
     of source trees that share at least three taxa (``distances.flat_source_tree_distances``) is written there as
     TSV, and with ``source_triplets_out`` their rooted triplet distance
-    (``distances.flat_source_tree_triplet_distances``).  The supertree is built once either way."""
+    (``distances.flat_source_tree_triplet_distances``); with ``mast_out`` the maximum agreement subtree of every
+    source tree and the supertree (``mast.flat_mast_fit``) is written there as TSV.  The supertree is built once either
+    way."""
     forest = load_forest(in_file)
     if forest.num_trees == 0:  # what construct_supertree says about an empty list (ref: scs.py:63-65)
         msg = "There must be at least one tree to make a supertree."
         raise ValueError(msg)
-    extras = (support_out, triplets_out, taxon_triplets_out, mrp_out, source_rf_out, source_triplets_out)
+    extras = (support_out, triplets_out, taxon_triplets_out, mrp_out, source_rf_out, source_triplets_out, mast_out)
     if all(path is None for path in extras):
         text = supertree_newick_of_forest(forest, weighting.lower(), contract_edges=contract_edges)
         Path(out_file).write_text(text + "\n")
@@ -61,6 +65,9 @@ def run(in_file: str, out_file: str, weighting: str = "branch", contract_edges: 
     if mrp_out is not None:
         score = flat_mrp_score(forest, built["parent"], built["taxon"], engine=engine)
         Path(mrp_out).write_text(score.tsv())
+    if mast_out is not None:
+        fit_mast = flat_mast_fit(forest, built["parent"], built["taxon"], engine=engine)
+        Path(mast_out).write_text(fit_mast.tsv())
     if source_rf_out is not None:
         distances = flat_source_tree_distances(forest, engine=engine)
         Path(source_rf_out).write_text(distances.tsv())
@@ -118,6 +125,12 @@ def run(in_file: str, out_file: str, weighting: str = "branch", contract_edges: 
     help="Also write the rooted triplet distance between every pair of source trees on the taxa they share (TSV).",
     default=None,
 )
+@click.option(
+    "--mast-out",
+    help="Also write, per source tree, the taxa it shares with the supertree and how many of them the largest "
+    "agreement subtree keeps (TSV).",
+    default=None,
+)
 def scs(
     in_file: str,
     out_file: str,
@@ -130,11 +143,12 @@ def scs(
     mrp_out: str | None,
     source_rf_out: str | None,
     source_triplets_out: str | None,
+    mast_out: str | None,
 ) -> None:
     """Run spectral cluster supertree over the given set of source trees."""
     run(in_file, out_file, pcg_weighting, contract_edges=not disable_contraction, support_out=support_out,
         triplets_out=triplets_out, taxon_triplets_out=taxon_triplets_out, mrp_out=mrp_out,
-        source_rf_out=source_rf_out, source_triplets_out=source_triplets_out)
+        source_rf_out=source_rf_out, source_triplets_out=source_triplets_out, mast_out=mast_out)
 
 
 if __name__ == "__main__":

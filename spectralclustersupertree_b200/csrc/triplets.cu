@@ -48,6 +48,16 @@
 // a time.  The stack holds (depth, balance) of the open nodes, at most one per level of S, in shared memory: the same
 // two ints per level as the per-tree triplet row.  A character costs O(rw - lw + 1): |c| when S agrees with it, k at
 // worst.
+//
+// Maximum agreement subtree (scs_supertree_mast).  t' and s' become explicit trees: in an (order, gap depth)
+// sequence a node is a window of positions whose inner gaps are all at least as deep as its shallowest one, a run of
+// equal depths being one polytomy, and it is named by its leftmost shallowest gap, so node ids are gap indices and leaf
+// ids positions (t' positions on one side, S-ranks on the other).  One CTA per tree builds both with a monotone stack
+// (one thread each), then fills mast(u, v) for every internal u of t' and v of s' (Steel & Warnow) in wavefronts of
+// h(u) + h(v), children always lying on a lower level, into a (k - 1)^2 int table indexed by the naming gaps.  A leaf
+// against a node is a range test.  The maximum-weight matching of the children is a closed form when one side has two
+// children (the top two weights of each row); otherwise a warp runs the shortest-augmenting-path Hungarian method with
+// the smaller child list as rows, reading the weights on demand.
 
 #include <algorithm>
 #include <climits>
@@ -67,6 +77,8 @@ constexpr int kMaxRowWarps = 8;
 constexpr size_t kScratchBytes = size_t(1024) << 20;         // per-leaf scratch of one chunk
 constexpr size_t kLeafScratch = 3 * sizeof(int32_t) + 4 * sizeof(int64_t);  // qpos, spos, td + four row counts
 constexpr size_t kMatrixBytes = size_t(256) << 20;           // per-taxon counts of one chunk's trees
+constexpr size_t kTableBytes = size_t(4) << 30;              // MAST regions of one chunk, and the cap of one tree's
+constexpr int kMastThreads = 512, kMastWarps = kMastThreads / 32;
 
 struct TripletArgs {
     // supertree: taxon -> leaf position (-1 if S lacks it), depth of every leaf, sparse table over the depths of the
@@ -98,6 +110,11 @@ struct TripletArgs {
     int32_t *sr;             // [chunk leaves]: S-rank of t' position q
     int32_t *sdep;           // [chunk leaves]: depth in S of the LCA of S-ranks r and r + 1
     int32_t *len;            // [chunk leaves]: length of the character of gap q, 0 if gap q names no character
+    // MAST (with sq, sr, sdep): per tree a region of mtab at moff[t] - moff[t0] ints, laid out by mast_ints
+    const int64_t *moff;     // [trees + 1]
+    const int32_t *mk;       // [trees]: k as counted on the host, which sized the region
+    const int32_t *mhw;      // [trees]: Hungarian width, 0 when no node pair of t' and s' has both degrees >= 3
+    int32_t *mtab;
 };
 
 // One CTA per tree: t' positions, the S positions of its taxa and the depths between t'-neighbours.
@@ -556,6 +573,297 @@ __global__ void mp_reduce(TripletArgs a) {
     }
 }
 
+// A tree's MAST region in ints: the (k - 1)^2 table, the two restricted trees (MastSide, 10 k + 4 ints each), the
+// prefix of one level's cells (k + 2) and per warp six Hungarian arrays of hw + 2 ints.  Nothing when k < 3.
+__host__ __device__ __forceinline__ int64_t mast_side_ints(int k) { return 10 * static_cast<int64_t>(k) + 4; }
+__host__ __device__ __forceinline__ int64_t mast_ints(int k, int hw) {
+    if (k < 3) return 0;
+    const int64_t n = k - 1;
+    const int64_t ints = n * n + 2 * mast_side_ints(k) + (k + 2) + (hw > 0 ? int64_t(kMastWarps) * 6 * (hw + 2) : 0);
+    return (ints + 3) & ~int64_t(3);
+}
+
+// A restricted tree as explicit nodes.  Internal node ids are the gaps that name them, leaf ids are positions (encoded
+// ~p in child lists).  For a naming gap g: leaf range [lo[g], hi[g]], height h[g] and children child[coff[g],
+// coff[g + 1]); the other gaps have no children.  byh lists the internal nodes by height, those of height x at
+// [hoff[x], hoff[x + 1]).  stk and cur are the builder's stack and cursors.
+struct MastSide {
+    int32_t *b;
+    int k;
+    __device__ int32_t *lo() const { return b; }
+    __device__ int32_t *hi() const { return b + k; }
+    __device__ int32_t *h() const { return b + 2 * k; }
+    __device__ int32_t *coff() const { return b + 3 * k; }
+    __device__ int32_t *child() const { return b + 4 * k + 1; }
+    __device__ int32_t *byh() const { return b + 6 * k + 1; }
+    __device__ int32_t *hoff() const { return b + 7 * k + 1; }
+    __device__ int32_t *stk() const { return b + 8 * k + 3; }
+    __device__ int32_t *cur() const { return b + 9 * k + 3; }
+    __device__ int count(int x) const { return hoff()[x + 1] - hoff()[x]; }
+};
+
+// One thread: the nodes of the restricted tree of k >= 3 leaves with gap depths g[0, k - 1) (a monotone stack, replayed
+// once to place the children); returns its height, the root's id in *root.
+__device__ __noinline__ int mast_build(const MastSide &side, const int32_t *g, int k, int *root) {
+    const int n = k - 1;
+    struct {
+        int32_t *lo, *hi, *h, *coff, *child, *byh, *hoff, *stk, *cur;
+    } s{side.lo(), side.hi(), side.h(), side.coff(), side.child(), side.byh(), side.hoff(), side.stk(), side.cur()};
+    for (int i = 0; i <= n; ++i) s.coff[i] = 0;
+    int top = -1, height = 0;
+    for (int i = 0; i < k; ++i) {  // ranges, heights and child counts
+        int cur = ~i, curh = 0, curlo = i;
+        const int d = i < n ? g[i] : -1;
+        while (top >= 0 && g[s.stk[top]] > d) {
+            const int v = s.stk[top--];
+            s.coff[v]++;
+            s.h[v] = max(s.h[v], curh + 1);
+            s.hi[v] = i;
+            cur = v;
+            curh = s.h[v];
+            curlo = s.lo[v];
+        }
+        if (d < 0) {
+            *root = cur;
+            height = curh;
+            break;
+        }
+        if (top < 0 || g[s.stk[top]] < d) {
+            s.stk[++top] = i;
+            s.lo[i] = curlo;
+            s.h[i] = 0;
+        }
+        const int v = s.stk[top];
+        s.coff[v]++;
+        s.h[v] = max(s.h[v], curh + 1);
+    }
+    for (int i = 0, acc = 0; i <= n; ++i) {
+        const int c = s.coff[i];
+        s.coff[i] = acc;
+        s.cur[i] = acc;
+        acc += c;
+    }
+    top = -1;
+    for (int i = 0; i < k; ++i) {  // the same walk, placing each child at its parent's cursor
+        int cur = ~i;
+        const int d = i < n ? g[i] : -1;
+        while (top >= 0 && g[s.stk[top]] > d) {
+            const int v = s.stk[top--];
+            s.child[s.cur[v]++] = cur;
+            cur = v;
+        }
+        if (d < 0) break;
+        if (top < 0 || g[s.stk[top]] < d) s.stk[++top] = i;
+        s.child[s.cur[s.stk[top]]++] = cur;
+    }
+    for (int x = 0; x <= height + 1; ++x) s.hoff[x] = 0;
+    for (int i = 0; i < n; ++i)
+        if (s.coff[i + 1] > s.coff[i]) s.hoff[s.h[i]]++;
+    for (int x = 0, acc = 0; x <= height + 1; ++x) {
+        const int c = s.hoff[x];
+        s.hoff[x] = acc;
+        s.cur[x] = acc;
+        acc += c;
+    }
+    for (int i = 0; i < n; ++i)
+        if (s.coff[i + 1] > s.coff[i]) s.byh[s.cur[s.h[i]]++] = i;
+    return height;
+}
+
+// The table of one tree with the two restricted trees; w(x, y) = mast of t' node x against s' node y when at least
+// one of them is a leaf or both lie on a level already filled.
+struct MastCells {
+    MastSide T, S;
+    const int32_t *sq, *sr;
+    int32_t *tab;
+    int n;
+    __device__ int w(int x, int y) const {
+        if (x >= 0 && y >= 0) return tab[static_cast<int64_t>(x) * n + y];
+        if (x >= 0) {
+            const int q = sq[~y];
+            return q >= T.lo()[x] && q <= T.hi()[x];
+        }
+        if (y >= 0) {
+            const int r = sr[~x];
+            return r >= S.lo()[y] && r <= S.hi()[y];
+        }
+        return sr[~x] == ~y;
+    }
+    // weight of row child i against column child j of the cell (u, v), rows being u's children when rows_t
+    __device__ int rc(bool rows_t, int u, int v, int i, int j) const {
+        return rows_t ? w(T.child()[T.coff()[u] + i], S.child()[S.coff()[v] + j])
+                      : w(T.child()[T.coff()[u] + j], S.child()[S.coff()[v] + i]);
+    }
+};
+
+// The maximum-weight matching of the children of u and v by the whole warp: the shortest-augmenting-path Hungarian
+// method (minimising -w) with the nr <= nc children of one side as rows.  sc: six arrays of nc + 2 <= hw + 2 ints.
+__device__ __noinline__ int mast_hungarian(const MastCells &m, int u, int v, int32_t *sc, int hw) {
+    const int lane = threadIdx.x & 31;
+    const unsigned full = 0xffffffffu;
+    const int p = m.T.coff()[u + 1] - m.T.coff()[u], q = m.S.coff()[v + 1] - m.S.coff()[v];
+    const bool rows_t = p <= q;
+    const int nr = rows_t ? p : q, nc = rows_t ? q : p;
+    const int inf = 0x3fffffff;
+    const int64_t w2 = hw + 2;
+    int32_t *U = sc, *V = sc + w2, *P = sc + 2 * w2, *way = sc + 3 * w2, *minv = sc + 4 * w2, *used = sc + 5 * w2;
+    for (int j = lane; j <= nc; j += 32) V[j] = P[j] = 0;
+    for (int i = lane; i <= nr; i += 32) U[i] = 0;
+    __syncwarp();
+    for (int i = 1; i <= nr; ++i) {
+        for (int j = lane; j <= nc; j += 32) {
+            minv[j] = inf;
+            used[j] = 0;
+        }
+        if (lane == 0) P[0] = i;
+        __syncwarp();
+        int j0 = 0;
+        do {
+            if (lane == 0) used[j0] = 1;
+            __syncwarp();
+            const int i0 = P[j0], ui = U[i0];
+            int delta = inf, j1 = INT_MAX;
+            for (int j = 1 + lane; j <= nc; j += 32) {
+                if (used[j]) continue;
+                const int cur = -m.rc(rows_t, u, v, i0 - 1, j - 1) - ui - V[j];
+                if (cur < minv[j]) {
+                    minv[j] = cur;
+                    way[j] = j0;
+                }
+                if (minv[j] < delta) {
+                    delta = minv[j];
+                    j1 = j;
+                }
+            }
+#pragma unroll
+            for (int off = 16; off > 0; off >>= 1) {
+                const int od = __shfl_xor_sync(full, delta, off), oj = __shfl_xor_sync(full, j1, off);
+                if (od < delta || (od == delta && oj < j1)) {
+                    delta = od;
+                    j1 = oj;
+                }
+            }
+            __syncwarp();
+            for (int j = lane; j <= nc; j += 32) {
+                if (used[j]) {
+                    U[P[j]] += delta;  // the used columns hold distinct rows
+                    V[j] -= delta;
+                } else {
+                    minv[j] -= delta;
+                }
+            }
+            __syncwarp();
+            j0 = j1;
+        } while (P[j0] != 0);
+        if (lane == 0)
+            do {
+                const int j1 = way[j0];
+                P[j0] = P[j1];
+                j0 = j1;
+            } while (j0);
+        __syncwarp();
+    }
+    int total = 0;
+    for (int j = 1 + lane; j <= nc; j += 32)
+        if (P[j]) total += m.rc(rows_t, u, v, P[j] - 1, j - 1);
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) total += __shfl_xor_sync(full, total, off);
+    __syncwarp();
+    return total;
+}
+
+// One CTA per tree of the chunk: its restricted trees, then mast(u, v) for every pair of internal nodes level by level
+// (level h(u) + h(v)); per tree k and mast(root t', root s').
+__global__ void __launch_bounds__(kMastThreads, 1) ma_tree(TripletArgs a) {
+    __shared__ int32_t sums[33];
+    __shared__ int info[4];  // root and height of t', of s'
+    const int w = blockIdx.x, t = a.t0 + w;
+    const int k = a.k[w];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const unsigned full = 0xffffffffu;
+    int64_t *out = a.per_tree + 2 * static_cast<int64_t>(t);
+    if (k < 3 || k != a.mk[t]) {  // at most two shared taxa agree; the region was sized by the host count
+        if (threadIdx.x == 0) {
+            out[0] = k;
+            out[1] = k < 3 ? k : -1;
+        }
+        return;
+    }
+    const int64_t rel = a.leaf_off[t] - a.leaf0;
+    int32_t *base = a.mtab + (a.moff[t] - a.moff[a.t0]);
+    const int n = k - 1, hw = a.mhw[t];
+    MastCells m{{base + static_cast<int64_t>(n) * n, k}, {base + static_cast<int64_t>(n) * n + mast_side_ints(k), k},
+                a.sq + rel, a.sr + rel, base, n};
+    int32_t *pref = base + static_cast<int64_t>(n) * n + 2 * mast_side_ints(k);
+    int32_t *hung = pref + k + 2 + static_cast<int64_t>(warp) * 6 * (hw + 2);
+    if (threadIdx.x == 0) info[1] = mast_build(m.T, a.td + rel, k, &info[0]);
+    if (threadIdx.x == 32) info[3] = mast_build(m.S, a.sdep + rel, k, &info[2]);
+    __syncthreads();
+    const int Ht = info[1], Hs = info[3];
+    for (int L = 2; L <= Ht + Hs; ++L) {
+        // the cells of level L: pairs of heights (x, L - x), x in [xlo, xhi], counted and scanned
+        const int xlo = max(1, L - Hs), xhi = min(Ht, L - 1), nx = xhi - xlo + 1;
+        for (int i = threadIdx.x; i < nx; i += blockDim.x) pref[i] = m.T.count(xlo + i) * m.S.count(L - xlo - i);
+        __syncthreads();
+        const int total = block_scan(pref, nx, sums);
+        for (int b = warp * 32; b < total; b += blockDim.x) {
+            const int f = b + lane;
+            int u = 0, v = 0, best = 0;
+            bool hungarian = false;
+            if (f < total) {
+                int lo = 0, hi = nx - 1;  // the last i with pref[i] <= f
+                while (lo < hi) {
+                    const int mid = (lo + hi + 1) >> 1;
+                    if (pref[mid] <= f) lo = mid; else hi = mid - 1;
+                }
+                const int x = xlo + lo, cs = m.S.count(L - x), rem = f - pref[lo];
+                u = m.T.byh()[m.T.hoff()[x] + rem / cs];
+                v = m.S.byh()[m.S.hoff()[L - x] + rem % cs];
+                const int ub = m.T.coff()[u], ue = m.T.coff()[u + 1], vb = m.S.coff()[v], ve = m.S.coff()[v + 1];
+                for (int i = ub; i < ue; ++i) best = max(best, m.w(m.T.child()[i], v));
+                for (int j = vb; j < ve; ++j) best = max(best, m.w(u, m.S.child()[j]));
+                const int p = ue - ub, q = ve - vb;
+                if (p == 2 || q == 2) {  // rows r0, r1 against the other side: the top two of each row
+                    const bool rows_t = p == 2;
+                    int b0 = -1, s0 = -1, i0 = -1, b1 = -1, s1 = -1, i1 = -1;
+                    for (int j = 0; j < (rows_t ? q : p); ++j) {
+                        const int w0 = m.rc(rows_t, u, v, 0, j), w1 = m.rc(rows_t, u, v, 1, j);
+                        if (w0 > b0) {
+                            s0 = b0;
+                            b0 = w0;
+                            i0 = j;
+                        } else if (w0 > s0) {
+                            s0 = w0;
+                        }
+                        if (w1 > b1) {
+                            s1 = b1;
+                            b1 = w1;
+                            i1 = j;
+                        } else if (w1 > s1) {
+                            s1 = w1;
+                        }
+                    }
+                    best = max(best, i0 != i1 ? b0 + b1 : max(b0 + s1, s0 + b1));
+                    m.tab[static_cast<int64_t>(u) * n + v] = best;
+                } else {
+                    hungarian = true;
+                }
+            }
+            for (unsigned need = __ballot_sync(full, hungarian); need; need &= need - 1) {
+                const int src = __ffs(need) - 1;
+                const int cu = __shfl_sync(full, u, src), cv = __shfl_sync(full, v, src);
+                const int mwm = mast_hungarian(m, cu, cv, hung, hw);
+                if (lane == src) m.tab[static_cast<int64_t>(u) * n + v] = max(best, mwm);
+            }
+        }
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) {
+        out[0] = k;
+        out[1] = m.tab[static_cast<int64_t>(info[0]) * n + info[2]];
+    }
+}
+
 // What both entry points share: the supertree validated and in pre-order, the depth of its leaves and the sparse
 // table over the depths between consecutive leaves, the chunk plan, and on the device the source forest, its tours,
 // those supertree arrays and the per-leaf scratch of a chunk.
@@ -576,6 +884,14 @@ struct TripletPass {
     int prepare(scs_ctx *ctx, const char *name, const scs_forest *sources, int64_t num_nodes, const int32_t *parent,
                 const int32_t *taxon, int arrays, size_t tree_bytes,
                 const char *what = "the shared-memory Fenwick tree of a row") {
+        const int rc = supertree(ctx, name, sources, num_nodes, parent, taxon, arrays, what);
+        if (rc == SCS_OK) plan(sources, tree_bytes);
+        return rc;
+    }
+
+    // The supertree part of `prepare`; arrays = 0 for a pass without row warps.
+    int supertree(scs_ctx *ctx, const char *name, const scs_forest *sources, int64_t num_nodes, const int32_t *parent,
+                  const int32_t *taxon, int arrays, const char *what = "") {
         taxa = sources->num_taxa;
         if (preorder_supertree(num_nodes, parent, taxon, taxa, &s))
             return fail(ctx, SCS_ERR_INPUT, (std::string(name) + ": malformed supertree (parent[i] >= i, a tip without a "
@@ -603,25 +919,35 @@ struct TripletPass {
                                                                  stab[static_cast<size_t>(l - 1) * NL + i + (1 << (l - 1))]);
         // per row warp: `arrays` arrays of max_depth + 1 ints in shared memory (Fenwick trees, histograms)
         stride = max_depth + 1;
+        if (arrays == 0) return SCS_OK;
         const size_t warp_smem = static_cast<size_t>(arrays) * stride * sizeof(int32_t);
         warps = static_cast<int>(std::min<size_t>(kMaxRowWarps, ctx->smem_optin / warp_smem));
         if (warps < 1)
             return fail(ctx, SCS_ERR_INVALID, (std::string(name) + ": the supertree is too deep for " + what).c_str());
         row_smem = static_cast<size_t>(warps) * warp_smem;
+        return SCS_OK;
+    }
 
+    // The chunks: consecutive trees within the per-leaf scratch, tree_bytes per tree within kMatrixBytes and, given
+    // table (bytes per tree, each at most kTableBytes), their sum within kTableBytes.
+    void plan(const scs_forest *sources, size_t tree_bytes, const std::vector<int64_t> *table = nullptr) {
         const std::vector<int64_t> &loff = sources->leaf_offsets;
+        int64_t table_sum = 0;
         for (int t = 0; t < T;) {
             const int b = chunk_begin.back();
             int e = t + 1;
+            if (table) table_sum = (*table)[t];
             while (e < T && static_cast<size_t>(loff[e + 1] - loff[b]) * kLeafScratch <= kScratchBytes &&
-                   static_cast<size_t>(e + 1 - b) * tree_bytes <= kMatrixBytes)
+                   static_cast<size_t>(e + 1 - b) * tree_bytes <= kMatrixBytes &&
+                   (!table || static_cast<size_t>(table_sum + (*table)[e]) <= kTableBytes)) {
+                if (table) table_sum += (*table)[e];
                 ++e;
+            }
             most_leaves = std::max(most_leaves, loff[e] - loff[b]);
             most_trees = std::max<int64_t>(most_trees, e - b);
             chunk_begin.push_back(e);
             t = e;
         }
-        return SCS_OK;
     }
 
     // Uploads and scratch; fills the fields of `args` that do not change from chunk to chunk.
@@ -866,6 +1192,106 @@ extern "C" int scs_supertree_mrp(scs_ctx *ctx, const scs_forest *sources, int64_
     rc = run();
     p.release_all(ctx);
     release(ctx, d_per_tree);
+    cudaStreamSynchronize(ctx->stream);
+    return rc;
+}
+
+extern "C" int scs_supertree_mast(scs_ctx *ctx, const scs_forest *sources, int64_t num_nodes, const int32_t *parent,
+                                  const int32_t *taxon, int64_t *per_tree) {
+    if (!ctx) return SCS_ERR_INVALID;
+    if (!sources || !parent || !taxon || !per_tree || num_nodes <= 0 || num_nodes >= (int64_t(1) << 31))
+        return fail(ctx, SCS_ERR_INVALID, "scs_supertree_mast: bad argument");
+    TripletPass p;
+    int rc = p.supertree(ctx, "scs_supertree_mast", sources, num_nodes, parent, taxon, 0);
+    if (rc) return rc;
+    const int T = p.T, taxa = p.taxa;
+    const int words = (p.s.leaves + 31) / 32;
+    const size_t rank_smem = static_cast<size_t>(words) * 8;
+    if (rank_smem + 1024 > ctx->smem_optin)  // room for the static shared arrays
+        return fail(ctx, SCS_ERR_INVALID, "scs_supertree_mast: the supertree has too many tips for the shared-memory bitmap");
+    // per tree: k from its tips against S, the Hungarian width (restriction never raises a node's out-degree, so the
+    // unrestricted trees bound it) and the ints of its region, refused above the cap before anything runs
+    auto widest = [](const int32_t *par, int64_t nodes) {
+        std::vector<int32_t> kids(static_cast<size_t>(nodes), 0);
+        int most = 0;
+        for (int64_t i = 1; i < nodes; ++i)
+            if (par[i] >= 0 && par[i] < nodes) most = std::max(most, ++kids[par[i]]);
+        return most;
+    };
+    const int deg_s = widest(parent, num_nodes);
+    const std::vector<int64_t> &noff = sources->node_offsets;
+    std::vector<int32_t> hk(static_cast<size_t>(std::max(T, 1)), 0), hw(hk.size(), 0);
+    std::vector<int64_t> bytes(static_cast<size_t>(T), 0), off(static_cast<size_t>(T) + 1, 0);
+    for (int t = 0; t < T; ++t) {
+        int k = 0;
+        for (int64_t i = noff[t]; i < noff[t + 1]; ++i) {
+            const int x = sources->taxon[i];
+            k += x >= 0 && x < taxa && p.s.pos[x] >= 0;
+        }
+        const int deg_t = widest(&sources->parent[noff[t]], noff[t + 1] - noff[t]);
+        hk[t] = k;
+        hw[t] = std::min({deg_s, deg_t, k}) >= 3 ? std::min(std::max(deg_s, deg_t), k) : 0;
+        const int64_t ints = mast_ints(k, hw[t]);
+        bytes[t] = ints * static_cast<int64_t>(sizeof(int32_t));
+        if (static_cast<size_t>(bytes[t]) > kTableBytes)
+            return fail(ctx, SCS_ERR_INVALID, ("scs_supertree_mast: source tree " + std::to_string(t) + " shares " +
+                                               std::to_string(k) + " taxa with the supertree; its agreement table of " +
+                                               std::to_string(bytes[t] >> 20) + " MiB is above the cap of " +
+                                               std::to_string(kTableBytes >> 20) + " MiB").c_str());
+        off[t + 1] = off[t] + ints;
+    }
+    p.plan(sources, 0, &bytes);
+    std::fill(per_tree, per_tree + 2 * static_cast<int64_t>(T), 0);
+    if (T == 0) return SCS_OK;
+
+    GrowBuf d_per_tree, d_off, d_hk, d_hw, table;
+    auto run = [&]() -> int {
+        TripletArgs args{};
+        if ((rc = p.upload(ctx, sources, &args))) return rc;
+        int64_t most = 4;
+        for (size_t c = 0; c + 1 < p.chunk_begin.size(); ++c)
+            most = std::max(most, off[p.chunk_begin[c + 1]] - off[p.chunk_begin[c]]);
+        if ((rc = grow(ctx, d_per_tree, 2 * static_cast<size_t>(T) * sizeof(int64_t))) ||
+            (rc = TripletPass::put(ctx, d_off, off.data(), off.size() * sizeof(int64_t))) ||
+            (rc = TripletPass::put(ctx, d_hk, hk.data(), hk.size() * sizeof(int32_t))) ||
+            (rc = TripletPass::put(ctx, d_hw, hw.data(), hw.size() * sizeof(int32_t))) ||
+            (rc = grow(ctx, table, static_cast<size_t>(most) * sizeof(int32_t))))
+            return rc;
+        if (rank_smem > 48 * 1024)
+            SCS_CUDA(ctx, cudaFuncSetAttribute(mp_rank, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(rank_smem)));
+        // S-ranks and depths between S-rank neighbours in the scratch of the triplet rows, as the MRP pass
+        const int64_t L = p.most_leaves + 1;
+        int32_t *scratch = p.rows.as<int32_t>();
+        args.words = words;
+        args.sq = scratch;
+        args.sr = scratch + L;
+        args.sdep = scratch + 2 * L;
+        args.moff = d_off.as<int64_t>();
+        args.mk = d_hk.as<int32_t>();
+        args.mhw = d_hw.as<int32_t>();
+        args.mtab = table.as<int32_t>();
+        args.per_tree = d_per_tree.as<int64_t>();
+        for (size_t c = 0; c + 1 < p.chunk_begin.size(); ++c) {
+            if ((rc = p.prep_chunk(ctx, sources, c, &args))) return rc;
+            if (args.chunk_leaves > 0) {
+                mp_rank<<<args.t1 - args.t0, kPrepThreads, rank_smem, ctx->stream>>>(args);
+                SCS_LAUNCHED(ctx, "mp_rank");
+            }
+            ma_tree<<<args.t1 - args.t0, kMastThreads, 0, ctx->stream>>>(args);
+            SCS_LAUNCHED(ctx, "ma_tree");
+        }
+        const size_t out_bytes = 2 * static_cast<size_t>(T) * sizeof(int64_t);
+        SCS_CUDA(ctx, cudaMemcpyAsync(per_tree, d_per_tree.ptr, out_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+        SCS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        ctx->d2h_bytes += static_cast<int64_t>(out_bytes);
+        // a lone tip has no tour: it shares one taxon with S or none, and agrees on it
+        for (int t = 0; t < T; ++t)
+            if (noff[t + 1] - noff[t] == 1) per_tree[2 * static_cast<int64_t>(t)] = per_tree[2 * static_cast<int64_t>(t) + 1] = hk[t];
+        return SCS_OK;
+    };
+    rc = run();
+    p.release_all(ctx);
+    for (GrowBuf *b : {&d_per_tree, &d_off, &d_hk, &d_hw, &table}) release(ctx, *b);
     cudaStreamSynchronize(ctx->stream);
     return rc;
 }

@@ -331,6 +331,20 @@ class Engine:
         _check(status, self._ctx)
         return shared, resolved, agree, contradict
 
+    def supertree_mast(self, forest: "Forest", parent, taxon) -> np.ndarray:
+        """``scs_supertree_mast``: per source tree ``[T, 2]`` (int64): shared taxa, and the size of the maximum
+        agreement subtree of the source tree and the supertree, both restricted to those taxa."""
+        parent = np.ascontiguousarray(parent, dtype=np.int32)
+        taxon = np.ascontiguousarray(taxon, dtype=np.int32)
+        n = len(parent)
+        if len(taxon) != n:
+            msg = "parent and taxon must have the same length"
+            raise ValueError(msg)
+        per_tree = np.zeros((forest.num_trees, 2), dtype=np.int64)
+        status = self._lib.scs_supertree_mast(self._ctx, forest.handle, n, ptr(parent), ptr(taxon), ptr(per_tree))
+        _check(status, self._ctx)
+        return per_tree
+
     def _collect_supertree(self, handle, record: bool) -> dict:
         try:
             count = self._lib.scs_supertree_num_nodes(handle)
