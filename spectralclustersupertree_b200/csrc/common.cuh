@@ -236,6 +236,7 @@ int reserve_pinned(scs_ctx *ctx, size_t bytes, void **out);
 
 enum ProfileKind : int { PROFILE_MATVEC = 0, PROFILE_PCG_ROWS = 1, PROFILE_KINDS = 2 };
 constexpr int kSmallNode = 64;  // recursion nodes up to this many vertices take the one-CTA path (small.cu)
+constexpr int kSmallCap32 = 32;  // ... those up to this many the smaller-capacity instance of it
 constexpr int kSmallMaxTrees = 65535;  // ... if they have at most this many source trees (16-bit co-occurrence counts)
 // the per-launch roofline timers cover the launches whose matrix exceeds the 126 MB L2 (8 n^2 bytes > L2 from
 // n = 3969); smaller matrices stay L2-resident across the matvecs of a Lanczos run: no HBM roofline there
@@ -337,13 +338,21 @@ int small_node(scs_ctx *ctx, int n, int contract_edges, const double *W, const u
                const uint32_t *max_bits, int32_t *part, scs_node_stats *out_dev, int32_t *group_out,
                double *Wc_out);
 
-// A batch of small nodes, one CTA each, graph build included; all pointers are device pointers.
+// Launch order of a batch of small nodes (host arrays): the nodes of at most kSmallCap32 vertices first, each group
+// heaviest first (n^2 x trees) so that no heavy node starts in the last round of CTAs.  Returns the size of the first
+// group.
+int small_order(int num_nodes, const scs_small_node *nodes, int32_t *order);
+
+// A batch of small nodes, one CTA each, graph build included; all pointers are device pointers.  order_dev (from
+// small_order, num_cap32 its return value) is the launch order: the first num_cap32 nodes of it run on the
+// 32-capacity kernel, the rest on the 64-capacity one.  order_dev null: every node on the 64-capacity kernel, in
+// descriptor order.  Stats and labels land at each node's own slot either way.
 // absolute_offsets: leaf_offsets[tree_base + t] is the absolute tour position of tree t of a node (the device forest's
 // layout); otherwise node b reads leaf_offsets[tree_base + b + t], relative to its leaf_base (scs_small_node's layout).
-int small_batch(scs_ctx *ctx, int num_nodes, const scs_small_node *nodes_dev, const int64_t *leaf_offsets,
-                const int32_t *leaf_taxon, const int32_t *adj_depth, const double *adj_val, const int32_t *root_depth,
-                const double *tree_weight, int contract_edges, int32_t *part_dev, scs_node_stats *stats_dev,
-                int32_t *bad_dev, int absolute_offsets = 0);
+int small_batch(scs_ctx *ctx, int num_nodes, const scs_small_node *nodes_dev, const int32_t *order_dev, int num_cap32,
+                const int64_t *leaf_offsets, const int32_t *leaf_taxon, const int32_t *adj_depth, const double *adj_val,
+                const int32_t *root_depth, const double *tree_weight, int contract_edges, int32_t *part_dev,
+                scs_node_stats *stats_dev, int32_t *bad_dev, int absolute_offsets = 0);
 
 // SM cycles the batched small-node kernel spent in its graph build / in everything after it, summed over CTAs.
 int small_cycles(scs_ctx *ctx, unsigned long long *out2, int reset);

@@ -459,18 +459,23 @@ class DeviceDriver {
             desc[b].vertex_base = splits[b].part_at;
         }
         int rc;
-        const size_t bytes = sizeof(scs_small_node) * static_cast<size_t>(B);
-        scs_small_node *desc_dev;
-        if ((rc = reserve_as(ctx, SLOT_MED_NODES, static_cast<size_t>(B), &desc_dev))) return rc;
+        // descriptors, then the launch order, in one copy
+        const size_t desc_bytes = sizeof(scs_small_node) * static_cast<size_t>(B);
+        const size_t bytes = desc_bytes + sizeof(int32_t) * static_cast<size_t>(B);
+        unsigned char *desc_dev;
+        if ((rc = reserve_as(ctx, SLOT_MED_NODES, bytes, &desc_dev))) return rc;
         void *pin_v;
         if ((rc = reserve_pinned(ctx, bytes + sizeof(scs_node_stats) * static_cast<size_t>(B) + 512, &pin_v))) return rc;
         unsigned char *pin = static_cast<unsigned char *>(pin_v);
-        std::memcpy(pin, desc.data(), bytes);
+        std::memcpy(pin, desc.data(), desc_bytes);
+        const int num_cap32 = small_order(B, desc.data(), reinterpret_cast<int32_t *>(pin + desc_bytes));
         SCS_CUDA(ctx, cudaMemcpyAsync(desc_dev, pin, bytes, cudaMemcpyHostToDevice, ctx->stream));
         ctx->h2d_bytes += static_cast<int64_t>(bytes);
         scs_node_stats *stats_dev;
         if ((rc = reserve_as(ctx, SLOT_NODE_STATS, static_cast<size_t>(B), &stats_dev))) return rc;
-        rc = small_batch(ctx, B, desc_dev, forest.leaf_off.as<int64_t>(), tours_.leaf_taxon.as<int32_t>(),
+        rc = small_batch(ctx, B, reinterpret_cast<const scs_small_node *>(desc_dev),
+                         reinterpret_cast<const int32_t *>(desc_dev + desc_bytes), num_cap32, forest.leaf_off.as<int64_t>(),
+                         tours_.leaf_taxon.as<int32_t>(),
                          tours_.adj_depth.as<int32_t>(), tours_.adj_val.as<double>(), tours_.root_depth.as<int32_t>(),
                          forest.weight.as<double>(), contract_, part_dev_.as<int32_t>(), stats_dev, flags_dev_.as<int32_t>(), 1);
         if (rc) return rc;

@@ -106,9 +106,10 @@ struct Scratch {
 // says where each array lives in it, so the driver can flatten the tours straight into pinned memory;
 // small_run() copies, launches small_batch_kernel and brings partitions and stats back.
 struct SmallStage {
-    size_t o_nodes = 0, o_off = 0, o_val = 0, o_w = 0, o_tax = 0, o_dep = 0, o_root = 0, total = 0;
+    size_t o_nodes = 0, o_order = 0, o_off = 0, o_val = 0, o_w = 0, o_tax = 0, o_dep = 0, o_root = 0, total = 0;
     unsigned char *base = nullptr;  // pinned host memory
     scs_small_node *nodes() const { return reinterpret_cast<scs_small_node *>(base + o_nodes); }
+    int32_t *order() const { return reinterpret_cast<int32_t *>(base + o_order); }
     int64_t *off() const { return reinterpret_cast<int64_t *>(base + o_off); }
     double *val() const { return reinterpret_cast<double *>(base + o_val); }
     double *w() const { return reinterpret_cast<double *>(base + o_w); }
@@ -120,7 +121,8 @@ struct SmallStage {
 int small_stage(scs_ctx *ctx, int num_nodes, int64_t L_total, int64_t T_total, SmallStage *st) {
     const size_t nB = static_cast<size_t>(num_nodes), nL = static_cast<size_t>(L_total), nT = static_cast<size_t>(T_total);
     st->o_nodes = 0;
-    st->o_off = st->o_nodes + nB * sizeof(scs_small_node);
+    st->o_order = st->o_nodes + nB * sizeof(scs_small_node);
+    st->o_off = st->o_order + ((nB * sizeof(int32_t) + 7) & ~static_cast<size_t>(7));
     st->o_val = st->o_off + (nT + nB) * sizeof(int64_t);
     st->o_w = st->o_val + nL * sizeof(double);
     st->o_tax = st->o_w + nT * sizeof(double);
@@ -156,6 +158,7 @@ int small_run(scs_ctx *ctx, int num_nodes, const SmallStage &st, int contract_ed
     const size_t nB = static_cast<size_t>(num_nodes);
     unsigned char *dev;
     int rc;
+    const int num_cap32 = small_order(num_nodes, nodes, st.order());
     if ((rc = reserve_as(ctx, SLOT_TOUR_OFFSETS, st.total, &dev))) return rc;
     SCS_CUDA(ctx, cudaMemcpyAsync(dev, st.base, st.total - 64, cudaMemcpyHostToDevice, ctx->stream));
     ctx->h2d_bytes += static_cast<int64_t>(st.total - 64);
@@ -167,6 +170,7 @@ int small_run(scs_ctx *ctx, int num_nodes, const SmallStage &st, int contract_ed
     if ((rc = reserve_as(ctx, SLOT_SCALARS, 64, &bad_dev))) return rc;
     SCS_CUDA(ctx, cudaMemsetAsync(bad_dev, 0, sizeof(int32_t), ctx->stream));
     rc = small_batch(ctx, num_nodes, reinterpret_cast<const scs_small_node *>(dev + st.o_nodes),
+                     reinterpret_cast<const int32_t *>(dev + st.o_order), num_cap32,
                      reinterpret_cast<const int64_t *>(dev + st.o_off), reinterpret_cast<const int32_t *>(dev + st.o_tax),
                      reinterpret_cast<const int32_t *>(dev + st.o_dep), reinterpret_cast<const double *>(dev + st.o_val),
                      reinterpret_cast<const int32_t *>(dev + st.o_root), reinterpret_cast<const double *>(dev + st.o_w),
@@ -954,7 +958,7 @@ int scs_nodes_split_small_dev(scs_ctx *ctx, int num_nodes, const scs_small_node 
     int32_t *bad_dev;
     int rc;
     if ((rc = reserve_as(ctx, SLOT_SCALARS, 64, &bad_dev))) return rc;
-    return small_batch(ctx, num_nodes, nodes_dev, leaf_offsets_dev, leaf_taxon_dev, adj_depth_dev, adj_val_dev,
+    return small_batch(ctx, num_nodes, nodes_dev, nullptr, 0, leaf_offsets_dev, leaf_taxon_dev, adj_depth_dev, adj_val_dev,
                        root_depth_dev, tree_weight_dev, contract_edges, part_dev, stats_dev, bad_dev);
 }
 

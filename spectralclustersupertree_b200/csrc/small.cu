@@ -15,46 +15,79 @@
 //    next eigenvalue is exact as well (exact repeated-eigenvalue detection);
 //  * sign flip and exact 1-D 2-means as in spectral.cu.
 
+#include <algorithm>
+#include <numeric>
+
 #include "common.cuh"
 
 namespace scs {
 
 namespace {
 
-constexpr int kN = kSmallNode;  // 64
-constexpr int kThreads = 256;
+constexpr int kThreads = 256;  // fixed for both capacities: the Jacobi convergence sums are associated by it
+constexpr int kWarps = kThreads / 32;
 constexpr double kGapTie = 1e-7;
 constexpr double kMarginTie = 1e-9;
 
-struct SmallShared {
-    double A[kN][kN + 1];   // W, then Wc, then M (padded: column sweeps hit distinct banks)
-    double V[kN][kN + 1];   // Jacobi eigenvectors
-    double B[kN][kN + 1];   // the (contracted) weights the split was computed from: residual check
-    unsigned short cnt[kN][kN];  // co-occurrence counts (batched path: graph built in shared memory)
-    int occ[kN];
-    int tour_taxon[kN], tour_depth[kN];
-    double tour_val[kN];
-    double cs[kN / 2][2];
-    double deg[kN], isd[kN], q0[kN], u[kN], sorted[kN];
-    unsigned long long adj[kN], mx[kN], reach[kN];
-    int label[kN], group[kN], member_of[kN], side[kN];
-    double red[kThreads / 32 + 1];
-    int ired[4];
+// A chunk of a node's source trees staged for the graph build: their tours in input order, concatenated.
+template <int CAP>
+struct TourChunk {
+    static constexpr int kLeaves = 16 * CAP;  // a chunk always takes at least one well-formed tree (k <= n <= CAP)
+    static constexpr int kTrees = kThreads;   // one thread per tree reads the offsets: at most kThreads trees
+    static constexpr int kLevels = CAP == 32 ? 4 : 5;  // sparse-table levels 1 .. kLevels cover gap runs up to CAP - 1
+    int taxon[kLeaves], depth[kLeaves];
+    double val[kLeaves];
+    int start[kTrees], k[kTrees], rd[kTrees];
+    double w[kTrees];
+    long long span[kLevels][kLeaves];  // span[L - 1][e]: the least gap key of gaps e .. e + 2^L - 1
 };
 
-__device__ __forceinline__ double block_sum_small(double v, double *red) {
+template <int CAP>
+struct SmallShared {
+    double A[CAP][CAP + 1];  // W, then Wc, then M (padded: column sweeps hit distinct banks)
+    union {
+        struct {
+            double V[CAP][CAP + 1];  // Jacobi eigenvectors
+            double B[CAP][CAP + 1];  // the (contracted) weights the split was computed from: residual check
+        };
+        TourChunk<CAP> tours;        // graph build only (batched path), done before V and B are used
+    };
+    unsigned short cnt[CAP][CAP];    // co-occurrence counts (batched path: graph built in shared memory)
+    int occ[CAP];
+    double cs[CAP / 2][2];
+    double deg[CAP], isd[CAP], q0[CAP], u[CAP], sorted[CAP];
+    unsigned long long adj[CAP], mx[CAP], reach[CAP];
+    int label[CAP], group[CAP], member_of[CAP], side[CAP];
+    double red[2 * (kThreads / 32) + 2];
+    int ired[4];
+    long long clock_start;  // batched kernel, thread 0: profiling counters
+};
+
+// Two block sums at once, each associated as before: thread partials, a shuffle tree per warp, then the warp
+// partials in order -- the Jacobi sweep count depends on these bits.
+__device__ __forceinline__ void block_sum2_small(double &x, double &y, double *red) {
+    constexpr int W = kThreads / 32;
 #pragma unroll
-    for (int off = 16; off > 0; off >>= 1) v += __shfl_down_sync(0xffffffffu, v, off);
-    __syncthreads();
-    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = v;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        double s = 0.0;
-        for (int w = 0; w < kThreads / 32; ++w) s += red[w];
-        red[kThreads / 32] = s;
+    for (int off = 16; off > 0; off >>= 1) {
+        x += __shfl_down_sync(0xffffffffu, x, off);
+        y += __shfl_down_sync(0xffffffffu, y, off);
     }
     __syncthreads();
-    return red[kThreads / 32];
+    if ((threadIdx.x & 31) == 0) {
+        red[threadIdx.x >> 5] = x;
+        red[W + (threadIdx.x >> 5)] = y;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double s = 0.0, t = 0.0;
+        for (int w = 0; w < W; ++w) s += red[w];
+        for (int w = 0; w < W; ++w) t += red[W + w];
+        red[2 * W] = s;
+        red[2 * W + 1] = t;
+    }
+    __syncthreads();
+    x = red[2 * W];
+    y = red[2 * W + 1];
 }
 
 // reach[v] = bit set of the vertices connected to v (v included); label[v] = smallest of them
@@ -62,7 +95,7 @@ __device__ void closure(int n, const unsigned long long *rows, unsigned long lon
     const int v = threadIdx.x;
     if (v < n) reach[v] = rows[v] | (1ull << v);
     __syncthreads();
-    for (int round = 0; round < 6; ++round) {  // path lengths double every round: 2^6 >= 64
+    for (int len = 1; len < n - 1; len <<= 1) {  // path lengths double every round, up to n - 1
         unsigned long long acc = 0;
         if (v < n) {
             unsigned long long bits = reach[v];
@@ -81,10 +114,18 @@ __device__ void closure(int n, const unsigned long long *rows, unsigned long lon
     __syncthreads();
 }
 
+// Pair k of round-robin round `step` over me (even) players, p < q; q == me - 1 >= m is a bye.
+__device__ __forceinline__ void round_robin_pair(int me, int step, int k, int &p, int &q) {
+    if (k == 0) { p = me - 1; q = step; }
+    else { p = (step + k) % (me - 1); q = (step - k + (me - 1)) % (me - 1); }
+    if (p > q) { const int t = p; p = q; q = t; }
+}
+
 // Everything after the graph build for one node whose weights are in S.A (n x n) and whose adjacency /
 // max-graph rows are in S.adj / S.mx.  part, out, group_out, Wc_out are global pointers (the last two
 // may be null).
-__device__ void small_finish(SmallShared &S, int n, int contract_edges, int32_t *__restrict__ part,
+template <int CAP>
+__device__ void small_finish(SmallShared<CAP> &S, int n, int contract_edges, int32_t *__restrict__ part,
                              scs_node_stats *__restrict__ out, int32_t *__restrict__ group_out,
                              double *__restrict__ Wc_out) {
     const int tid = threadIdx.x;
@@ -237,8 +278,7 @@ __device__ void small_finish(SmallShared &S, int n, int contract_edges, int32_t 
             const double x = S.A[i][j];
             if (i == j) diag += x * x; else off += x * x;
         }
-        off = block_sum_small(off, S.red);
-        diag = block_sum_small(diag, S.red);
+        block_sum2_small(off, diag, S.red);
         // off-diagonal Frobenius norm below 1e-14 of the whole: eigenvalues are then converged to
         // rounding (their error is quadratic in it) and eigenvectors to ~1e-14 / gap
         if (off <= 1e-28 * (diag + off) || off < 1e-300) break;
@@ -246,9 +286,7 @@ __device__ void small_finish(SmallShared &S, int n, int contract_edges, int32_t 
         for (int step = 0; step < me - 1; ++step) {
             if (tid < half) {
                 int p, q;
-                if (tid == 0) { p = me - 1; q = step; }
-                else { p = (step + tid) % (me - 1); q = (step - tid + (me - 1)) % (me - 1); }
-                if (p > q) { const int t = p; p = q; q = t; }
+                round_robin_pair(me, step, tid, p, q);
                 double c = 1.0, s = 0.0;
                 if (q < m) {
                     const double apq = S.A[p][q];
@@ -267,9 +305,7 @@ __device__ void small_finish(SmallShared &S, int n, int contract_edges, int32_t 
             for (int e = tid; e < m * half; e += kThreads) {
                 const int r = e / half, k = e % half;
                 int p, q;
-                if (k == 0) { p = me - 1; q = step; }
-                else { p = (step + k) % (me - 1); q = (step - k + (me - 1)) % (me - 1); }
-                if (p > q) { const int t = p; p = q; q = t; }
+                round_robin_pair(me, step, k, p, q);
                 if (q >= m) continue;
                 const double c = S.cs[k][0], s = S.cs[k][1];
                 const double arp = S.A[r][p], arq = S.A[r][q];
@@ -284,9 +320,7 @@ __device__ void small_finish(SmallShared &S, int n, int contract_edges, int32_t 
             for (int e = tid; e < m * half; e += kThreads) {
                 const int r = e / half, k = e % half;
                 int p, q;
-                if (k == 0) { p = me - 1; q = step; }
-                else { p = (step + k) % (me - 1); q = (step - k + (me - 1)) % (me - 1); }
-                if (p > q) { const int t = p; p = q; q = t; }
+                round_robin_pair(me, step, k, p, q);
                 if (q >= m) continue;
                 const double c = S.cs[k][0], s = S.cs[k][1];
                 const double apr = S.A[p][r], aqr = S.A[q][r];
@@ -413,7 +447,7 @@ small_node_kernel(int n, int words, int contract_edges, const double *__restrict
                   int32_t *__restrict__ part, scs_node_stats *__restrict__ out,
                   int32_t *__restrict__ group_out, double *__restrict__ Wc_out) {
     extern __shared__ __align__(16) unsigned char raw[];
-    SmallShared &S = *reinterpret_cast<SmallShared *>(raw);
+    SmallShared<kSmallNode> &S = *reinterpret_cast<SmallShared<kSmallNode> *>(raw);
     const int tid = threadIdx.x;
     for (int e = tid; e < n * n; e += kThreads) S.A[e / n][e % n] = W[e];
     if (tid < n) {
@@ -434,31 +468,53 @@ small_node_kernel(int n, int words, int contract_edges, const double *__restrict
 // scs_debug_small_cycles).
 __device__ unsigned long long g_small_cycles[2];
 
+// (depth, position) of the gap after chunk position e, ordered so that the minimum is the leftmost shallowest gap
+__device__ __forceinline__ long long gap_key(int depth, int e) {
+    return static_cast<long long>(depth) * 4294967296ll + e;
+}
+
+// least gap key over gaps e .. e + 2^L - 1 of the staged chunk
+template <int CAP>
+__device__ __forceinline__ long long span_key(const TourChunk<CAP> &C, int L, int e) {
+    return L == 0 ? gap_key(C.depth[e], e) : C.span[L - 1][e];
+}
+
 // ---- batched entry: one CTA per node builds the node's graph from its leaf tours in shared memory
 //      (the reference's _proper_cluster_graph_edges, scs.py:495-663) and finishes it ------------------
-// Trees are taken in input order with a barrier between them; inside a tree thread i owns the pairs
-// (i, j > i) and walks j upwards with a running minimum of the consecutive-leaf LCA depths, so every
-// W entry receives its terms in tree order with separately rounded multiply and add -- the same sums,
-// bit for bit, as pcg_rows_kernel and the reference.
-__global__ void __launch_bounds__(kThreads)
-small_batch_kernel(const scs_small_node *__restrict__ nodes, const int64_t *__restrict__ leaf_offsets,
-                   const int32_t *__restrict__ leaf_taxon, const int32_t *__restrict__ adj_depth,
-                   const double *__restrict__ adj_val, const int32_t *__restrict__ root_depth,
-                   const double *__restrict__ tree_weight, int contract_edges, int32_t *__restrict__ part,
-                   scs_node_stats *__restrict__ stats, int32_t *__restrict__ bad, int absolute_offsets) {
+// The node's trees are staged in chunks, and a sparse table of the gap keys (least key over every run of 2^L gaps) is
+// built over each chunk: a few barriers per chunk, none per tree.  Warp w owns the rows a with a % kWarps == w (their
+// W and count cells and occ[a]) and walks the chunk's trees in input order; for a row at tour position p of a tree,
+// lane l holds positions l*E .. l*E + E - 1, and two table entries give every other position j the leftmost
+// shallowest gap between p and j: the LCA of the two leaves.  Entries that run past a tree's last gap are never read
+// (a query stays inside the gaps between the two leaves).  So every W entry
+// receives its terms in tree order with separately rounded multiply and add -- the same sums, bit for bit, as
+// pcg_rows_kernel and the reference -- and both triangles are built directly.
+// order (may be null: identity) lists the batch's nodes in launch order; CTA b runs node order[first + b].
+template <int CAP>
+__global__ void __launch_bounds__(kThreads, CAP == 32 ? 4 : 2)
+small_batch_kernel(const scs_small_node *__restrict__ nodes, const int32_t *__restrict__ order, int first,
+                   const int64_t *__restrict__ leaf_offsets, const int32_t *__restrict__ leaf_taxon,
+                   const int32_t *__restrict__ adj_depth, const double *__restrict__ adj_val,
+                   const int32_t *__restrict__ root_depth, const double *__restrict__ tree_weight, int contract_edges,
+                   int32_t *__restrict__ part, scs_node_stats *__restrict__ stats, int32_t *__restrict__ bad,
+                   int absolute_offsets) {
+    constexpr int E = CAP / 32;  // tour positions per lane
+    constexpr int kLeaves = TourChunk<CAP>::kLeaves;
     extern __shared__ __align__(16) unsigned char raw[];
-    SmallShared &S = *reinterpret_cast<SmallShared *>(raw);
-    const int tid = threadIdx.x;
-    const scs_small_node node = nodes[blockIdx.x];
+    SmallShared<CAP> &S = *reinterpret_cast<SmallShared<CAP> *>(raw);
+    TourChunk<CAP> &C = S.tours;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int b = order ? order[first + blockIdx.x] : first + static_cast<int>(blockIdx.x);
+    const scs_small_node node = nodes[b];
     const int n = node.n;
-    const long long clock_start = clock64();
-    if (node.num_trees > kSmallMaxTrees || n < 1 || n > kN) {
+    if (tid == 0) S.clock_start = clock64();
+    if (node.num_trees > kSmallMaxTrees || n < 1 || n > CAP) {
         // the co-occurrence counts are 16-bit here (the staged path switches to 32-bit counts at 65 536 trees,
         // pcg.cu `narrow`); the host entry points route such nodes to the staged path -- refuse loudly if one
         // arrives anyway
         if (tid == 0) {
             *bad = 1;
-            stats[blockIdx.x].solver = -1;
+            stats[b].solver = -1;
         }
         return;
     }
@@ -467,80 +523,119 @@ small_batch_kernel(const scs_small_node *__restrict__ nodes, const int64_t *__re
         S.cnt[e / n][e % n] = 0;
     }
     if (tid < n) S.occ[tid] = 0;
-    __syncthreads();
     // T + 1 offsets per node, relative to its first leaf -- or the forest's absolute offsets
-    const int64_t *offs = leaf_offsets + node.tree_base + (absolute_offsets ? 0 : blockIdx.x);
+    const int64_t *offs = leaf_offsets + node.tree_base + (absolute_offsets ? 0 : b);
     const int64_t leaf_base = absolute_offsets ? 0 : node.leaf_base;
-    for (int t = 0; t < node.num_trees; ++t) {
-        const int64_t tb = leaf_base + offs[t];
-        const int k = static_cast<int>(offs[t + 1] - offs[t]);
-        const double w = tree_weight[node.tree_base + t];
-        const int rd = root_depth[node.tree_base + t];
-        if (k > n) {  // more leaves than vertices: malformed input
+    for (int t0 = 0; t0 < node.num_trees;) {
+        // the chunk: trees t0 .. t0 + count - 1, as many as have their leaves within kLeaves of the chunk's first
+        const int64_t begin = offs[t0];
+        const int t = t0 + tid;
+        const bool fits = t < node.num_trees && offs[t + 1] - begin <= kLeaves;
+        const int count = __syncthreads_count(fits);  // also: the previous chunk is done with the staging area
+        if (count == 0) {  // one tree longer than a chunk has more leaves than vertices: malformed input
             if (tid == 0) *bad = 1;
+            ++t0;
             continue;
         }
-        if (tid < k) {
-            const int a = leaf_taxon[tb + tid];
-            S.tour_taxon[tid] = a;
-            S.tour_depth[tid] = adj_depth[tb + tid];
-            S.tour_val[tid] = adj_val[tb + tid];
+        if (tid < count) {
+            C.start[tid] = static_cast<int>(offs[t] - begin);
+            C.k[tid] = static_cast<int>(offs[t + 1] - offs[t]);
+            C.w[tid] = tree_weight[node.tree_base + t];
+            C.rd[tid] = root_depth[node.tree_base + t];
+        }
+        const int total = static_cast<int>(offs[t0 + count] - begin);
+        for (int e = tid; e < total; e += kThreads) {
+            const int64_t g = leaf_base + begin + e;
+            const int a = leaf_taxon[g];
+            C.taxon[e] = a;
+            C.depth[e] = adj_depth[g];
+            C.val[e] = adj_val[g];
             if (a < 0 || a >= n) *bad = 1;
         }
         __syncthreads();
-        // four threads share a leaf i: each walks the whole staircase (the running minimum needs every j) but adds
-        // only every fourth pair; a pair is stored once, at [smaller vertex][larger vertex], and mirrored after the
-        // last tree -- every entry still receives its terms in tree order, one rounded multiply and one rounded add
-        // each, so the sums are the reference's bit for bit
-        const int i = tid & (kN - 1), q = tid >> 6;
-        if (i < k) {
-            const int a = S.tour_taxon[i];
-            if (a >= 0 && a < n) {
-                if (q == 0) S.occ[a] += 1;
-                int best_depth = 0x7fffffff, best_idx = i;
-                for (int j = i + 1; j < k; ++j) {
-                    const int d = S.tour_depth[j - 1];
-                    if (d < best_depth) { best_depth = d; best_idx = j - 1; }  // leftmost shallowest entry
-                    if (best_depth == rd) break;  // the root separates everything further right too
-                    if (((j - i - 1) & 3) != q) continue;
-                    const int b = S.tour_taxon[j];
-                    if (b < 0 || b >= n) continue;
-                    const int lo = min(a, b), hi = max(a, b);
-                    S.A[lo][hi] = __dadd_rn(S.A[lo][hi], __dmul_rn(S.tour_val[best_idx], w));
-                    S.cnt[lo][hi] += 1;
+        for (int L = 1; L <= TourChunk<CAP>::kLevels; ++L) {
+            const int h = 1 << (L - 1);
+            for (int e = tid; e < total; e += kThreads)
+                C.span[L - 1][e] = min(span_key(C, L - 1, e), span_key(C, L - 1, min(e + h, total - 1)));
+            __syncthreads();
+        }
+        for (int i = 0; i < count; ++i) {  // trees in input order
+            const int k = C.k[i];
+            if (k > n) {  // more leaves than vertices: malformed input
+                if (tid == 0) *bad = 1;
+                continue;
+            }
+            const int base = C.start[i], rd = C.rd[i];
+            const double w = C.w[i];
+            int tx[E];
+            unsigned rows[E];
+#pragma unroll
+            for (int e = 0; e < E; ++e) {
+                const int j = lane * E + e;
+                tx[e] = j < k ? C.taxon[base + j] : -1;
+                rows[e] = __ballot_sync(0xffffffffu, tx[e] >= 0 && tx[e] < n && tx[e] % kWarps == warp);
+            }
+#pragma unroll
+            for (int e0 = 0; e0 < E; ++e0) {
+                for (unsigned bits = rows[e0]; bits; bits &= bits - 1) {
+                    const int p = (__ffs(bits) - 1) * E + e0;  // the row's tour position
+                    const int a = C.taxon[base + p];
+                    if (lane == 0) S.occ[a] += 1;
+#pragma unroll
+                    for (int e = 0; e < E; ++e) {
+                        const int j = lane * E + e;
+                        const int bj = tx[e];
+                        if (j == p || bj < 0 || bj >= n) continue;
+                        // gaps lo .. hi - 1 lie between the two leaves: two overlapping runs of 2^L gaps cover them
+                        const int lo = base + min(j, p), hi = base + max(j, p);
+                        const int L = 31 - __clz(hi - lo);
+                        const long long kk = min(span_key(C, L, lo), span_key(C, L, hi - (1 << L)));
+                        const int depth = static_cast<int>(kk >> 32);
+                        if (depth == rd) continue;  // the LCA is the root: no edge (scs.py:552-556)
+                        const int at = static_cast<int>(kk & 0xffffffffll);
+                        S.A[a][bj] = __dadd_rn(S.A[a][bj], __dmul_rn(C.val[at], w));
+                        S.cnt[a][bj] += 1;
+                    }
                 }
             }
         }
-        __syncthreads();
-    }
-    for (int e = tid; e < n * n; e += kThreads) {  // mirror the upper triangle
-        const int r = e / n, c = e % n;
-        if (r > c) {
-            S.A[r][c] = S.A[c][r];
-            S.cnt[r][c] = S.cnt[c][r];
-        }
+        t0 += count;
     }
     __syncthreads();
     if (tid < n) {
         unsigned long long a = 0, m = 0;
         const int occ_a = S.occ[tid];
-        for (int b = 0; b < n; ++b) {
-            const int c = S.cnt[tid][b];
-            if (c > 0) {
-                a |= 1ull << b;
-                if (c == max(occ_a, S.occ[b])) m |= 1ull << b;
+        for (int c = 0; c < n; ++c) {
+            const int k = S.cnt[tid][c];
+            if (k > 0) {
+                a |= 1ull << c;
+                if (k == max(occ_a, S.occ[c])) m |= 1ull << c;
             }
         }
         S.adj[tid] = a;
         S.mx[tid] = contract_edges ? m : 0ull;
     }
     __syncthreads();
-    const long long clock_built = clock64();
-    small_finish(S, n, contract_edges, part + node.vertex_base, stats + blockIdx.x, nullptr, nullptr);
     if (tid == 0) {
-        atomicAdd(&g_small_cycles[0], static_cast<unsigned long long>(clock_built - clock_start));
-        atomicAdd(&g_small_cycles[1], static_cast<unsigned long long>(clock64() - clock_built));
+        const long long clock_built = clock64();
+        atomicAdd(&g_small_cycles[0], static_cast<unsigned long long>(clock_built - S.clock_start));
+        S.clock_start = clock_built;
     }
+    small_finish(S, n, contract_edges, part + node.vertex_base, stats + b, nullptr, nullptr);
+    if (tid == 0) atomicAdd(&g_small_cycles[1], static_cast<unsigned long long>(clock64() - S.clock_start));
+}
+
+template <int CAP>
+int launch_small_batch(scs_ctx *ctx, int count, int first, const scs_small_node *nodes_dev, const int32_t *order_dev,
+                       const int64_t *leaf_offsets, const int32_t *leaf_taxon, const int32_t *adj_depth,
+                       const double *adj_val, const int32_t *root_depth, const double *tree_weight, int contract_edges,
+                       int32_t *part_dev, scs_node_stats *stats_dev, int32_t *bad_dev, int absolute_offsets) {
+    if (count <= 0) return SCS_OK;
+    small_batch_kernel<CAP><<<count, kThreads, sizeof(SmallShared<CAP>), ctx->stream>>>(
+        nodes_dev, order_dev, first, leaf_offsets, leaf_taxon, adj_depth, adj_val, root_depth, tree_weight,
+        contract_edges, part_dev, stats_dev, bad_dev, absolute_offsets);
+    SCS_LAUNCHED(ctx, "small_batch_kernel");
+    return SCS_OK;
 }
 
 }  // namespace
@@ -549,7 +644,7 @@ int small_node(scs_ctx *ctx, int n, int contract_edges, const double *W, const u
                const uint32_t *max_bits, int32_t *part, scs_node_stats *out_dev, int32_t *group_out,
                double *Wc_out) {
     if (n < 1 || n > kSmallNode) return fail(ctx, SCS_ERR_INVALID, "small_node: size out of range");
-    const size_t smem = sizeof(SmallShared);
+    const size_t smem = sizeof(SmallShared<kSmallNode>);
     if (!ctx->small_configured) {
         SCS_CUDA(ctx, cudaFuncSetAttribute(small_node_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                            static_cast<int>(smem)));
@@ -572,22 +667,38 @@ int small_cycles(scs_ctx *ctx, unsigned long long *out2, int reset) {
     return SCS_OK;
 }
 
-int small_batch(scs_ctx *ctx, int num_nodes, const scs_small_node *nodes_dev, const int64_t *leaf_offsets,
-                const int32_t *leaf_taxon, const int32_t *adj_depth, const double *adj_val, const int32_t *root_depth,
-                const double *tree_weight, int contract_edges, int32_t *part_dev, scs_node_stats *stats_dev,
-                int32_t *bad_dev, int absolute_offsets) {
+int small_order(int num_nodes, const scs_small_node *nodes, int32_t *order) {
+    std::iota(order, order + num_nodes, 0);
+    const auto cost = [nodes](int32_t b) { return static_cast<int64_t>(nodes[b].n) * nodes[b].n * nodes[b].num_trees; };
+    std::stable_sort(order, order + num_nodes, [&](int32_t x, int32_t y) {
+        const bool bx = nodes[x].n > kSmallCap32, by = nodes[y].n > kSmallCap32;
+        return bx != by ? by : cost(x) > cost(y);
+    });
+    int count = 0;
+    for (int b = 0; b < num_nodes; ++b) count += nodes[b].n <= kSmallCap32;
+    return count;
+}
+
+int small_batch(scs_ctx *ctx, int num_nodes, const scs_small_node *nodes_dev, const int32_t *order_dev, int num_cap32,
+                const int64_t *leaf_offsets, const int32_t *leaf_taxon, const int32_t *adj_depth, const double *adj_val,
+                const int32_t *root_depth, const double *tree_weight, int contract_edges, int32_t *part_dev,
+                scs_node_stats *stats_dev, int32_t *bad_dev, int absolute_offsets) {
     if (num_nodes <= 0) return SCS_OK;
-    const size_t smem = sizeof(SmallShared);
+    if (!order_dev) num_cap32 = 0;  // launch order unknown on the host: every node takes the 64-capacity kernel
     if (!ctx->batch_configured) {
-        SCS_CUDA(ctx, cudaFuncSetAttribute(small_batch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                           static_cast<int>(smem)));
+        SCS_CUDA(ctx, cudaFuncSetAttribute(small_batch_kernel<kSmallCap32>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                           static_cast<int>(sizeof(SmallShared<kSmallCap32>))));
+        SCS_CUDA(ctx, cudaFuncSetAttribute(small_batch_kernel<kSmallNode>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                           static_cast<int>(sizeof(SmallShared<kSmallNode>))));
         ctx->batch_configured = true;
     }
-    small_batch_kernel<<<num_nodes, kThreads, smem, ctx->stream>>>(nodes_dev, leaf_offsets, leaf_taxon, adj_depth,
-                                                                  adj_val, root_depth, tree_weight, contract_edges,
-                                                                  part_dev, stats_dev, bad_dev, absolute_offsets);
-    SCS_LAUNCHED(ctx, "small_batch_kernel");
-    return SCS_OK;
+    int rc = launch_small_batch<kSmallCap32>(ctx, num_cap32, 0, nodes_dev, order_dev, leaf_offsets, leaf_taxon,
+                                             adj_depth, adj_val, root_depth, tree_weight, contract_edges, part_dev,
+                                             stats_dev, bad_dev, absolute_offsets);
+    if (rc) return rc;
+    return launch_small_batch<kSmallNode>(ctx, num_nodes - num_cap32, num_cap32, nodes_dev, order_dev, leaf_offsets,
+                                          leaf_taxon, adj_depth, adj_val, root_depth, tree_weight, contract_edges,
+                                          part_dev, stats_dev, bad_dev, absolute_offsets);
 }
 
 }  // namespace scs
