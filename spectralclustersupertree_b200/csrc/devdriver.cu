@@ -66,6 +66,8 @@ struct DriverCache {
     DevForest forest[2];
     DevTours tours;
     GrowBuf vertex_dev, offsets_rel, part_dev, flags_dev;
+    void *vertex_pin = nullptr;  // pinned staging of the vertex ids
+    size_t vertex_pin_bytes = 0;
     scs_device_forest resident;
 };
 
@@ -77,6 +79,7 @@ void release_driver_cache(scs_ctx *ctx, void *raw) {
     for (GrowBuf *b : {&cache->vertex_dev, &cache->offsets_rel, &cache->part_dev, &cache->flags_dev}) release(ctx, *b);
     cache->resident.trees.free_all(ctx);
     cudaStreamSynchronize(ctx->stream);
+    if (cache->vertex_pin) cudaFreeHost(cache->vertex_pin);
     delete cache;
 }
 
@@ -249,7 +252,7 @@ class DeviceDriver {
                         const std::vector<int32_t> &taxa = wave[i].taxa;
                         for (size_t v = 0; v < taxa.size(); ++v) vertex_[taxa[v]] = static_cast<int32_t>(v);
                     }
-                if ((rc = upload_ints(vertex_dev_, vertex_.data(), vertex_.size()))) return rc;
+                if ((rc = upload_vertex_ids())) return rc;
                 if ((rc = devforest_tours(ctx_, forest, weighting_, vertex_dev_.as<int32_t>(), &tours_, flags_dev_.as<int32_t>())))
                     return rc;
             }
@@ -351,16 +354,25 @@ class DeviceDriver {
         return plan_children(wave, splits, next);
     }
 
-    int upload_ints(GrowBuf &dev, const int32_t *host, size_t count) {
+    // The vertex ids go through a pinned block of their own, which nothing else writes: the copy stays asynchronous.  The
+    // next wave rewrites the block only after the label copy of this wave has synchronised the stream.
+    int upload_vertex_ids() {
+        const size_t bytes = vertex_.size() * sizeof(int32_t);
         int rc;
-        if ((rc = grow(ctx_, dev, count * sizeof(int32_t)))) return rc;
-        void *pin_v;
-        if ((rc = reserve_pinned(ctx_, count * sizeof(int32_t) + 256, &pin_v))) return rc;
-        std::memcpy(pin_v, host, count * sizeof(int32_t));
-        SCS_CUDA(ctx_, cudaMemcpyAsync(dev.ptr, pin_v, count * sizeof(int32_t), cudaMemcpyHostToDevice, ctx_->stream));
-        // the pinned block is reused by the calls that follow: the copy must have left it
-        SCS_CUDA(ctx_, cudaStreamSynchronize(ctx_->stream));
-        ctx_->h2d_bytes += static_cast<int64_t>(count * sizeof(int32_t));
+        if ((rc = grow(ctx_, vertex_dev_, bytes))) return rc;
+        if (cache_.vertex_pin_bytes < bytes) {
+            if (cache_.vertex_pin) {
+                SCS_CUDA(ctx_, cudaStreamSynchronize(ctx_->stream));
+                SCS_CUDA(ctx_, cudaFreeHost(cache_.vertex_pin));
+                cache_.vertex_pin = nullptr;
+                cache_.vertex_pin_bytes = 0;
+            }
+            SCS_CUDA(ctx_, cudaMallocHost(&cache_.vertex_pin, bytes));
+            cache_.vertex_pin_bytes = bytes;
+        }
+        std::memcpy(cache_.vertex_pin, vertex_.data(), bytes);
+        SCS_CUDA(ctx_, cudaMemcpyAsync(vertex_dev_.ptr, cache_.vertex_pin, bytes, cudaMemcpyHostToDevice, ctx_->stream));
+        ctx_->h2d_bytes += static_cast<int64_t>(bytes);
         return SCS_OK;
     }
 
@@ -492,8 +504,13 @@ class DeviceDriver {
     int plan_children(std::vector<Job> &wave, std::vector<Split> &splits, std::vector<Job> &next) {
         const int J = static_cast<int>(wave.size());
         std::vector<int32_t> job_tree_begin(static_cast<size_t>(J) + 1, 0), job_parts(J, 0), job_part_base(J, 0);
-        for (int j = 0; j < J; ++j) job_tree_begin[j] = wave[j].where.tree_begin;
+        std::vector<int64_t> job_node_begin(static_cast<size_t>(J) + 1, 0);  // the jobs' trees are laid out in job order
+        for (int j = 0; j < J; ++j) {
+            job_tree_begin[j] = wave[j].where.tree_begin;
+            job_node_begin[j] = wave[j].where.node_begin;
+        }
         job_tree_begin[J] = static_cast<int32_t>(current().trees);
+        job_node_begin[J] = current().nodes;
         std::sort(splits.begin(), splits.end(), [](const Split &a, const Split &b) { return a.job < b.job; });
         struct Pending {
             int32_t parent_slot;
@@ -565,7 +582,8 @@ class DeviceDriver {
         std::vector<DevJobInfo> info(static_cast<size_t>(new_jobs) + 1);
         if (new_jobs > 0) {
             Stopwatch sw_restrict(&restrict_device_s_);
-            const int rc = devforest_restrict(ctx_, current(), J, job_tree_begin.data(), job_parts.data(), job_part_base.data(),
+            const int rc = devforest_restrict(ctx_, current(), J, job_tree_begin.data(), job_node_begin.data(), job_parts.data(),
+                                              job_part_base.data(),
                                               static_cast<int>(part_newjob.size()), part_newjob.data(), new_jobs, owner_.data(),
                                               num_taxa_, &other(), info.data(), present_.data());
             if (rc) return rc;

@@ -64,18 +64,20 @@ int devforest_tours(scs_ctx *ctx, const DevForest &forest, int weighting, const 
                     int32_t *flags_dev);
 
 // Restriction of a wave's forest to the children of its jobs.
-//   src jobs j = 0..J-1: trees [job_tree_begin[j], job_tree_begin[j + 1]); job j was split into job_parts[j] parts
-//   (0: not split), numbered globally from job_part_base[j]; owner_dev[x] = global part of taxon x, or -1 (the taxon
-//   needs no restricted trees); part_newjob[p] = job of part p in the new forest, or -1.
+//   src jobs j = 0..J-1: trees [job_tree_begin[j], job_tree_begin[j + 1]), nodes [job_node_begin[j],
+//   job_node_begin[j + 1]); job j was split into job_parts[j] parts (0: not split), numbered globally from
+//   job_part_base[j]; owner_dev[x] = global part of taxon x, or -1 (the taxon needs no restricted trees);
+//   part_newjob[p] = job of part p in the new forest, or -1.
 // A tree is restricted to every part that keeps at least two of its tips (scs.py:447-448), exactly as
 // PhyloNode.get_sub_tree(names, ignore_missing=True, as_rooted=True): tips outside the part vanish, unary nodes are
 // merged into their child with  length(node) + length(child)  bottom-up, the new root loses its length.
 // The new forest is ordered by new job, trees in source order.  info[new_jobs] and present_host[num_taxa] (1 where a
-// taxon is still a tip of a kept tree) are filled before the call returns (two small synchronisations inside).
+// taxon is still a tip of a kept tree) are filled before the call returns, by its one synchronisation (two when a
+// split into many parts makes the bound of the workspace too large and its exact size is read back first).
 int devforest_restrict(scs_ctx *ctx, const DevForest &src, int num_jobs, const int32_t *job_tree_begin,
-                       const int32_t *job_parts, const int32_t *job_part_base, int num_parts, const int32_t *part_newjob,
-                       int new_jobs, const int32_t *owner_host, int num_taxa, DevForest *dst, DevJobInfo *info,
-                       uint8_t *present_host);
+                       const int64_t *job_node_begin, const int32_t *job_parts, const int32_t *job_part_base, int num_parts,
+                       const int32_t *part_newjob, int new_jobs, const int32_t *owner_host, int num_taxa, DevForest *dst,
+                       DevJobInfo *info, uint8_t *present_host);
 
 // (parent, taxon) of whole trees of the forest, packed one after the other into host arrays: tree i occupies forest
 // nodes [first_node[i], first_node[i] + tree_nodes[i]) (DevJobInfo.node_begin / first_tree_nodes).
