@@ -456,6 +456,19 @@ int scs_supertree_mrp(scs_ctx *ctx, const scs_forest *sources, int64_t num_nodes
 int scs_supertree_mast(scs_ctx *ctx, const scs_forest *sources, int64_t num_nodes, const int32_t *parent,
                        const int32_t *taxon, int64_t *per_tree);
 
+/* The same pass, also naming the taxa: per source tree t one maximum agreement set Y_t, read back from the table by a
+ * fixed tie rule (DESIGN.md §3.18; another maximum set may exist), so repeated calls give the same bytes.  per_tree[2 *
+ * T] is bit for bit that of scs_supertree_mast.  tip_state has one entry per forest node: 1 for a tip in Y_t, 0 for a
+ * tip in X_t \ Y_t, -1 for an internal node or a tip whose taxon the supertree lacks (a shared lone tip gets 1).  For
+ * every taxon p, over the trees t with p in X_t, int64 per_taxon[2 * num_taxa], row p: the number of such trees and
+ * the number of them with p not in Y_t (zero for taxa that are not tips of the supertree); weighted (may be NULL)
+ * [num_taxa]: w_t summed over the latter trees in tree order as acc = acc + w_t.  Refusals and messages are those of
+ * scs_supertree_mast under this name; SCS_ERR_CUDA with a message naming the tree if the device check of a traceback
+ * fails (kept count against the table, stack bound, a cell without support).  Returns after the results landed. */
+int scs_supertree_mast_taxa(scs_ctx *ctx, const scs_forest *sources, int64_t num_nodes, const int32_t *parent,
+                            const int32_t *taxon, int64_t *per_tree, int8_t *tip_state, int64_t *per_taxon,
+                            double *weighted);
+
 /* Rooted Robinson-Foulds distances between every pair of source trees of the forest, each pair restricted to the k
  * taxa X it shares (as scs_forest_induce restricts; no supertree is involved).  Three caller-owned T x T row-major
  * int32 arrays: shared_taxa[i][j] = k (symmetric; the diagonal is the tree's tip count); clusters[i][j] = the

@@ -17,7 +17,7 @@ import click
 from . import __version__
 from .distances import flat_source_tree_distances, flat_source_tree_triplet_distances
 from .load import load_forest
-from .mast import flat_mast_fit
+from .mast import flat_mast_fit, flat_mast_taxa
 from .engine import default_engine
 from .mrp import flat_mrp_score
 from .scs import flat_newick, supertree_newick_of_forest
@@ -29,7 +29,7 @@ def run(in_file: str, out_file: str, weighting: str = "branch", contract_edges: 
         support_out: str | None = None, triplets_out: str | None = None,
         taxon_triplets_out: str | None = None, mrp_out: str | None = None,
         source_rf_out: str | None = None, source_triplets_out: str | None = None,
-        mast_out: str | None = None) -> None:
+        mast_out: str | None = None, mast_taxa_out: str | None = None) -> None:
     """``load_trees`` + ``construct_supertree`` + ``write`` of the reference's command (ref: cli.py:33-39).  With
     ``support_out`` the supertree is also written there with the V support index of every internal non-root node
     (``support.flat_clade_support``) as its label; with ``triplets_out`` the triplet fit of every source tree
@@ -39,13 +39,15 @@ def run(in_file: str, out_file: str, weighting: str = "branch", contract_edges: 
     of source trees that share at least three taxa (``distances.flat_source_tree_distances``) is written there as
     TSV, and with ``source_triplets_out`` their rooted triplet distance
     (``distances.flat_source_tree_triplet_distances``); with ``mast_out`` the maximum agreement subtree of every
-    source tree and the supertree (``mast.flat_mast_fit``) is written there as TSV.  The supertree is built once either
-    way."""
+    source tree and the supertree (``mast.flat_mast_fit``) is written there as TSV, and with ``mast_taxa_out``, per
+    supertree tip, how many source trees share it and how many of their maximum agreement sets drop it
+    (``mast.flat_mast_taxa``).  The supertree is built once either way."""
     forest = load_forest(in_file)
     if forest.num_trees == 0:  # what construct_supertree says about an empty list (ref: scs.py:63-65)
         msg = "There must be at least one tree to make a supertree."
         raise ValueError(msg)
-    extras = (support_out, triplets_out, taxon_triplets_out, mrp_out, source_rf_out, source_triplets_out, mast_out)
+    extras = (support_out, triplets_out, taxon_triplets_out, mrp_out, source_rf_out, source_triplets_out, mast_out,
+              mast_taxa_out)
     if all(path is None for path in extras):
         text = supertree_newick_of_forest(forest, weighting.lower(), contract_edges=contract_edges)
         Path(out_file).write_text(text + "\n")
@@ -68,6 +70,9 @@ def run(in_file: str, out_file: str, weighting: str = "branch", contract_edges: 
     if mast_out is not None:
         fit_mast = flat_mast_fit(forest, built["parent"], built["taxon"], engine=engine)
         Path(mast_out).write_text(fit_mast.tsv())
+    if mast_taxa_out is not None:
+        taxa_mast = flat_mast_taxa(forest, built["parent"], built["taxon"], engine=engine)
+        Path(mast_taxa_out).write_text(taxa_mast.tsv())
     if source_rf_out is not None:
         distances = flat_source_tree_distances(forest, engine=engine)
         Path(source_rf_out).write_text(distances.tsv())
@@ -131,6 +136,12 @@ def run(in_file: str, out_file: str, weighting: str = "branch", contract_edges: 
     "agreement subtree keeps (TSV).",
     default=None,
 )
+@click.option(
+    "--mast-taxa-out",
+    help="Also write, per supertree taxon, how many source trees share it and how many of their largest agreement "
+    "subtrees drop it (TSV).",
+    default=None,
+)
 def scs(
     in_file: str,
     out_file: str,
@@ -144,11 +155,13 @@ def scs(
     source_rf_out: str | None,
     source_triplets_out: str | None,
     mast_out: str | None,
+    mast_taxa_out: str | None,
 ) -> None:
     """Run spectral cluster supertree over the given set of source trees."""
     run(in_file, out_file, pcg_weighting, contract_edges=not disable_contraction, support_out=support_out,
         triplets_out=triplets_out, taxon_triplets_out=taxon_triplets_out, mrp_out=mrp_out,
-        source_rf_out=source_rf_out, source_triplets_out=source_triplets_out, mast_out=mast_out)
+        source_rf_out=source_rf_out, source_triplets_out=source_triplets_out, mast_out=mast_out,
+        mast_taxa_out=mast_taxa_out)
 
 
 if __name__ == "__main__":

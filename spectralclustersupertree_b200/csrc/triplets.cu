@@ -58,6 +58,11 @@
 // against a node is a range test.  The maximum-weight matching of the children is a closed form when one side has two
 // children (the top two weights of each row); otherwise a warp runs the shortest-augmenting-path Hungarian method with
 // the smaller child list as rows, reading the weights on demand.
+//
+// Agreement sets (scs_supertree_mast_taxa).  After ma_tree a warp per tree reads one maximum agreement set back from
+// the table with a stack of pending cells (ma_trace, DESIGN.md §3.18): a cell descends into the first child cell of the
+// same value, t' side first, else into the positive pairs of a maximum matching of the children; the host turns the
+// kept flags of the t' positions into per-node states and per-taxon counts.
 
 #include <algorithm>
 #include <climits>
@@ -115,6 +120,11 @@ struct TripletArgs {
     const int32_t *mk;       // [trees]: k as counted on the host, which sized the region
     const int32_t *mhw;      // [trees]: Hungarian width, 0 when no node pair of t' and s' has both degrees >= 3
     int32_t *mtab;
+    // MAST traceback: tree t's t' positions at mkeep[mkoff[t]], 1 when the agreement set keeps them; merr[t] = 1 when
+    // a check of its traceback failed
+    const int64_t *mkoff;    // [trees + 1]
+    int8_t *mkeep;
+    int32_t *merr;           // [trees]
 };
 
 // One CTA per tree: t' positions, the S positions of its taxa and the depths between t'-neighbours.
@@ -864,6 +874,153 @@ __global__ void __launch_bounds__(kMastThreads, 1) ma_tree(TripletArgs a) {
     }
 }
 
+// The leftmost shallowest of the n gap depths g, by the whole warp: the root's id, as mast_build names it.
+__device__ int mast_root(const int32_t *g, int n) {
+    int best = INT_MAX, at = INT_MAX;
+    for (int i = threadIdx.x & 31; i < n; i += 32)
+        if (g[i] < best) {
+            best = g[i];
+            at = i;
+        }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) {
+        const int ob = __shfl_xor_sync(0xffffffffu, best, off), oa = __shfl_xor_sync(0xffffffffu, at, off);
+        if (ob < best || (ob == best && oa < at)) {
+            best = ob;
+            at = oa;
+        }
+    }
+    return at;
+}
+
+constexpr int kTraceWarps = 4;
+
+// One warp per tree of the chunk, after ma_tree filled its table: one maximum agreement set, read back from the table
+// from (root t', root s') with a stack of pending cells.  A cell (u, v) of value m descends into the first child u_i
+// of u with w(u_i, v) = m, else the first child v_j of v with w(u, v_j) = m, else into every pair of positive weight of
+// a maximum-weight matching of their children (the closed form with its pairing explicit, or mast_hungarian's
+// assignment); a leaf cell of value 1 keeps its t' position.  Pending cells have disjoint leaf sets of positive value,
+// so at most k of them wait, as (u, v) pairs in the builders' stk and cur of t' (2k + 1 ints, free after the fill).
+// Writes the k kept flags of the tree; merr[t] = 1, and the warp stops, if the kept count is not the table's root
+// value, the stack would pass k, or a cell on the way has no support.  Every lane walks the same cells; lane 0 writes.
+__global__ void __launch_bounds__(kTraceWarps * 32) ma_trace(TripletArgs a) {
+    const int lane = threadIdx.x & 31;
+    const int w = blockIdx.x * kTraceWarps + (threadIdx.x >> 5);
+    if (w >= a.t1 - a.t0) return;
+    const int t = a.t0 + w, k = a.k[w];
+    int8_t *keep = a.mkeep + a.mkoff[t];
+    if (k != a.mk[t]) {  // as ma_tree; a lone tip has no tour, and the host knows its state
+        if (lane == 0 && a.leaf_off[t + 1] > a.leaf_off[t]) a.merr[t] = 1;
+        return;
+    }
+    for (int q = lane; q < k; q += 32) keep[q] = k < 3;  // at most two shared taxa agree
+    if (k < 3) return;
+    const int64_t rel = a.leaf_off[t] - a.leaf0;
+    int32_t *base = a.mtab + (a.moff[t] - a.moff[a.t0]);
+    const int n = k - 1, hw = a.mhw[t];
+    const MastCells m{{base + static_cast<int64_t>(n) * n, k}, {base + static_cast<int64_t>(n) * n + mast_side_ints(k), k},
+                      a.sq + rel, a.sr + rel, base, n};
+    int32_t *hung = base + static_cast<int64_t>(n) * n + 2 * mast_side_ints(k) + k + 2;  // warp 0's arrays
+    int32_t *stk = m.T.stk();
+    const int rt = mast_root(a.td + rel, n), rs = mast_root(a.sdep + rel, n);
+    const int want = m.w(rt, rs);
+    int top = 0, kept = 0;
+    bool bad = false;
+    auto push = [&](int u, int v) {
+        if (top == k) {
+            bad = true;
+            return;
+        }
+        if (lane == 0) {
+            stk[2 * top] = u;
+            stk[2 * top + 1] = v;
+        }
+        ++top;
+    };
+    push(rt, rs);
+    __syncwarp();
+    while (top > 0 && !bad) {
+        --top;
+        const int u = stk[2 * top], v = stk[2 * top + 1];
+        const int val = m.w(u, v);
+        __syncwarp();  // every lane has read the slot before lane 0 reuses it
+        if (val <= 0) {
+            bad = true;
+            break;
+        }
+        if (u < 0 || v < 0) {  // a leaf against a node or a leaf, of value 1: its taxon is kept
+            if (lane == 0) keep[u < 0 ? ~u : m.sq[~v]] = 1;
+            ++kept;
+            continue;
+        }
+        const int ub = m.T.coff()[u], ue = m.T.coff()[u + 1], vb = m.S.coff()[v], ve = m.S.coff()[v + 1];
+        int one = -1;
+        for (int i = ub; i < ue && one < 0; ++i)
+            if (m.w(m.T.child()[i], v) == val) one = i;
+        if (one >= 0) {
+            push(m.T.child()[one], v);
+        } else {
+            for (int j = vb; j < ve && one < 0; ++j)
+                if (m.w(u, m.S.child()[j]) == val) one = j;
+            if (one >= 0) push(u, m.S.child()[one]);
+        }
+        if (one < 0) {
+            const int p = ue - ub, q = ve - vb;
+            int sum = 0;
+            auto pair = [&](bool rows_t, int i, int j) {  // row child i with column child j
+                const int wt = m.rc(rows_t, u, v, i, j);
+                sum += wt;
+                if (wt > 0) push(m.T.child()[ub + (rows_t ? i : j)], m.S.child()[vb + (rows_t ? j : i)]);
+            };
+            if (p == 2 || q == 2) {  // as ma_tree, with the columns of the top two of each row kept
+                const bool rows_t = p == 2;
+                int b0 = -1, s0 = -1, i0 = -1, j0 = -1, b1 = -1, s1 = -1, i1 = -1, j1 = -1;
+                for (int j = 0; j < (rows_t ? q : p); ++j) {
+                    const int w0 = m.rc(rows_t, u, v, 0, j), w1 = m.rc(rows_t, u, v, 1, j);
+                    if (w0 > b0) {
+                        s0 = b0;
+                        j0 = i0;
+                        b0 = w0;
+                        i0 = j;
+                    } else if (w0 > s0) {
+                        s0 = w0;
+                        j0 = j;
+                    }
+                    if (w1 > b1) {
+                        s1 = b1;
+                        j1 = i1;
+                        b1 = w1;
+                        i1 = j;
+                    } else if (w1 > s1) {
+                        s1 = w1;
+                        j1 = j;
+                    }
+                }
+                if (i0 != i1) {
+                    pair(rows_t, 0, i0);
+                    pair(rows_t, 1, i1);
+                } else if (b0 + s1 >= s0 + b1) {
+                    pair(rows_t, 0, i0);
+                    pair(rows_t, 1, j1);
+                } else {
+                    pair(rows_t, 0, j0);
+                    pair(rows_t, 1, i1);
+                }
+            } else {
+                mast_hungarian(m, u, v, hung, hw);
+                const bool rows_t = p <= q;
+                const int32_t *P = hung + 2 * static_cast<int64_t>(hw + 2);
+                for (int j = 1; j <= (rows_t ? q : p); ++j)
+                    if (P[j]) pair(rows_t, P[j] - 1, j - 1);
+                __syncwarp();  // P is read before the next cell's Hungarian run resets it
+            }
+            bad |= sum != val;
+        }
+        __syncwarp();
+    }
+    if (lane == 0 && (bad || kept != want)) a.merr[t] = 1;
+}
+
 // What both entry points share: the supertree validated and in pre-order, the depth of its leaves and the sparse
 // table over the depths between consecutive leaves, the chunk plan, and on the device the source forest, its tours,
 // those supertree arrays and the per-leaf scratch of a chunk.
@@ -1008,6 +1165,121 @@ struct TripletPass {
         forest.free_all(ctx);
         tours.free_all(ctx);
         for (GrowBuf *b : {&ident, &flags, &pos, &d_leaf_depth, &d_stab, &qpos, &spos, &td, &kbuf, &rows}) release(ctx, *b);
+    }
+};
+
+// What both MAST entry points share: the supertree step, per tree k (from its tips against S), the Hungarian width and
+// the ints of its region, refused above the cap before anything runs, the chunk plan, and the loop of mp_rank and
+// ma_tree over the chunks.
+struct MastPass {
+    TripletPass p;
+    int words = 0;
+    size_t rank_smem = 0;
+    std::vector<int32_t> hk, hw;
+    std::vector<int64_t> off;
+    GrowBuf d_per_tree, d_off, d_hk, d_hw, table;
+
+    // Host side; returns the failure status (message set, `name` leading it) or SCS_OK.
+    int prepare(scs_ctx *ctx, const char *name, const scs_forest *sources, int64_t num_nodes, const int32_t *parent,
+                const int32_t *taxon) {
+        int rc = p.supertree(ctx, name, sources, num_nodes, parent, taxon, 0);
+        if (rc) return rc;
+        const int T = p.T, taxa = p.taxa;
+        words = (p.s.leaves + 31) / 32;
+        rank_smem = static_cast<size_t>(words) * 8;
+        if (rank_smem + 1024 > ctx->smem_optin)  // room for the static shared arrays
+            return fail(ctx, SCS_ERR_INVALID, (std::string(name) + ": the supertree has too many tips for the shared-memory bitmap").c_str());
+        // per tree: k from its tips against S, the Hungarian width (restriction never raises a node's out-degree, so
+        // the unrestricted trees bound it) and the ints of its region, refused above the cap before anything runs
+        auto widest = [](const int32_t *par, int64_t nodes) {
+            std::vector<int32_t> kids(static_cast<size_t>(nodes), 0);
+            int most = 0;
+            for (int64_t i = 1; i < nodes; ++i)
+                if (par[i] >= 0 && par[i] < nodes) most = std::max(most, ++kids[par[i]]);
+            return most;
+        };
+        const int deg_s = widest(parent, num_nodes);
+        const std::vector<int64_t> &noff = sources->node_offsets;
+        hk.assign(static_cast<size_t>(std::max(T, 1)), 0);
+        hw.assign(hk.size(), 0);
+        off.assign(static_cast<size_t>(T) + 1, 0);
+        std::vector<int64_t> bytes(static_cast<size_t>(T), 0);
+        for (int t = 0; t < T; ++t) {
+            int k = 0;
+            for (int64_t i = noff[t]; i < noff[t + 1]; ++i) {
+                const int x = sources->taxon[i];
+                k += x >= 0 && x < taxa && p.s.pos[x] >= 0;
+            }
+            const int deg_t = widest(&sources->parent[noff[t]], noff[t + 1] - noff[t]);
+            hk[t] = k;
+            hw[t] = std::min({deg_s, deg_t, k}) >= 3 ? std::min(std::max(deg_s, deg_t), k) : 0;
+            const int64_t ints = mast_ints(k, hw[t]);
+            bytes[t] = ints * static_cast<int64_t>(sizeof(int32_t));
+            if (static_cast<size_t>(bytes[t]) > kTableBytes)
+                return fail(ctx, SCS_ERR_INVALID, (std::string(name) + ": source tree " + std::to_string(t) + " shares " +
+                                                   std::to_string(k) + " taxa with the supertree; its agreement table of " +
+                                                   std::to_string(bytes[t] >> 20) + " MiB is above the cap of " +
+                                                   std::to_string(kTableBytes >> 20) + " MiB").c_str());
+            off[t + 1] = off[t] + ints;
+        }
+        p.plan(sources, 0, &bytes);
+        return SCS_OK;
+    }
+
+    // Device side, for T > 0: per_tree[2 * T] on the host when it returns SCS_OK.  after(args) runs on every chunk
+    // once ma_tree is queued, before the next chunk reuses the scratch and the tables; `args` is set up for it.
+    template <class After>
+    int run(scs_ctx *ctx, const scs_forest *sources, int64_t *per_tree, TripletArgs &args, After after) {
+        int rc;
+        const int T = p.T;
+        if ((rc = p.upload(ctx, sources, &args))) return rc;
+        int64_t most = 4;
+        for (size_t c = 0; c + 1 < p.chunk_begin.size(); ++c)
+            most = std::max(most, off[p.chunk_begin[c + 1]] - off[p.chunk_begin[c]]);
+        if ((rc = grow(ctx, d_per_tree, 2 * static_cast<size_t>(T) * sizeof(int64_t))) ||
+            (rc = TripletPass::put(ctx, d_off, off.data(), off.size() * sizeof(int64_t))) ||
+            (rc = TripletPass::put(ctx, d_hk, hk.data(), hk.size() * sizeof(int32_t))) ||
+            (rc = TripletPass::put(ctx, d_hw, hw.data(), hw.size() * sizeof(int32_t))) ||
+            (rc = grow(ctx, table, static_cast<size_t>(most) * sizeof(int32_t))))
+            return rc;
+        if (rank_smem > 48 * 1024)
+            SCS_CUDA(ctx, cudaFuncSetAttribute(mp_rank, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(rank_smem)));
+        // S-ranks and depths between S-rank neighbours in the scratch of the triplet rows, as the MRP pass
+        const int64_t L = p.most_leaves + 1;
+        int32_t *scratch = p.rows.as<int32_t>();
+        args.words = words;
+        args.sq = scratch;
+        args.sr = scratch + L;
+        args.sdep = scratch + 2 * L;
+        args.moff = d_off.as<int64_t>();
+        args.mk = d_hk.as<int32_t>();
+        args.mhw = d_hw.as<int32_t>();
+        args.mtab = table.as<int32_t>();
+        args.per_tree = d_per_tree.as<int64_t>();
+        for (size_t c = 0; c + 1 < p.chunk_begin.size(); ++c) {
+            if ((rc = p.prep_chunk(ctx, sources, c, &args))) return rc;
+            if (args.chunk_leaves > 0) {
+                mp_rank<<<args.t1 - args.t0, kPrepThreads, rank_smem, ctx->stream>>>(args);
+                SCS_LAUNCHED(ctx, "mp_rank");
+            }
+            ma_tree<<<args.t1 - args.t0, kMastThreads, 0, ctx->stream>>>(args);
+            SCS_LAUNCHED(ctx, "ma_tree");
+            if ((rc = after(args))) return rc;
+        }
+        const size_t out_bytes = 2 * static_cast<size_t>(T) * sizeof(int64_t);
+        SCS_CUDA(ctx, cudaMemcpyAsync(per_tree, d_per_tree.ptr, out_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+        SCS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+        ctx->d2h_bytes += static_cast<int64_t>(out_bytes);
+        // a lone tip has no tour: it shares one taxon with S or none, and agrees on it
+        const std::vector<int64_t> &noff = sources->node_offsets;
+        for (int t = 0; t < T; ++t)
+            if (noff[t + 1] - noff[t] == 1) per_tree[2 * static_cast<int64_t>(t)] = per_tree[2 * static_cast<int64_t>(t) + 1] = hk[t];
+        return SCS_OK;
+    }
+
+    void release_all(scs_ctx *ctx) {
+        p.release_all(ctx);
+        for (GrowBuf *b : {&d_per_tree, &d_off, &d_hk, &d_hw, &table}) release(ctx, *b);
     }
 };
 
@@ -1201,97 +1473,93 @@ extern "C" int scs_supertree_mast(scs_ctx *ctx, const scs_forest *sources, int64
     if (!ctx) return SCS_ERR_INVALID;
     if (!sources || !parent || !taxon || !per_tree || num_nodes <= 0 || num_nodes >= (int64_t(1) << 31))
         return fail(ctx, SCS_ERR_INVALID, "scs_supertree_mast: bad argument");
-    TripletPass p;
-    int rc = p.supertree(ctx, "scs_supertree_mast", sources, num_nodes, parent, taxon, 0);
+    MastPass m;
+    int rc = m.prepare(ctx, "scs_supertree_mast", sources, num_nodes, parent, taxon);
     if (rc) return rc;
-    const int T = p.T, taxa = p.taxa;
-    const int words = (p.s.leaves + 31) / 32;
-    const size_t rank_smem = static_cast<size_t>(words) * 8;
-    if (rank_smem + 1024 > ctx->smem_optin)  // room for the static shared arrays
-        return fail(ctx, SCS_ERR_INVALID, "scs_supertree_mast: the supertree has too many tips for the shared-memory bitmap");
-    // per tree: k from its tips against S, the Hungarian width (restriction never raises a node's out-degree, so the
-    // unrestricted trees bound it) and the ints of its region, refused above the cap before anything runs
-    auto widest = [](const int32_t *par, int64_t nodes) {
-        std::vector<int32_t> kids(static_cast<size_t>(nodes), 0);
-        int most = 0;
-        for (int64_t i = 1; i < nodes; ++i)
-            if (par[i] >= 0 && par[i] < nodes) most = std::max(most, ++kids[par[i]]);
-        return most;
-    };
-    const int deg_s = widest(parent, num_nodes);
+    std::fill(per_tree, per_tree + 2 * static_cast<int64_t>(m.p.T), 0);
+    if (m.p.T == 0) return SCS_OK;
+    TripletArgs args{};
+    rc = m.run(ctx, sources, per_tree, args, [](const TripletArgs &) { return SCS_OK; });
+    m.release_all(ctx);
+    cudaStreamSynchronize(ctx->stream);
+    return rc;
+}
+
+extern "C" int scs_supertree_mast_taxa(scs_ctx *ctx, const scs_forest *sources, int64_t num_nodes,
+                                       const int32_t *parent, const int32_t *taxon, int64_t *per_tree,
+                                       int8_t *tip_state, int64_t *per_taxon, double *weighted) {
+    if (!ctx) return SCS_ERR_INVALID;
+    if (!sources || !parent || !taxon || !per_tree || !tip_state || !per_taxon || num_nodes <= 0 ||
+        num_nodes >= (int64_t(1) << 31))
+        return fail(ctx, SCS_ERR_INVALID, "scs_supertree_mast_taxa: bad argument");
+    MastPass m;
+    int rc = m.prepare(ctx, "scs_supertree_mast_taxa", sources, num_nodes, parent, taxon);
+    if (rc) return rc;
+    const int T = m.p.T, taxa = m.p.taxa;
     const std::vector<int64_t> &noff = sources->node_offsets;
-    std::vector<int32_t> hk(static_cast<size_t>(std::max(T, 1)), 0), hw(hk.size(), 0);
-    std::vector<int64_t> bytes(static_cast<size_t>(T), 0), off(static_cast<size_t>(T) + 1, 0);
-    for (int t = 0; t < T; ++t) {
-        int k = 0;
-        for (int64_t i = noff[t]; i < noff[t + 1]; ++i) {
-            const int x = sources->taxon[i];
-            k += x >= 0 && x < taxa && p.s.pos[x] >= 0;
-        }
-        const int deg_t = widest(&sources->parent[noff[t]], noff[t + 1] - noff[t]);
-        hk[t] = k;
-        hw[t] = std::min({deg_s, deg_t, k}) >= 3 ? std::min(std::max(deg_s, deg_t), k) : 0;
-        const int64_t ints = mast_ints(k, hw[t]);
-        bytes[t] = ints * static_cast<int64_t>(sizeof(int32_t));
-        if (static_cast<size_t>(bytes[t]) > kTableBytes)
-            return fail(ctx, SCS_ERR_INVALID, ("scs_supertree_mast: source tree " + std::to_string(t) + " shares " +
-                                               std::to_string(k) + " taxa with the supertree; its agreement table of " +
-                                               std::to_string(bytes[t] >> 20) + " MiB is above the cap of " +
-                                               std::to_string(kTableBytes >> 20) + " MiB").c_str());
-        off[t + 1] = off[t] + ints;
-    }
-    p.plan(sources, 0, &bytes);
     std::fill(per_tree, per_tree + 2 * static_cast<int64_t>(T), 0);
+    std::fill(tip_state, tip_state + noff[T], int8_t(-1));
+    std::fill(per_taxon, per_taxon + 2 * static_cast<int64_t>(taxa), 0);
+    if (weighted) std::fill(weighted, weighted + taxa, 0.0);
     if (T == 0) return SCS_OK;
 
-    GrowBuf d_per_tree, d_off, d_hk, d_hw, table;
+    // the kept flags of tree t's t' positions at koff[t], all offsets known from the host counts
+    std::vector<int64_t> koff(static_cast<size_t>(T) + 1, 0);
+    for (int t = 0; t < T; ++t) koff[t + 1] = koff[t] + m.hk[t];
+    std::vector<int8_t> keep(static_cast<size_t>(std::max<int64_t>(koff[T], 1)), 0);
+    std::vector<int32_t> err(static_cast<size_t>(T), 0);
+    GrowBuf d_koff, d_keep, d_err;
     auto run = [&]() -> int {
-        TripletArgs args{};
-        if ((rc = p.upload(ctx, sources, &args))) return rc;
-        int64_t most = 4;
-        for (size_t c = 0; c + 1 < p.chunk_begin.size(); ++c)
-            most = std::max(most, off[p.chunk_begin[c + 1]] - off[p.chunk_begin[c]]);
-        if ((rc = grow(ctx, d_per_tree, 2 * static_cast<size_t>(T) * sizeof(int64_t))) ||
-            (rc = TripletPass::put(ctx, d_off, off.data(), off.size() * sizeof(int64_t))) ||
-            (rc = TripletPass::put(ctx, d_hk, hk.data(), hk.size() * sizeof(int32_t))) ||
-            (rc = TripletPass::put(ctx, d_hw, hw.data(), hw.size() * sizeof(int32_t))) ||
-            (rc = grow(ctx, table, static_cast<size_t>(most) * sizeof(int32_t))))
+        if ((rc = TripletPass::put(ctx, d_koff, koff.data(), koff.size() * sizeof(int64_t))) ||
+            (rc = grow(ctx, d_keep, keep.size())) || (rc = grow(ctx, d_err, err.size() * sizeof(int32_t))))
             return rc;
-        if (rank_smem > 48 * 1024)
-            SCS_CUDA(ctx, cudaFuncSetAttribute(mp_rank, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(rank_smem)));
-        // S-ranks and depths between S-rank neighbours in the scratch of the triplet rows, as the MRP pass
-        const int64_t L = p.most_leaves + 1;
-        int32_t *scratch = p.rows.as<int32_t>();
-        args.words = words;
-        args.sq = scratch;
-        args.sr = scratch + L;
-        args.sdep = scratch + 2 * L;
-        args.moff = d_off.as<int64_t>();
-        args.mk = d_hk.as<int32_t>();
-        args.mhw = d_hw.as<int32_t>();
-        args.mtab = table.as<int32_t>();
-        args.per_tree = d_per_tree.as<int64_t>();
-        for (size_t c = 0; c + 1 < p.chunk_begin.size(); ++c) {
-            if ((rc = p.prep_chunk(ctx, sources, c, &args))) return rc;
-            if (args.chunk_leaves > 0) {
-                mp_rank<<<args.t1 - args.t0, kPrepThreads, rank_smem, ctx->stream>>>(args);
-                SCS_LAUNCHED(ctx, "mp_rank");
-            }
-            ma_tree<<<args.t1 - args.t0, kMastThreads, 0, ctx->stream>>>(args);
-            SCS_LAUNCHED(ctx, "ma_tree");
-        }
-        const size_t out_bytes = 2 * static_cast<size_t>(T) * sizeof(int64_t);
-        SCS_CUDA(ctx, cudaMemcpyAsync(per_tree, d_per_tree.ptr, out_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+        SCS_CUDA(ctx, cudaMemsetAsync(d_err.ptr, 0, err.size() * sizeof(int32_t), ctx->stream));
+        TripletArgs args{};
+        args.mkoff = d_koff.as<int64_t>();
+        args.mkeep = d_keep.as<int8_t>();
+        args.merr = d_err.as<int32_t>();
+        rc = m.run(ctx, sources, per_tree, args, [&](const TripletArgs &a) -> int {
+            ma_trace<<<ceil_div(a.t1 - a.t0, kTraceWarps), kTraceWarps * 32, 0, ctx->stream>>>(a);
+            SCS_LAUNCHED(ctx, "ma_trace");
+            return SCS_OK;
+        });
+        if (rc) return rc;
+        SCS_CUDA(ctx, cudaMemcpyAsync(keep.data(), d_keep.ptr, static_cast<size_t>(koff[T]), cudaMemcpyDeviceToHost, ctx->stream));
+        SCS_CUDA(ctx, cudaMemcpyAsync(err.data(), d_err.ptr, err.size() * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
         SCS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-        ctx->d2h_bytes += static_cast<int64_t>(out_bytes);
-        // a lone tip has no tour: it shares one taxon with S or none, and agrees on it
+        ctx->d2h_bytes += koff[T] + static_cast<int64_t>(err.size() * sizeof(int32_t));
         for (int t = 0; t < T; ++t)
-            if (noff[t + 1] - noff[t] == 1) per_tree[2 * static_cast<int64_t>(t)] = per_tree[2 * static_cast<int64_t>(t) + 1] = hk[t];
+            if (err[t])
+                return fail(ctx, SCS_ERR_CUDA, ("scs_supertree_mast_taxa: the agreement-set traceback of source tree " +
+                                                std::to_string(t) + " failed its device check").c_str());
         return SCS_OK;
     };
     rc = run();
-    p.release_all(ctx);
-    for (GrowBuf *b : {&d_per_tree, &d_off, &d_hk, &d_hw, &table}) release(ctx, *b);
+    m.release_all(ctx);
+    for (GrowBuf *b : {&d_koff, &d_keep, &d_err}) release(ctx, *b);
     cudaStreamSynchronize(ctx->stream);
-    return rc;
+    if (rc) return rc;
+
+    // t' position q of tree t is its q-th shared tip in node order (pre-order, the order of its tour); counts per taxon
+    // in tree order
+    const std::vector<int32_t> &spos = m.p.s.pos;
+    for (int t = 0; t < T; ++t) {
+        const int64_t b = noff[t], e = noff[t + 1];
+        const int32_t *par = &sources->parent[b];
+        const double wt = sources->weight[t];
+        int64_t q = koff[t];
+        for (int64_t i = b; i < e; ++i) {
+            if (i + 1 < e && par[i + 1 - b] == i - b) continue;  // not a tip
+            const int x = sources->taxon[i];
+            if (x < 0 || x >= taxa || spos[x] < 0) continue;
+            const bool kept = e - b == 1 || keep[q++];  // a lone tip has no tour, and agrees on itself
+            tip_state[i] = kept;
+            per_taxon[2 * static_cast<int64_t>(x)]++;
+            if (!kept) {
+                per_taxon[2 * static_cast<int64_t>(x) + 1]++;
+                if (weighted) weighted[x] = weighted[x] + wt;
+            }
+        }
+    }
+    return SCS_OK;
 }

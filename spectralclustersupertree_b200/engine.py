@@ -345,6 +345,28 @@ class Engine:
         _check(status, self._ctx)
         return per_tree
 
+    def supertree_mast_taxa(self, forest: "Forest", parent, taxon) -> tuple[np.ndarray, np.ndarray, np.ndarray,
+                                                                            np.ndarray]:  # fmt: skip
+        """``scs_supertree_mast_taxa``: ``per_tree`` ``[T, 2]`` (int64) as ``supertree_mast``; ``tip_state``
+        ``[num_nodes of forest]`` (int8): 1 for a tip the returned maximum agreement set keeps, 0 for a shared tip it
+        drops, -1 for internal nodes and tips the supertree lacks; per taxon id ``[num_taxa, 2]`` (int64): trees
+        sharing it and those of them dropping it; ``[num_taxa]``: the weights of the dropping trees summed in tree
+        order."""
+        parent = np.ascontiguousarray(parent, dtype=np.int32)
+        taxon = np.ascontiguousarray(taxon, dtype=np.int32)
+        n = len(parent)
+        if len(taxon) != n:
+            msg = "parent and taxon must have the same length"
+            raise ValueError(msg)
+        per_tree = np.zeros((forest.num_trees, 2), dtype=np.int64)
+        tip_state = np.zeros(forest.num_nodes, dtype=np.int8)
+        per_taxon = np.zeros((forest.num_taxa, 2), dtype=np.int64)
+        weighted = np.zeros(forest.num_taxa, dtype=np.float64)
+        status = self._lib.scs_supertree_mast_taxa(self._ctx, forest.handle, n, ptr(parent), ptr(taxon), ptr(per_tree),
+                                                   ptr(tip_state), ptr(per_taxon), ptr(weighted))  # fmt: skip
+        _check(status, self._ctx)
+        return per_tree, tip_state, per_taxon, weighted
+
     def _collect_supertree(self, handle, record: bool) -> dict:
         try:
             count = self._lib.scs_supertree_num_nodes(handle)

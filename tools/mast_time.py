@@ -1,13 +1,15 @@
 """Time ``scs_supertree_mast`` (csrc/triplets.cu) on the synthetic workloads of bench.py.
 
-    python tools/mast_time.py [--workload c4|c5] [--steps 5]
+    python tools/mast_time.py [--workload c4|c5] [--steps 5] [--warmup 1] [--taxa]
 
 The supertree is built through the product path (``Engine.supertree_build``) from the same seeded forest, then the
 MAST pass is timed with CUDA events on the context's stream after one warm-up call (the call includes uploading the
 source forest and copying the results back).  The per-tree triplet pass is timed the same way in the same run, for
 scale.  ``cells`` is the number of table cells the pass fills, sum_t I_t * I_s over the trees with k >= 3 (internal
-nodes of the two restrictions), next to its bound sum_t (k_t - 1)^2.  Prints one JSON line with the card name and
-power limit."""
+nodes of the two restrictions), next to its bound sum_t (k_t - 1)^2.  With ``--taxa`` ``scs_supertree_mast_taxa``
+(the same pass plus the traceback of one agreement set per tree) is timed the same way in the same run, and its
+per-tree counts are checked against ``scs_supertree_mast``'s.  ``--warmup 0`` skips the warm-up calls (C5's MAST call
+takes minutes).  Prints one JSON line with the card name and power limit."""
 
 from __future__ import annotations
 
@@ -90,6 +92,8 @@ def main() -> None:
     parser = argparse.ArgumentParser()
     parser.add_argument("--workload", default="c4", choices=["c4", "c5"])
     parser.add_argument("--steps", type=int, default=5)
+    parser.add_argument("--warmup", type=int, default=1)
+    parser.add_argument("--taxa", action="store_true", help="also time scs_supertree_mast_taxa")
     args = parser.parse_args()
     n, t, weighting, seed, tw = WORKLOADS[args.workload]
     t0 = time.perf_counter()
@@ -107,8 +111,9 @@ def main() -> None:
     parent, taxon = built["parent"], built["taxon"]
 
     def timed(call):
-        call(forest, parent, taxon)  # warm-up: modules loaded, allocator primed
-        print(f"{call.__name__}: warmed up", file=sys.stderr, flush=True)
+        for _ in range(args.warmup):  # modules loaded, allocator primed
+            call(forest, parent, taxon)
+            print(f"{call.__name__}: warmed up", file=sys.stderr, flush=True)
         ms = []
         for _ in range(args.steps):
             engine.timer_start()
@@ -118,6 +123,15 @@ def main() -> None:
         return out, ms
 
     per_tree, ms = timed(engine.supertree_mast)
+    extra = {}
+    if args.taxa:
+        (taxa_per_tree, tip_state, per_taxon, _weighted), taxa_ms = timed(engine.supertree_mast_taxa)
+        assert taxa_per_tree.tobytes() == per_tree.tobytes()
+        assert per_taxon[:, 0].sum() == per_tree[:, 0].sum()
+        assert per_taxon[:, 1].sum() == (per_tree[:, 0] - per_tree[:, 1]).sum()
+        extra = {"mast_taxa_ms_median": float(np.median(taxa_ms)), "mast_taxa_ms": taxa_ms,
+                 "kept_tips": int((tip_state == 1).sum()), "pruned_tips": int((tip_state == 0).sum()),
+                 "taxa_most_pruned": int(per_taxon[:, 1].max())}  # fmt: skip
     _triplets, triplet_ms = timed(engine.supertree_triplets)
     k, i_t, i_s = internal_counts(arrays, np.asarray(parent), np.asarray(taxon))
     assert np.array_equal(k, per_tree[:, 0])
@@ -133,7 +147,7 @@ def main() -> None:
         "pruned": shared - agreement, "trees_agreeing": int((per_tree[:, 0] == per_tree[:, 1]).sum()),
         "cells": int((i_t[big] * i_s[big]).sum()), "cells_bound": int(((k[big] - 1) ** 2).sum()),
         "mast_ms_median": float(np.median(ms)), "mast_ms_min": float(min(ms)), "mast_ms": ms,
-        "triplets_ms_median": float(np.median(triplet_ms)), "triplets_ms": triplet_ms,
+        **extra, "triplets_ms_median": float(np.median(triplet_ms)), "triplets_ms": triplet_ms,
         "build_s_first": build_s, "generate_s": gen_s, **gpu_info(),
     }))  # fmt: skip
     engine.close()
